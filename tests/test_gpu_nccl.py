@@ -42,9 +42,7 @@ def test_gather_records_over_nccl_two_ranks():
         pytest.skip("needs two GPUs")
     import torch.multiprocessing as mp
     from oracle import oracle as O
-    if not O.have_ref():
-        pytest.skip("oracle/_ref (the unmodified reference) is needed")
-    orc = O.load_ref()
+    from test_gpu_parity import assert_records_equal, reference_records
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
@@ -55,11 +53,10 @@ def test_gather_records_over_nccl_two_ranks():
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
-    dt = np.dtype(orc.RECORD_DTYPE)
+    dt = np.dtype(O.Oracle.RECORD_DTYPE)
     for strategy in ("degree", "random"):
-        want = orc.run_records("3-20-10-weighted", strategy, TOTAL, seed0=20, sel_seed0=5, compute_gb=True)
+        want = reference_records("3-20-10-weighted", strategy, TOTAL, seed0=20, sel_seed0=5)
         for rank in (0, 1):
             rec = np.frombuffer(got[rank][strategy], dtype=dt)
             assert rec.shape == (TOTAL,)
-            for f in dt.names:
-                assert np.array_equal(rec[f], want[f]), (strategy, rank, f)
+            assert_records_equal(rec, want, "%s, rank %d" % (strategy, rank))

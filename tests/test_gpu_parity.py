@@ -217,7 +217,13 @@ RECORD_FIELDS = ("steps", "additions", "zero_reductions", "nonzero_reductions", 
 
 def assert_records_equal(got, want, what):
     """Every field of every episode record (bb_episode_stats) bit-equal: pair sequence + rewards (trace_hash), length,
-    final basis, reduced Groebner basis, discounted return."""
+    final basis, reduced Groebner basis, discounted return.  `want` is a records array or, from reference_records, the
+    name of a run whose stored digests stand for the reference's records."""
+    if isinstance(want, str):
+        from oracle import golden
+        bad = golden.mismatches(got, want, RECORD_FIELDS)
+        assert not bad, "%s: %s differ from the reference's records (tests/golden/records.json)" % (what, bad)
+        return
     assert len(got) == len(want)
     for f in RECORD_FIELDS:
         bad = np.nonzero(got[f] != want[f])[0]
@@ -225,11 +231,17 @@ def assert_records_equal(got, want, what):
             what, len(bad), f, bad[0], got[f][bad[0]], want[f][bad[0]])
 
 
-def ref_oracle():
+def reference_records(dist, selection, count, seed0=0, sel_seed0=0, max_steps=0, **env_kw):
+    """The unmodified reference's records of a run (gamma 0.99, reduced basis computed): run live on oracle/_ref where
+    it is built, else the name of the run in tests/golden/records.json, for assert_records_equal."""
+    from oracle import golden
     from oracle import oracle as O
-    if not O.have_ref():
-        pytest.skip("oracle/_ref/libdgref.so (the unmodified reference) is needed for whole-run records")
-    return O.load_ref()
+    if O.have_ref():
+        return O.load_ref().run_records(dist, selection, count, seed0=seed0, sel_seed0=sel_seed0, max_steps=max_steps,
+                                        gamma=0.99, compute_gb=True, **env_kw)
+    k = golden.key(dist, selection, count, seed0=seed0, sel_seed0=sel_seed0, max_steps=max_steps, **env_kw)
+    assert golden.have(k), "no stored records of run %s: add it to tests/golden/make_records.py" % k
+    return k
 
 
 @pytest.mark.parametrize("strategy", ["degree", "first", "normal"])
@@ -238,7 +250,6 @@ def test_full_size_every_episode_16384(torch_cuda, strategy):
     record field against the unmodified reference env (buchberger.cpp:299-329 driven by oracle/ref_shim.cpp
     ref_run_records); plus counter identities and a bit-identical second run."""
     from deepgroebner_b200.buchberger import BuchbergerEngine
-    orc = ref_oracle()
     eng = BuchbergerEngine("3-20-10-weighted", num_envs=3552)
     eng.counters(reset=True)
     s1, _ = eng.run_episodes(strategy, episodes=16384, seed_base=0, compute_gb=True)
@@ -251,8 +262,7 @@ def test_full_size_every_episode_16384(torch_cuda, strategy):
     for f in RECORD_FIELDS:
         assert np.array_equal(s1[f], s2[f]), f
     assert (s1["additions"] >= s1["steps"]).all() and (s1["nbasis"] == 10 + s1["nonzero_reductions"]).all()
-    assert_records_equal(s1, orc.run_records("3-20-10-weighted", strategy, 16384, seed0=0, compute_gb=True),
-                         "3-20-10-weighted/" + strategy)
+    assert_records_equal(s1, reference_records("3-20-10-weighted", strategy, 16384), "3-20-10-weighted/" + strategy)
 
 
 @pytest.mark.parametrize("dist,s", [("3-20-10-uniform", 10), ("5-5-10-uniform", 10)])
@@ -260,7 +270,6 @@ def test_full_size_every_episode_65536(torch_cuda, dist, s):
     """BASELINE configs[2] at full size: ALL 65536 episodes of the uniform distributions under Degree selection (one
     resident wave of slots, like bench.py), every record field against the unmodified reference env."""
     from deepgroebner_b200.buchberger import BuchbergerEngine, resident_envs
-    orc = ref_oracle()
     E = 65536
     eng = BuchbergerEngine(dist, num_envs=resident_envs(0, int(dist.split("-")[0])))
     eng.counters(reset=True)
@@ -270,7 +279,7 @@ def test_full_size_every_episode_65536(torch_cuda, dist, s):
     assert c["episodes"] == E and c["env_steps"] == int(s1["steps"].sum()) and c["additions"] == int(s1["additions"].sum())
     assert c["zero_reductions"] + c["nonzero_reductions"] == c["env_steps"]
     assert (s1["additions"] >= s1["steps"]).all() and (s1["nbasis"] == s + s1["nonzero_reductions"]).all()
-    assert_records_equal(s1, orc.run_records(dist, "degree", E, seed0=0, compute_gb=True), dist)
+    assert_records_equal(s1, reference_records(dist, "degree", E), dist)
 
 
 ALL_STRATEGIES = ["first", "degree", "normal", "sugar", "random", "last", "codegree", "strange", "spice"]
@@ -446,13 +455,12 @@ def test_cyclic6_seeded_random_episodes(torch_cuda):
     seed) loop (reduction counts, additions, discounted return, reduced Groebner basis).  Degree is checked with its
     full pair sequence."""
     from deepgroebner_b200.buchberger import BuchbergerEngine
-    orc = ref_oracle()
+    orc = best_oracle()
     episodes, sel_seed = 256, 1234
     eng = BuchbergerEngine("cyclic-6", num_envs=episodes)
     stats, _ = eng.run_episodes("random", episodes=episodes, compute_gb=True, selection_seed=sel_seed, gamma=0.99)
     assert (stats["status"] == 2).all()
-    want = orc.run_records("cyclic-6", "random", episodes, sel_seed0=sel_seed, gamma=0.99, compute_gb=True)
-    assert_records_equal(stats, want, "cyclic-6/random")
+    assert_records_equal(stats, reference_records("cyclic-6", "random", episodes, sel_seed0=sel_seed), "cyclic-6/random")
     assert len(set(stats["steps"].tolist())) > episodes // 4   # the episodes really are different trajectories
     env = orc.env("cyclic-6")
     F, _ = env.reset()
@@ -550,5 +558,4 @@ def test_episode_preparation_by_thread_equals_by_warp(torch_cuda, dist, kw):
         assert np.array_equal(s0[f], s1[f]), f
     assert np.array_equal(t0, t1) and c0 == c1
     if not kw.get("sort_input") and kw.get("elimination", "gebauermoeller") == "gebauermoeller":   # lcm / none overflow the binomial pair capacity (flagged, equal in both modes)
-        want = ref_oracle().run_records(dist, "normal", episodes, seed0=11, compute_gb=True, max_steps=400, **kw)
-        assert_records_equal(s0, want, dist)
+        assert_records_equal(s0, reference_records(dist, "normal", episodes, seed0=11, max_steps=400, **kw), dist)

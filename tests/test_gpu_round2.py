@@ -5,7 +5,7 @@ BuchbergerEnv and the discount kernel.  Everything goes through the C-ABI; the o
 import numpy as np
 import pytest
 
-from test_gpu_parity import assert_records_equal, best_oracle, ref_oracle, trim
+from test_gpu_parity import assert_records_equal, best_oracle, reference_records, trim
 
 pytestmark = pytest.mark.gpu
 
@@ -81,13 +81,12 @@ def test_seven_and_eight_variables(torch_cuda, dist):
     8-variable order), lcm / divisibility, Gebauer-Moeller and the reduced basis: every record of 2048 episodes equals the
     unmodified reference's."""
     from deepgroebner_b200.buchberger import BuchbergerEngine
-    orc = ref_oracle()
     E = 2048
     eng = BuchbergerEngine(dist, num_envs=1024)
     for strategy in ("normal", "degree"):
         stats, _ = eng.run_episodes(strategy, episodes=E, seed_base=3, compute_gb=True)
         assert (stats["status"] == 2).all()
-        assert_records_equal(stats, orc.run_records(dist, strategy, E, seed0=3, compute_gb=True), dist + "/" + strategy)
+        assert_records_equal(stats, reference_records(dist, strategy, E, seed0=3), dist + "/" + strategy)
 
 
 def test_eight_variable_monomial_order(torch_cuda):
@@ -113,7 +112,7 @@ def test_cyclic6_observation_and_cxx_nvars_quirk(torch_cuda):
     (FixedIdealGenerator::nvars, ideals.cpp:146-154); compat_cxx_nvars=True reproduces its matrices byte for byte, the
     default shows all 6 (24 columns) with the same leading 5 of every monomial."""
     from deepgroebner_b200 import LeadMonomialsEnv
-    orc = ref_oracle()
+    orc = best_oracle()
     ref = orc.lm_env("cyclic-6", k=2)
     env = LeadMonomialsEnv("cyclic-6", k=2, compat_cxx_nvars=True)
     full = LeadMonomialsEnv("cyclic-6", k=2)
@@ -220,11 +219,10 @@ def test_prepared_batches_pipeline(torch_cuda):
     that does not match the next run is ignored; back-to-back pipelined calls on alternating staging sets stay exact."""
     torch = torch_cuda
     from deepgroebner_b200.buchberger import BuchbergerEngine
-    orc = ref_oracle()
     E = 3000
     eng = BuchbergerEngine("3-20-10-weighted", num_envs=1024)
     side = torch.cuda.Stream()
-    want = {b: orc.run_records("3-20-10-weighted", "degree", E, seed0=b, compute_gb=True) for b in (0, 5000, 9000)}
+    want = {b: reference_records("3-20-10-weighted", "degree", E, seed0=b) for b in (0, 5000, 9000)}
     seeds = torch.arange(5000, 5000 + E, dtype=torch.int32, device="cuda")
     # plain, then prepared with explicit seeds, then a prepared batch that is NOT the one run next
     stats, _ = eng.run_episodes("degree", episodes=E, seed_base=0, compute_gb=True)
@@ -268,8 +266,7 @@ def test_shards_follow_the_global_episode_index(torch_cuda):
     total = 157
     eng = BuchbergerEngine("3-20-10-uniform", num_envs=64)
     whole = sharding.run_sharded(eng, "random", total, seed_base=10, compute_gb=True, selection_seed=77)
-    orc = ref_oracle()
-    assert_records_equal(whole, orc.run_records("3-20-10-uniform", "random", total, seed0=10, sel_seed0=77, compute_gb=True),
+    assert_records_equal(whole, reference_records("3-20-10-uniform", "random", total, seed0=10, sel_seed0=77),
                          "random, one block")
     for ws in (2, 3):
         parts = []
@@ -281,6 +278,7 @@ def test_shards_follow_the_global_episode_index(torch_cuda):
             parts.append(st.copy())
         assert_records_equal(np.concatenate(parts), whole, "random, %d shards" % ws)
     # fixed ideals: three different staged ideals, episode g replays ideal g mod 3
+    orc = best_oracle()
     env = orc.env("3-20-10-weighted")
     ideals = []
     for s in (1, 2, 3):
@@ -426,11 +424,10 @@ def test_runners_of_two_batches_overlap_on_two_streams(torch_cuda):
     torch = torch_cuda
     from deepgroebner_b200 import _lib
     from deepgroebner_b200.buchberger import BuchbergerEngine, resident_envs
-    orc = ref_oracle()
     E = 6000
     eng = BuchbergerEngine("3-20-10-weighted", num_envs=min(resident_envs(0, 3), E))
     bases = [0, 7000, 14000, 0, 7000, 14000, 0]
-    want = {b: orc.run_records("3-20-10-weighted", "degree", E, seed0=b, compute_gb=True) for b in set(bases)}
+    want = {b: reference_records("3-20-10-weighted", "degree", E, seed0=b) for b in set(bases)}
     main, alt, side = torch.cuda.current_stream(), torch.cuda.Stream(), torch.cuda.Stream()
     outs = [torch.empty(E * 72, dtype=torch.uint8, device="cuda") for _ in bases]
     torch.cuda.synchronize()
