@@ -7,11 +7,14 @@ there is no CPU fallback.  Importing this package does not load CUDA; constructi
 from .ideals import BinomialSpec, FixedIdealGenerator, PolySpec, cyclic, parse_ideal_dist  # noqa: F401
 
 __all__ = ["BuchbergerEnv", "LeadMonomialsEnv", "BuchbergerEngine", "BuchbergerAgent", "BinomialSpec", "PolySpec",
-           "FixedIdealGenerator", "cyclic", "parse_ideal_dist"]
+           "FixedIdealGenerator", "cyclic", "parse_ideal_dist", "groebner_bases"]
 
 
 def __getattr__(name):  # torch / CUDA are only pulled in when an environment class is requested
     if name in ("BuchbergerEnv", "LeadMonomialsEnv", "BuchbergerEngine", "BuchbergerAgent"):
         from . import buchberger
         return getattr(buchberger, name)
+    if name == "groebner_bases":
+        from . import strat
+        return strat.groebner_bases
     raise AttributeError(name)

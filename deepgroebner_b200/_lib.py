@@ -47,6 +47,12 @@ class BBEpisodeStats(C.Structure):
                 ("gb_terms", C.c_int32), ("discounted_return", C.c_double)]
 
 
+class BBPolySink(C.Structure):
+    """bb_poly_sink: a packed, caller-owned device buffer of polynomials (bb_run_export)."""
+    _fields_ = [("lens_dev", C.c_void_p), ("exps_dev", C.c_void_p), ("coefs_dev", C.c_void_p), ("where_dev", C.c_void_p),
+                ("used_dev", C.c_void_p), ("cap_polys", C.c_int64), ("cap_terms", C.c_int64)]
+
+
 # numpy view of bb_episode_stats (same layout; checked against sizeof in load())
 STATS_DTYPE = [("steps", "<i4"), ("additions", "<i4"), ("zero_reductions", "<i4"), ("nonzero_reductions", "<i4"),
                ("nbasis", "<i4"), ("nterms", "<i4"), ("status", "<i4"), ("rerolls", "<i4"), ("trace_hash", "<u8"),
@@ -60,6 +66,7 @@ EXPORTS = [
     "bb_seed_selection", "bb_value", "bb_copy_env", "bb_set_auto_reset", "bb_step_observe", "bb_step_host", "bb_reset_host", "bb_observe_host", "bb_set_wide", "bb_set_prepare_mode", "bb_set_selection_seed_stride", "bb_policy_pmlp", "bb_rollout",
     "bb_seed_on", "bb_prepare", "bb_set_episode_offset", "bb_set_timing", "bb_last_run_ms", "bb_set_max_episode_length",
     "bb_set_compaction", "bb_compact", "bb_status_summary", "bb_set_obs_nvars", "bb_discount", "bb_set_serve", "bb_set_prefetch",
+    "bb_run_export",
 ]
 
 _lib = None
@@ -125,6 +132,8 @@ def load():
     lib.bb_stats.argtypes = [vp, vp, vp]
     lib.bb_run.restype = i
     lib.bb_run.argtypes = [vp, i, i, i, vp, i, i, C.c_double, i, vp, vp, i, i, vp]
+    lib.bb_run_export.restype = i
+    lib.bb_run_export.argtypes = lib.bb_run.argtypes + [C.POINTER(BBPolySink), C.POINTER(BBPolySink)]
     lib.bb_value.restype = i
     lib.bb_value.argtypes = [vp, i, C.c_double, i, i, i, vp, vp]
     lib.bb_copy_env.restype = i

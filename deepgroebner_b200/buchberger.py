@@ -23,6 +23,82 @@ CAPACITY_PRESETS = {
 }
 
 
+# default room per episode of the polynomial sinks of run_episodes(return_gb / return_basis), as (polynomials, terms);
+# a run that needs more is repeated once with the exact totals.  Measured on the C restatement of the reference (2000
+# seeds): reduced bases average 3.6 / 4.0 (3-20-10-weighted) and 17 / 22 (5-5-10-uniform, max 54 / 74) polynomials / terms,
+# final bases 63 and 82 terms.  The "poly" and "general" rows are not measured (a fraction of the arena capacities).
+SINK_ROOM = {
+    "binomial": dict(gb=(24, 32), basis=(64, 128)),
+    "poly": dict(gb=(32, 512), basis=(128, 2048)),
+    "general": dict(gb=(128, 8192), basis=(512, 32768)),
+}
+# word index (int32) of the record fields that size an episode's entry in each sink
+_REC = {f: np.dtype(_lib.STATS_DTYPE).fields[f][1] // 4 for f in ("nbasis", "nterms", "gb_polys", "gb_terms")}
+_SINK_COUNTS = {"gb": ("gb_polys", "gb_terms"), "basis": ("nbasis", "nterms")}
+
+
+class PolyBatch:
+    """Polynomials of every episode of a run, device-resident, in episode order (run_episodes(return_gb / return_basis)).
+
+    ep_offsets int64 [E+1] indexes polynomials, poly_offsets int64 [P+1] indexes terms, exps int32 [T, n], coefs int32 [T]
+    in [0, p), stored bool [E] (False: the episode did not end in a state that stores anything).  ``batch[e]`` is the
+    ``[(coef, exps), ...]`` list of episode e as final_gb() / basis() return it, or None when nothing was stored."""
+
+    def __init__(self, ep_offsets, poly_offsets, exps, coefs, stored):
+        self.ep_offsets, self.poly_offsets, self.exps, self.coefs, self.stored = ep_offsets, poly_offsets, exps, coefs, stored
+
+    def __len__(self):
+        return self.stored.numel()
+
+    def to_lists(self):
+        """Every episode as batch[e] gives it (one copy to the host)."""
+        eo, po = self.ep_offsets.tolist(), self.poly_offsets.tolist()
+        ex, cf, st = self.exps.cpu().tolist(), self.coefs.cpu().tolist(), self.stored.tolist()
+        out = []
+        for e in range(len(st)):
+            if not st[e]:
+                out.append(None)
+                continue
+            out.append([[(cf[t], tuple(ex[t])) for t in range(po[q], po[q + 1])] for q in range(eo[e], eo[e + 1])])
+        return out
+
+    def __getitem__(self, e):
+        e = int(e)
+        if not bool(self.stored[e]):
+            return None
+        q0, q1 = int(self.ep_offsets[e]), int(self.ep_offsets[e + 1])
+        po = self.poly_offsets[q0:q1 + 1].tolist()
+        ex = self.exps[po[0]:po[-1]].cpu().tolist()
+        cf = self.coefs[po[0]:po[-1]].cpu().tolist()
+        return [[(cf[t - po[0]], tuple(ex[t - po[0]])) for t in range(po[q], po[q + 1])] for q in range(len(po) - 1)]
+
+    def __eq__(self, other):
+        return isinstance(other, PolyBatch) and all(
+            torch.equal(getattr(self, f), getattr(other, f)) for f in ("ep_offsets", "poly_offsets", "exps", "coefs", "stored"))
+
+    @staticmethod
+    def from_sink(lens, exps, coefs, where, npolys, nterms, nvars):
+        """Canonical episode order from a packed bb_poly_sink, with tensor ops on the sink's device: where int64 [E, 2]
+        (first polynomial, first term of each episode, -1 where nothing was stored), npolys / nterms [E] the size of each
+        episode's entry (taken from the episode records)."""
+        dev = where.device
+        E = where.shape[0]
+        stored = where[:, 0] >= 0
+        zero = torch.zeros(1, dtype=torch.int64, device=dev)
+        npol = torch.where(stored, npolys.to(torch.int64), 0)
+        nter = torch.where(stored, nterms.to(torch.int64), 0)
+        ep_offsets = torch.cat([zero, torch.cumsum(npol, 0)])
+        term_offsets = torch.cat([zero, torch.cumsum(nter, 0)])
+        P, T = (int(x) for x in torch.stack([ep_offsets[-1], term_offsets[-1]]).tolist())
+        eps = torch.arange(E, device=dev)
+        ep_of_poly = torch.repeat_interleave(eps, npol, output_size=P)
+        src_poly = where[ep_of_poly, 0] + torch.arange(P, device=dev) - ep_offsets[ep_of_poly]
+        poly_offsets = torch.cat([zero, torch.cumsum(lens[src_poly].to(torch.int64), 0)])
+        ep_of_term = torch.repeat_interleave(eps, nter, output_size=T)
+        src_term = where[ep_of_term, 1] + torch.arange(T, device=dev) - term_offsets[ep_of_term]
+        return PolyBatch(ep_offsets, poly_offsets, exps.view(-1, nvars)[src_term], coefs[src_term], stored)
+
+
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
@@ -60,7 +136,8 @@ class BuchbergerEngine:
         self.k, self.num_envs, self.prime = int(k), int(num_envs), int(prime)
         self.elimination, self.rewards = elimination, rewards
         default = {BinomialSpec: "binomial", PolySpec: "poly"}.get(type(self.spec), "general")
-        preset = dict(CAPACITY_PRESETS[capacity or default])
+        self.preset = capacity or default
+        preset = dict(CAPACITY_PRESETS[self.preset])
         gen_caps = {k_: caps.pop(k_) for k_ in ("max_gens", "max_gen_terms") if k_ in caps}
         preset.update(caps)
         if isinstance(self.spec, BinomialSpec):
@@ -339,15 +416,23 @@ class BuchbergerEngine:
 
     def run_episodes(self, strategy="degree", episodes=None, seed_base=0, seeds=None, max_steps=0, gamma=0.99,
                      compute_gb=False, trace_episodes=0, trace_cap=0, to_host=True, selection_seed=0, out_host=None,
-                     out=None):
-        """Runs `episodes` episodes to completion with on-device selection (bb_run).  Returns (stats, trace):
+                     out=None, return_gb=False, return_basis=False, gb_capacity=None, basis_capacity=None):
+        """Runs `episodes` episodes to completion with on-device selection (bb_run_export).  Returns (stats, trace):
         stats is a structured array of bb_episode_stats (numpy if to_host else a uint8 cuda tensor), trace an
         int32 [trace_episodes, trace_cap, 4] array of (i, j, additions, |P| after), -1 padded.
         seeds: per-episode ideal-stream seeds, a numpy array or an int32 torch tensor (pinned host memory is copied
         asynchronously); out_host: a pinned uint8 host tensor of episodes * 72 bytes that receives the records (the
         returned array is a view of it); out: a uint8 cuda tensor of episodes * 72 bytes for the records instead of the
-        engine's own buffer (calls in flight on different streams need different ones)."""
+        engine's own buffer (calls in flight on different streams need different ones).
+        return_gb / return_basis: also return every episode's reduced Groebner basis (return_gb implies compute_gb; stored
+        for episodes that end done) and / or final basis G in insertion order (episodes that end done or are cut by
+        max_steps), as (stats, trace, {"gb": PolyBatch, "basis": PolyBatch}).  gb_capacity / basis_capacity: room of each
+        sink as (polynomials, terms) over the whole call (default: SINK_ROOM per episode of the capacity preset).  A run
+        whose polynomials do not fit is repeated once with the exact totals -- a second run of the same episodes, with
+        the same records (runs are deterministic).  Reading the sinks' fill synchronises the stream."""
         episodes = self.num_envs if episodes is None else int(episodes)
+        want = [k for k, on in (("gb", return_gb), ("basis", return_basis)) if on]
+        compute_gb = compute_gb or return_gb
         with torch.cuda.device(self.device):
             nbytes = max(episodes, 1) * C.sizeof(_lib.BBEpisodeStats)
             buf = out if out is not None else getattr(self, "_run_buf", None)
@@ -372,19 +457,54 @@ class BuchbergerEngine:
                 else:
                     d_seeds = torch.as_tensor(np.ascontiguousarray(seeds, np.int32), device=self.device)
                     assert d_seeds.numel() == episodes
-            self._ck(self.lib.bb_run(self.h, _lib.SELECTION[strategy], episodes, int(seed_base), _ptr(d_seeds),
-                                     int(selection_seed), int(max_steps), float(gamma), int(bool(compute_gb)),
-                                     _ptr(buf), _ptr(trace),
-                                     int(trace_episodes), int(trace_cap), _stream()), "bb_run")
+            room = {"gb": gb_capacity, "basis": basis_capacity}
+            for k in want:
+                if room[k] is None:
+                    room[k] = tuple(episodes * x for x in SINK_ROOM[self.preset][k])
+            for attempt in range(2):
+                sinks = {k: self._sink(episodes, *room[k]) for k in want}
+                self._ck(self.lib.bb_run_export(self.h, _lib.SELECTION[strategy], episodes, int(seed_base), _ptr(d_seeds),
+                                                int(selection_seed), int(max_steps), float(gamma), int(bool(compute_gb)),
+                                                _ptr(buf), _ptr(trace), int(trace_episodes), int(trace_cap), _stream(),
+                                                sinks["gb"][1] if "gb" in sinks else None,
+                                                sinks["basis"][1] if "basis" in sinks else None), "bb_run_export")
+                if not want:
+                    break
+                used = {k: sinks[k][0]["used"].tolist() for k in want}
+                if attempt or all(used[k][2] == 0 for k in want):
+                    break
+                room = {k: (used[k][0], used[k][1]) for k in want}
+            polys = {}
+            if want:
+                rec = buf[:episodes * C.sizeof(_lib.BBEpisodeStats)].view(torch.int32).view(-1, C.sizeof(_lib.BBEpisodeStats) // 4)
+                for k in want:
+                    t = sinks[k][0]
+                    fp, ft = _SINK_COUNTS[k]
+                    polys[k] = PolyBatch.from_sink(t["lens"], t["exps"], t["coefs"], t["where"], rec[:, _REC[fp]],
+                                                   rec[:, _REC[ft]], self.n)
             if not to_host:
-                return buf[:nbytes], trace
+                return (buf[:nbytes], trace, polys) if want else (buf[:nbytes], trace)
             if out_host is not None:
                 out_host[:nbytes].copy_(buf[:nbytes], non_blocking=True)
                 torch.cuda.current_stream().synchronize()
                 stats = out_host.numpy().view(np.dtype(_lib.STATS_DTYPE))[:episodes]
             else:
                 stats = buf[:nbytes].cpu().numpy().view(np.dtype(_lib.STATS_DTYPE))[:episodes]
-            return stats, (trace.cpu().numpy() if trace is not None else None)
+            trace = trace.cpu().numpy() if trace is not None else None
+            return (stats, trace, polys) if want else (stats, trace)
+
+    def _sink(self, episodes, polys, terms):
+        """Device buffers of one bb_poly_sink for `episodes` episodes and its ctypes struct."""
+        d, i32 = self.device, torch.int32
+        t = dict(lens=torch.empty(max(int(polys), 1), dtype=i32, device=d),
+                 exps=torch.empty(max(int(terms), 1) * self.n, dtype=i32, device=d),
+                 coefs=torch.empty(max(int(terms), 1), dtype=i32, device=d),
+                 where=torch.empty((max(episodes, 1), 2), dtype=torch.int64, device=d)[:episodes],
+                 used=torch.zeros(3, dtype=torch.int64, device=d))
+        s = _lib.BBPolySink(lens_dev=t["lens"].data_ptr(), exps_dev=t["exps"].data_ptr(), coefs_dev=t["coefs"].data_ptr(),
+                            where_dev=t["where"].data_ptr(), used_dev=t["used"].data_ptr(), cap_polys=int(polys),
+                            cap_terms=int(terms))
+        return t, C.byref(s), s
 
     def value(self, strategy="degree", gamma=0.99, rollouts=None, selection_seed=0, max_steps=0, out=None):
         """BuchbergerEnv.value for every environment (bb_value): float64 cuda tensor [N].  strategy is a selection

@@ -1233,6 +1233,42 @@ __device__ __noinline__ unsigned long long warp_terms_hash(const uint64_t* tk, c
   return h;
 }
 
+// The same polynomial list (lengths with a stride, as in warp_terms_hash) written to a caller's bb_poly_sink as episode
+// `ep`: lane 0 reserves room with two atomics and publishes where[ep] (-1, -1 and used[2] += 1 when it does not fit), the
+// lanes unpack the keys into NV int32 exponents.  Once per episode, out of line (cold).
+template <int NV>
+__device__ __noinline__ void warp_export_polys(const uint64_t* tk, const uint32_t* tc, const int* lens, int lens_stride,
+                                               int npoly, int nT, const bb_poly_sink& sink, int ep) {
+  typedef KL<NV> K;
+  const int lane = bb_lane();
+  long long p0 = 0, t0 = 0;
+  int ok = 0;
+  if (lane == 0) {
+    p0 = (long long)atomicAdd(&sink.used_dev[0], (unsigned long long)npoly);
+    t0 = (long long)atomicAdd(&sink.used_dev[1], (unsigned long long)nT);
+    ok = p0 + npoly <= sink.cap_polys && t0 + nT <= sink.cap_terms;
+    if (!ok) atomicAdd(&sink.used_dev[2], 1ull);
+    sink.where_dev[2 * (size_t)ep] = ok ? p0 : -1;
+    sink.where_dev[2 * (size_t)ep + 1] = ok ? t0 : -1;
+  }
+  ok = __shfl_sync(BB_FULL, ok, 0);
+  if (!ok) return;
+  p0 = (long long)bb_shfl64((uint64_t)p0, 0);
+  t0 = (long long)bb_shfl64((uint64_t)t0, 0);
+  int32_t* lo = sink.lens_dev + p0;
+  int32_t* eo = sink.exps_dev + t0 * NV;
+  int32_t* co = sink.coefs_dev + t0;
+#pragma unroll 1
+  for (int p = lane; p < npoly; p += 32) lo[p] = lens[(size_t)p * lens_stride];
+#pragma unroll 1
+  for (int t = lane; t < nT; t += 32) {
+    const uint64_t k = tk[t];
+#pragma unroll
+    for (int v = 0; v < NV; v++) eo[(size_t)t * NV + v] = (int32_t)K::exp(k, v);
+    co[t] = (int32_t)tc[t];
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------- final GB
 // interreduce(minimalize(G)), buchberger.cpp:102-122.  minimalize: G sorted ascending by lead monomial (stable),
 // g kept iff no kept lead monomial divides LM g  <=>  no f with LM f strictly dividing LM g and no earlier f

@@ -43,6 +43,7 @@ struct BBRunArgs {
   int max_steps;
   double gamma;
   int compute_gb;
+  bb_poly_sink gb_sink, basis_sink;   // bb_run_export (lens_dev == NULL: no sink); where_dev is indexed by ep_base + b
   bb_episode_stats* out;
   int32_t* trace;
   int trace_eps, trace_cap;
@@ -736,10 +737,30 @@ __device__ __forceinline__ void run_episode(const BBParams& P, Env& e, int strat
   }
 }
 
+// bb_run_export's sinks at the end of episode `ep` of slot `slot` (the runners' epilogue, after env_store and the reduced
+// basis): the reduced basis of an episode that ends done from the slot's GB arena, G of an episode that ends done or is cut
+// by max_steps (status still running) from the slot's term arena.  One out-of-line call per episode, and only when a sink
+// is attached, so the runners' step loop does not change.
+template <int NV>
+__device__ __noinline__ void warp_export_episode(const BBParams& P, const BBRunArgs& A, int slot, int ep, int status) {
+  if (A.gb_sink.lens_dev && status == BB_STATUS_DONE)
+    warp_export_polys<NV>(P.gkey + (size_t)slot * P.max_terms, P.gcoef + (size_t)slot * P.max_terms,
+                          P.glen + (size_t)slot * P.max_basis, 1, P.gcount[2 * slot], P.gcount[2 * slot + 1], A.gb_sink, ep);
+  if (A.basis_sink.lens_dev && (status == BB_STATUS_DONE || status == BB_STATUS_RUNNING)) {
+    Env e; env_load(P, slot, e);
+    const GHeadMem* gh = ENV_PTR(GHeadMem, e, P, o_ghead);
+    warp_export_polys<NV>(ENV_PTR(uint64_t, e, P, o_tkey), ENV_PTR(uint32_t, e, P, o_tcoef),
+                          reinterpret_cast<const int*>(&gh[0].len), (int)(sizeof(GHeadMem) / sizeof(int)), e.nG, e.nT,
+                          A.basis_sink, ep);
+  }
+}
+
 // Persistent episode runner.  Each warp owns slot = its global warp index and loops: pop an episode, copy its
 // prepared initial state from the staging arena, select/step until P is empty (or max_steps), write the episode
-// record, repeat.  WARPS = warps per CTA.
-template <int NV, bool STREAMS, int WARPS>
+// record, repeat.  WARPS = warps per CTA.  EXPORT: bb_run_export's sinks may be attached (an instantiation of its own, so
+// the runner without sinks keeps the parent's code: k_run is issue- and instruction-footprint-bound, and the one extra call
+// site in its loop measured 3 % on configs[1]).
+template <int NV, bool STREAMS, int WARPS, bool EXPORT>
 __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S, const BBRunArgs& A) {
   __shared__ unsigned long long sh[WARPS][CT_COUNT];
   __shared__ BBEpisodeAcc acc_sh[WARPS];  // per-episode accumulators only lane 0 touches: kept out of registers
@@ -792,6 +813,7 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
           status = BB_STATUS_OVERFLOW_SCRATCH;
         }
       }
+      if (EXPORT && (A.gb_sink.lens_dev || A.basis_sink.lens_dev)) warp_export_episode<NV>(P, A, slot, ep, status);
       if (lane == 0) {
         const unsigned long long th = acc.th; const double ret = acc.ret;
         bb_episode_stats o;
@@ -819,11 +841,11 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
   }
 }
 
-template <int NV>
+template <int NV, bool EXPORT = false>
 __global__ void __launch_bounds__(BB_THREADS, BB_MIN_BLOCKS) k_run(const __grid_constant__ BBParams P,
                                                                   const __grid_constant__ BBParams S,
                                                                   const __grid_constant__ BBRunArgs A) {
-  run_worker<NV, false, BB_WARPS>(P, S, A);
+  run_worker<NV, false, BB_WARPS, EXPORT>(P, S, A);
 }
 
 // The same runner for long polynomials: reduce() by streams, the warp's stream table in dynamic shared memory.
@@ -833,11 +855,11 @@ __global__ void __launch_bounds__(BB_THREADS, BB_MIN_BLOCKS) k_run(const __grid_
 #ifndef BBS_MIN_CTAS
 #define BBS_MIN_CTAS 2
 #endif
-template <int NV>
+template <int NV, bool EXPORT = false>
 __global__ void __launch_bounds__(BBS_WARPS * 32, BBS_MIN_CTAS) k_run_streams(const __grid_constant__ BBParams P,
                                                                              const __grid_constant__ BBParams S,
                                                                              const __grid_constant__ BBRunArgs A) {
-  run_worker<NV, true, BBS_WARPS>(P, S, A);
+  run_worker<NV, true, BBS_WARPS, EXPORT>(P, S, A);
 }
 
 // block-strided copy of n 32-bit words
@@ -935,6 +957,7 @@ __global__ void __launch_bounds__(BBW_THREADS, BBW_MIN_CTAS) k_run_wide(const __
           status = BB_STATUS_OVERFLOW_SCRATCH;
         }
       }
+      if (A.gb_sink.lens_dev || A.basis_sink.lens_dev) warp_export_episode<NV>(P, A, slot, ep, status);
       if (tid == 0) {
         const unsigned long long th = acc.th; const double ret = acc.ret;
         bb_episode_stats o;
@@ -1146,6 +1169,7 @@ struct BBLaunch {
     done = true;
     const int pct = 7;   // -> the 16 KB split: three runner CTAs use ~6.5 KB of it
     cudaFuncSetAttribute(k_run<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+    cudaFuncSetAttribute(k_run<NV, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_prepare<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_prepare_lanes<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_order<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
@@ -1162,7 +1186,8 @@ struct BBLaunch {
   }
   static cudaError_t run(const BBParams& P, const BBParams& S, const BBRunArgs& A, int nwarps, cudaStream_t s) {
     same_carveout();
-    k_run<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+    if (A.gb_sink.lens_dev || A.basis_sink.lens_dev) k_run<NV, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+    else k_run<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
     return cudaGetLastError();
   }
   static size_t streams_smem() { return 0; }   // every stream lives in registers (bb_rstreams.cuh)
@@ -1175,9 +1200,12 @@ struct BBLaunch {
   }
   static cudaError_t run_streams(const BBParams& P, const BBParams& S, const BBRunArgs& A, int nwarps, cudaStream_t s) {
     const size_t sm = streams_smem();
-    cudaError_t e = cudaFuncSetAttribute(k_run_streams<NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    const bool ex = A.gb_sink.lens_dev || A.basis_sink.lens_dev;
+    cudaError_t e = cudaFuncSetAttribute(ex ? k_run_streams<NV, true> : k_run_streams<NV>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     if (e != cudaSuccess) return e;
-    k_run_streams<NV><<<(nwarps + BBS_WARPS - 1) / BBS_WARPS, BBS_WARPS * 32, sm, s>>>(P, S, A);
+    if (ex) k_run_streams<NV, true><<<(nwarps + BBS_WARPS - 1) / BBS_WARPS, BBS_WARPS * 32, sm, s>>>(P, S, A);
+    else k_run_streams<NV><<<(nwarps + BBS_WARPS - 1) / BBS_WARPS, BBS_WARPS * 32, sm, s>>>(P, S, A);
     return cudaGetLastError();
   }
   static int wide_ctas_per_sm() {

@@ -1032,15 +1032,35 @@ int bb_prepare(bb_handle* h, int episodes, int seed_base, const int32_t* seeds_d
   return 0;
 }
 
+static int check_sink(bb_handle* h, const bb_poly_sink* k, const char* which) {
+  if (!k) return 0;
+  if (!k->lens_dev || !k->exps_dev || !k->coefs_dev || !k->where_dev || !k->used_dev)
+    return fail(h, std::string("bb_run_export: the ") + which + " sink has a NULL buffer");
+  if (k->cap_polys < 0 || k->cap_terms < 0)
+    return fail(h, std::string("bb_run_export: the ") + which + " sink has a negative capacity");
+  return 0;
+}
+
 int bb_run(bb_handle* h, int strategy, int episodes, int seed_base, const int32_t* seeds_dev, int sel_seed_base,
            int max_steps, double gamma, int compute_gb, bb_episode_stats* stats_dev, int32_t* trace_dev,
            int trace_episodes, int trace_cap, void* stream) {
+  return bb_run_export(h, strategy, episodes, seed_base, seeds_dev, sel_seed_base, max_steps, gamma, compute_gb, stats_dev,
+                       trace_dev, trace_episodes, trace_cap, stream, nullptr, nullptr);
+}
+
+int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const int32_t* seeds_dev, int sel_seed_base,
+                  int max_steps, double gamma, int compute_gb, bb_episode_stats* stats_dev, int32_t* trace_dev,
+                  int trace_episodes, int trace_cap, void* stream, const bb_poly_sink* gb, const bb_poly_sink* basis) {
   if (!h) return -1;
   if ((unsigned)strategy > 8u || episodes < 0 || !stats_dev) return fail(h, "bb_run: bad argument");
+  if (gb && !compute_gb) return fail(h, "bb_run_export: a gb sink needs compute_gb != 0");
+  int rc = check_sink(h, gb, "gb");
+  if (rc == 0) rc = check_sink(h, basis, "basis");
+  if (rc < 0) return rc;
   ENTER(h);
   cudaStream_t s = (cudaStream_t)stream;
   if (episodes == 0) return 0;
-  int rc = check_staged(h, "bb_run");
+  rc = check_staged(h, "bb_run");
   if (rc < 0) return rc;
   // long polynomials (general capacities): reduce() by streams (bb_streams.cuh), by default with one CTA per
   // environment (bb_wide.cuh: the shortest chain of additions); mode 4: one warp per environment
@@ -1119,6 +1139,9 @@ int bb_run(bb_handle* h, int strategy, int episodes, int seed_base, const int32_
     if (h->timing) CK(cudaEventRecord(h->ev_t[1], s));
   }
   if (nbatch > 1) CK(cudaEventRecord(h->ev_entry, s));   // seeds_dev and the ideals are valid on the side stream from here on
+  // where = (-1, -1) for every episode; the runners overwrite it for the episodes they store
+  for (const bb_poly_sink* k : {gb, basis})
+    if (k) CK(cudaMemsetAsync(k->where_dev, 0xff, sizeof(int64_t) * 2 * (size_t)episodes, s));
   for (int bi = 0; bi < nbatch; bi++) {
     const int base = bi * BB_RUN_BATCH, count = std::min(BB_RUN_BATCH, episodes - base);
     int next = -1;
@@ -1136,6 +1159,8 @@ int bb_run(bb_handle* h, int strategy, int episodes, int seed_base, const int32_
     prepare_args(h, which, base, count, seed_base, seeds_dev, A);
     A.strategy = strategy; A.sel_seed_base = sel_seed_base; A.sel_seed_stride = h->sel_seed_stride;
     A.max_steps = max_steps; A.gamma = gamma; A.compute_gb = compute_gb; A.out = stats_dev;
+    if (gb) A.gb_sink = *gb;
+    if (basis) A.basis_sink = *basis;
     A.trace = trace_dev; A.trace_eps = trace_dev ? trace_episodes : 0; A.trace_cap = trace_cap;
     A.stream_kmax = (h->wide_mode == 2 || h->wide_mode == 5) ? 6 : ((h->wide_mode == 3 || h->wide_mode == 6) ? 48 : BBS_KMAX);
     A.stream_regs = h->wide_mode == 7 ? 8 : A.stream_kmax;
