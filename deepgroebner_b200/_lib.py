@@ -63,7 +63,7 @@ EXPORTS = [
     "bb_abi_version", "bb_resident_envs", "bb_create", "bb_destroy", "bb_last_error", "bb_cols", "bb_num_envs", "bb_sm_count",
     "bb_set_distribution", "bb_set_distribution_poly", "bb_seed", "bb_set_ideals", "bb_reset", "bb_step", "bb_select", "bb_observe", "bb_pairs",
     "bb_status", "bb_stats", "bb_run", "bb_download_basis", "bb_final_gb", "bb_counters_read", "bb_hash_item",
-    "bb_seed_selection", "bb_value", "bb_copy_env", "bb_set_auto_reset", "bb_step_observe", "bb_step_host", "bb_reset_host", "bb_observe_host", "bb_set_wide", "bb_set_prepare_mode", "bb_set_selection_seed_stride", "bb_policy_pmlp", "bb_rollout",
+    "bb_seed_selection", "bb_value", "bb_copy_env", "bb_set_auto_reset", "bb_step_observe", "bb_step_host", "bb_reset_host", "bb_observe_host", "bb_set_wide", "bb_set_prepare_mode", "bb_set_two_term", "bb_set_selection_seed_stride", "bb_policy_pmlp", "bb_rollout",
     "bb_seed_on", "bb_prepare", "bb_set_episode_offset", "bb_set_timing", "bb_last_run_ms", "bb_set_max_episode_length",
     "bb_set_compaction", "bb_compact", "bb_status_summary", "bb_set_obs_nvars", "bb_discount", "bb_set_serve", "bb_set_prefetch",
     "bb_run_export",
@@ -144,6 +144,8 @@ def load():
     lib.bb_set_wide.argtypes = [vp, i]
     lib.bb_set_prepare_mode.restype = i
     lib.bb_set_prepare_mode.argtypes = [vp, i]
+    lib.bb_set_two_term.restype = i
+    lib.bb_set_two_term.argtypes = [vp, i]
     lib.bb_set_selection_seed_stride.restype = i
     lib.bb_set_selection_seed_stride.argtypes = [vp, i]
     lib.bb_seed_on.restype = i

@@ -536,6 +536,11 @@ class BuchbergerEngine:
         (default) or always one warp per episode.  Results are identical; only speed differs."""
         self._ck(self.lib.bb_set_prepare_mode(self.h, int(bool(by_warp))), "bb_set_prepare_mode")
 
+    def set_two_term(self, on=True):
+        """Runner of run_episodes for binomial distributions (bb_set_two_term): True (default) the two-term runner, False the
+        general one.  Both give bit-identical results; the switch exists to compare them."""
+        self._ck(self.lib.bb_set_two_term(self.h, int(bool(on))), "bb_set_two_term")
+
     def set_selection_seed_stride(self, stride=1):
         """run_episodes seeds episode e's 'random' selection stream with selection_seed + e * stride
         (0: one seed for every episode, as scripts/make_strat.cpp does)."""

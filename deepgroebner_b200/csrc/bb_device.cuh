@@ -329,6 +329,15 @@ __device__ __forceinline__ void tiny_merge(const BBField& F, bool hasA, uint64_t
   else o.n = 0;
 }
 
+// The remainder of a reduction in the two-term instantiations (TWO): at most two terms, warp-uniform registers, ascending
+// key order.  In a binomial ideal every polynomial has at most two terms (DESIGN.md §3): the lead terms of an S-polynomial
+// and of every reduction step cancel, leaving the two tails, and once a term has moved to the remainder the dividend has at
+// most one term left.
+struct Rem2 {
+  uint64_t k0, k1;
+  uint32_t c0, c1;
+};
+
 // h <- the n-term list a general merge left at the start of scratch half `buf`
 __device__ __forceinline__ void dividend_from_scratch(const BBParams& P, const Env& e, Dividend& h, int n, int buf) {
   const uint64_t* hk = ENV_PTR(uint64_t, e, P, o_hkey) + (size_t)buf * P.max_poly_terms;
@@ -346,11 +355,13 @@ __device__ __forceinline__ void dividend_from_scratch(const BBParams& P, const E
 // `sorted`: the reducer list is ascending in lead monomial, so the scan may stop at the first reducer whose lead
 // monomial exceeds LM(h) (it and everything after it cannot divide); the count of examined lead monomials that
 // feeds the traffic model stays the reference's (found + 1, or all of them).
-template <int NV>
+// TWO: h and every reducer have at most two terms.  Only the register merge runs, and the remainder goes to *rem instead of
+// (rk, rc), which stay untouched (the caller's update() writes it to the term arena); rcap still bounds its length.
+template <int NV, bool TWO = false>
 __device__ __forceinline__ int warp_reduce(const BBParams& P, Env& e, Dividend& h, const uint64_t* __restrict__ rlm,
                                            const uint32_t* __restrict__ ridx, int nR, bool sorted,
                                            uint64_t* __restrict__ rk, uint32_t* __restrict__ rc, int rcap, int& steps,
-                                           Ctr& ct) {
+                                           Ctr& ct, Rem2* rem = nullptr) {
   typedef KL<NV> K;
   const BBField F = P.F;
   const int lane = bb_lane();
@@ -381,13 +392,13 @@ __device__ __forceinline__ int warp_reduce(const BBParams& P, Env& e, Dividend& 
         h.sug = sf > h.sug ? sf : h.sug;
       }
       ct.tread += (unsigned)h.n + f.len;
-      if (h.n <= 2 && f.len <= 2) {
+      if (TWO || (h.n <= 2 && f.len <= 2)) {
         const uint64_t kb = f.k1 + adj;
         const bool hasB = f.len == 2;
         if (hasB) e.guard |= kb;
         tiny_merge(F, h.n == 2, h.k1, h.c1, hasB, kb, bbf_mulmod(F, f.c1, nc), h);
         if (e.guard & K::g_all) return -3;  // garbage keys could otherwise keep the loop alive
-      } else {
+      } else if constexpr (!TWO) {
         uint64_t* hk = ENV_PTR(uint64_t, e, P, o_hkey);
         uint32_t* hc = ENV_PTR(uint32_t, e, P, o_hcoef);
         if (h.loc < 0) {  // the register-resident dividend (n <= 2) goes to scratch half 0; only its tail is read
@@ -408,19 +419,26 @@ __device__ __forceinline__ int warp_reduce(const BBParams& P, Env& e, Dividend& 
       steps++;
     } else {
       if (rlen >= rcap) return -2;
-      if (lane == 0) { rk[rlen] = lead; rc[rlen] = h.c0; }
+      if constexpr (TWO) {
+        if (rlen == 0) { rem->k0 = lead; rem->c0 = h.c0; }
+        else { rem->k1 = lead; rem->c1 = h.c0; }
+      } else {
+        if (lane == 0) { rk[rlen] = lead; rc[rlen] = h.c0; }
+      }
       rlen++;
       ct.moves++;
       h.n--; h.k0 = h.k1; h.c0 = h.c1;  // drop the lead term
-      if (h.loc >= 0) {
-        h.loc++;
-        if (h.n > 1) {
-          h.k1 = ENV_PTR(uint64_t, e, P, o_hkey)[h.loc + 1]; h.c1 = ENV_PTR(uint32_t, e, P, o_hcoef)[h.loc + 1];
+      if constexpr (!TWO) {
+        if (h.loc >= 0) {
+          h.loc++;
+          if (h.n > 1) {
+            h.k1 = ENV_PTR(uint64_t, e, P, o_hkey)[h.loc + 1]; h.c1 = ENV_PTR(uint32_t, e, P, o_hcoef)[h.loc + 1];
+          }
         }
       }
     }
   }
-  __syncwarp();
+  if constexpr (!TWO) __syncwarp();
   return rlen;
 }
 
@@ -468,18 +486,20 @@ __device__ __forceinline__ void hot_init(const BBParams&) {}
 // Every pair carries the key of its lcm (plcm), so step (1) and the selection strategies read one array.
 // One out-of-line copy shared by step and reset.  Returns (emitted << 32) | new |P|, or -1 on pair-list overflow /
 // -2 when the basis is full / -3 when an lcm's degree does not fit the packed layout; the caller bumps nG and nT.
-template <int NV>
-__device__ BB_ADD_BASIS_INLINE long long warp_add_basis(const BBParams& P, unsigned char* base, int m, int nP, int off, int len,
-                                                 int sug) {
+// TWO: the polynomial (len <= 2 terms: lead key fk, coefficient c0, second term (k1, c1)) comes in registers and is written
+// to arena[off, off+len) here, so update() starts without a dependent load.
+template <int NV, bool TWO>
+__device__ __forceinline__ long long add_basis_body(const BBParams& P, unsigned char* base, int m, int nP, int off, int len,
+                                                    int sug, uint64_t fk, uint64_t k1, uint32_t c0, uint32_t c1) {
   typedef KL<NV> K;
   const auto& H = BB_HOT(P);
   const int lane = bb_lane();
   const uint32_t ltm = bb_lt_mask();
   if (m >= H.max_basis) return -2;
   base = bb_global(base);
-  const uint64_t* tk = reinterpret_cast<const uint64_t*>(base + H.o_tkey) + off;
-  const uint32_t* tc = reinterpret_cast<const uint32_t*>(base + H.o_tcoef) + off;
-  const uint64_t fk = tk[0];
+  uint64_t* tk = reinterpret_cast<uint64_t*>(base + H.o_tkey) + off;
+  uint32_t* tc = reinterpret_cast<uint32_t*>(base + H.o_tcoef) + off;
+  if constexpr (!TWO) fk = tk[0];
   uint64_t* lm = reinterpret_cast<uint64_t*>(base + H.o_lm);
   uint64_t* lscr = reinterpret_cast<uint64_t*>(base + H.o_lscr);
   uint64_t* plcm = reinterpret_cast<uint64_t*>(base + H.o_plcm);
@@ -723,14 +743,33 @@ __device__ BB_ADD_BASIS_INLINE long long warp_add_basis(const BBParams& P, unsig
     rlm[pos] = fk; ridx[pos] = (uint32_t)m;
     lm[m] = fk;
     GHeadMem* g = reinterpret_cast<GHeadMem*>(base + H.o_ghead) + m;
-    const uint32_t inv = bb_global(H.invtab)[tc[0]];  // 1/LC: one table load instead of a 15-step power ladder
-    const uint64_t k1 = len > 1 ? tk[1] : 0ull;
-    const uint32_t c1 = len > 1 ? tc[1] : 0u;
+    if constexpr (TWO) {
+      tk[0] = fk; tc[0] = c0;
+      if (len > 1) { tk[1] = k1; tc[1] = c1; }
+      else { k1 = 0ull; c1 = 0u; }
+    }
+    const uint32_t inv = bb_global(H.invtab)[TWO ? c0 : tc[0]];  // 1/LC: one table load instead of a 15-step power ladder
+    if constexpr (!TWO) {
+      k1 = len > 1 ? tk[1] : 0ull;
+      c1 = len > 1 ? tc[1] : 0u;
+    }
     reinterpret_cast<uint4*>(g)[0] = make_uint4((uint32_t)fk, (uint32_t)(fk >> 32), (uint32_t)k1, (uint32_t)(k1 >> 32));
     reinterpret_cast<uint4*>(g)[1] = make_uint4(inv | (c1 << 16), (uint32_t)sug, (uint32_t)off, (uint32_t)len);
   }
   __syncwarp();
   return ((long long)emitted << 32) | (long long)nP;
+}
+// the polynomial already sits at arena[off, off+len)
+template <int NV>
+__device__ BB_ADD_BASIS_INLINE long long warp_add_basis(const BBParams& P, unsigned char* base, int m, int nP, int off, int len,
+                                                        int sug) {
+  return add_basis_body<NV, false>(P, base, m, nP, off, len, sug, 0ull, 0ull, 0u, 0u);
+}
+// two-term instantiation: the polynomial in registers, see add_basis_body
+template <int NV>
+__device__ BB_ADD_BASIS_INLINE long long warp_add_basis(const BBParams& P, unsigned char* base, int m, int nP, int off, int len,
+                                                        int sug, uint64_t fk, uint64_t k1, uint32_t c0, uint32_t c1) {
+  return add_basis_body<NV, true>(P, base, m, nP, off, len, sug, fk, k1, c0, c1);
 }
 
 // ---------------------------------------------------------------------------------------------------- step
@@ -759,7 +798,9 @@ __device__ __forceinline__ void warp_take_pair(const BBParams& P, Env& e, int ro
 // :318-329): erase the pair, s = spoly(G[i], G[j]) (:18-21), (r, steps) = reduce(s, G_), if r != 0 update + sorted
 // insert.  Returns the number of polynomial additions 1 + steps (reward = -(1+steps) under Additions, -1 under
 // Reductions).  `pair` receives (j << 16) | i, or 0xffffffff for a bad action.
-template <int NV>
+// TWO: every polynomial of the environment has at most two terms (binomial ideals): no general merge, no scratch, and the
+// remainder reaches update() in registers.  Same results and counters as the general instantiation.
+template <int NV, bool TWO = false>
 __device__ __forceinline__ int warp_step(const BBParams& P, Env& e, int row, uint32_t& pair, Ctr& ct) {
   typedef KL<NV> K;
   const BBField F = P.F;
@@ -782,13 +823,13 @@ __device__ __forceinline__ int warp_step(const BBParams& P, Env& e, int row, uin
   }
   const uint64_t adjf = gam - hf.lm, adjg = gam - hg.lm;
   const uint32_t cg = F.p - hg.invlc;  // -(1/LC g), invlc != 0
-  if (hf.len <= 2 && hg.len <= 2) {
+  if (TWO || (hf.len <= 2 && hg.len <= 2)) {
     const uint64_t ka = hf.k1 + adjf, kb = hg.k1 + adjg;
     const bool hasA = hf.len == 2, hasB = hg.len == 2;
     if (hasA) e.guard |= ka;
     if (hasB) e.guard |= kb;
     tiny_merge(F, hasA, ka, bbf_mulmod(F, hf.c1, hf.invlc), hasB, kb, bbf_mulmod(F, hg.c1, cg), h);
-  } else {
+  } else if constexpr (!TWO) {
     const uint64_t* tk = ENV_PTR(uint64_t, e, P, o_tkey);
     const uint32_t* tc = ENV_PTR(uint32_t, e, P, o_tcoef);
     const int n = warp_merge<NV>(F, tk + hf.off + 1, tc + hf.off + 1, (int)hf.len - 1, hf.invlc, adjf, tk + hg.off + 1,
@@ -801,16 +842,19 @@ __device__ __forceinline__ int warp_step(const BBParams& P, Env& e, int row, uin
   if (e.guard & K::g_all) { e.status = BB_STATUS_OVERFLOW_EXPONENT; return 1; }
   ct.twrite += (unsigned)h.n;
   int steps = 0;
-  const int rlen = warp_reduce<NV>(P, e, h, ENV_PTR(uint64_t, e, P, o_rlm), ENV_PTR(uint32_t, e, P, o_ridx), e.nG,
-                                   P.sort_reducers != 0, ENV_PTR(uint64_t, e, P, o_tkey) + e.nT,
-                                   ENV_PTR(uint32_t, e, P, o_tcoef) + e.nT, P.max_terms - e.nT, steps, ct);
+  Rem2 rem;
+  const int rlen = warp_reduce<NV, TWO>(P, e, h, ENV_PTR(uint64_t, e, P, o_rlm), ENV_PTR(uint32_t, e, P, o_ridx), e.nG,
+                                        P.sort_reducers != 0, ENV_PTR(uint64_t, e, P, o_tkey) + e.nT,
+                                        ENV_PTR(uint32_t, e, P, o_tcoef) + e.nT, P.max_terms - e.nT, steps, ct, &rem);
   if (rlen < 0 || (e.guard & K::g_all)) {   // one test on the hot path; which fault it was is sorted out here
     e.status = rlen == -1 ? BB_STATUS_OVERFLOW_SCRATCH : (rlen == -2 ? BB_STATUS_OVERFLOW_TERMS : BB_STATUS_OVERFLOW_EXPONENT);
     return 1 + steps;
   }
   if (rlen > 0) {
     ct.upb += (unsigned)e.nG; ct.upp += (unsigned)e.nP;
-    const long long r = warp_add_basis<NV>(P, e.base, e.nG, e.nP, e.nT, rlen, h.sug);
+    long long r;
+    if constexpr (TWO) r = warp_add_basis<NV>(P, e.base, e.nG, e.nP, e.nT, rlen, h.sug, rem.k0, rem.k1, rem.c0, rem.c1);
+    else r = warp_add_basis<NV>(P, e.base, e.nG, e.nP, e.nT, rlen, h.sug);
     if (r < 0) {
       e.status = (r == -1) ? BB_STATUS_OVERFLOW_PAIRS : (r == -2 ? BB_STATUS_OVERFLOW_BASIS : BB_STATUS_OVERFLOW_EXPONENT);
       return 1 + steps;

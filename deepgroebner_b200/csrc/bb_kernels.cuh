@@ -54,6 +54,7 @@ struct BBRunArgs {
   int* queue;        // [0]: next queue position; [BB_LPT_HIST .. +BB_LPT_BUCKETS): histogram of the cost keys of the batch, then as many cursors
   int* order;        // [episodes] queue position -> episode of the batch, longest predicted first (k_order)
   uint8_t* cost_key; // [episodes] predicted-cost bucket of each episode of the batch (k_prepare)
+  int two_term;      // k_run: every polynomial has at most two terms (binomial ideals): the two-term instantiation
 };
 #define BB_LPT_BUCKETS 256
 #define BB_LPT_HIST 4
@@ -713,8 +714,8 @@ __global__ void __launch_bounds__(BB_PREP_THREADS, BB_PREP_MIN_BLOCKS) k_prefill
 
 // The loop of buchberger() (buchberger.cpp:243-263) on one environment: select, step, accumulate the trace checksum and
 // the discounted return (discounted_return += discount * reward; discount *= gamma, :250-251) until P is empty.
-// STREAMS: reduce() by streams (bb_streams.cuh), ws / st = the warp's stream state and table.
-template <int NV, bool STREAMS>
+// STREAMS: reduce() by streams (bb_streams.cuh), ws / st = the warp's stream state and table.  TWO: see warp_step.
+template <int NV, bool STREAMS, bool TWO = false>
 __device__ __forceinline__ void run_episode(const BBParams& P, Env& e, int strategy, int max_steps, double gamma,
                                             BBEpisodeAcc& acc, Ctr& ct, int& steps, int& adds, int4* trace, int trace_cap,
                                             RegStreams* ws) {
@@ -724,7 +725,7 @@ __device__ __forceinline__ void run_episode(const BBParams& P, Env& e, int strat
     uint32_t pr;
     int a;
     if (STREAMS) a = warp_step_rstreams<NV>(P, e, *ws, prow, pr, ct);
-    else a = warp_step<NV>(P, e, prow, pr, ct);
+    else a = warp_step<NV, TWO>(P, e, prow, pr, ct);
     if (lane == 0) {
       const int pi = pr & 0xffffu, pj = pr >> 16;
       acc.th = trace_hash_step(acc.th, pr, a);
@@ -759,8 +760,8 @@ __device__ __noinline__ void warp_export_episode(const BBParams& P, const BBRunA
 // prepared initial state from the staging arena, select/step until P is empty (or max_steps), write the episode
 // record, repeat.  WARPS = warps per CTA.  EXPORT: bb_run_export's sinks may be attached (an instantiation of its own, so
 // the runner without sinks keeps the parent's code: k_run is issue- and instruction-footprint-bound, and the one extra call
-// site in its loop measured 3 % on configs[1]).
-template <int NV, bool STREAMS, int WARPS, bool EXPORT>
+// site in its loop measured 3 % on configs[1]).  TWO: the two-term step (warp_step), for runs whose ideals are binomial.
+template <int NV, bool STREAMS, int WARPS, bool EXPORT, bool TWO = false>
 __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S, const BBRunArgs& A) {
   __shared__ unsigned long long sh[WARPS][CT_COUNT];
   __shared__ BBEpisodeAcc acc_sh[WARPS];  // per-episode accumulators only lane 0 touches: kept out of registers
@@ -792,7 +793,7 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
       int steps = 0, adds = 0;
       if (lane == 0) { acc.th = 0ull; acc.ret = 0.0; acc.disc = 1.0; acc.sel_rng = rng_seed(A.sel_seed_base + (A.ep_offset + ep) * A.sel_seed_stride); }
       __syncwarp();
-      run_episode<NV, STREAMS>(P, e, A.strategy, A.max_steps, A.gamma, acc, ct, steps, adds,
+      run_episode<NV, STREAMS, TWO>(P, e, A.strategy, A.max_steps, A.gamma, acc, ct, steps, adds,
                                (A.trace && ep < A.trace_eps) ? reinterpret_cast<int4*>(A.trace) + (size_t)ep * A.trace_cap : nullptr,
                                A.trace_cap, &ws);
       const int nonzero = e.nG - g_start, zero = steps - nonzero;
@@ -841,11 +842,11 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
   }
 }
 
-template <int NV, bool EXPORT = false>
+template <int NV, bool EXPORT = false, bool TWO = false>
 __global__ void __launch_bounds__(BB_THREADS, BB_MIN_BLOCKS) k_run(const __grid_constant__ BBParams P,
                                                                   const __grid_constant__ BBParams S,
                                                                   const __grid_constant__ BBRunArgs A) {
-  run_worker<NV, false, BB_WARPS, EXPORT>(P, S, A);
+  run_worker<NV, false, BB_WARPS, EXPORT, TWO>(P, S, A);
 }
 
 // The same runner for long polynomials: reduce() by streams, the warp's stream table in dynamic shared memory.
@@ -1170,6 +1171,8 @@ struct BBLaunch {
     const int pct = 7;   // -> the 16 KB split: three runner CTAs use ~6.5 KB of it
     cudaFuncSetAttribute(k_run<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_run<NV, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+    cudaFuncSetAttribute(k_run<NV, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+    cudaFuncSetAttribute(k_run<NV, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_prepare<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_prepare_lanes<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_order<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
@@ -1186,8 +1189,14 @@ struct BBLaunch {
   }
   static cudaError_t run(const BBParams& P, const BBParams& S, const BBRunArgs& A, int nwarps, cudaStream_t s) {
     same_carveout();
-    if (A.gb_sink.lens_dev || A.basis_sink.lens_dev) k_run<NV, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
-    else k_run<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+    const bool ex = A.gb_sink.lens_dev || A.basis_sink.lens_dev;
+    if (A.two_term) {
+      if (ex) k_run<NV, true, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+      else k_run<NV, false, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+    } else {
+      if (ex) k_run<NV, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+      else k_run<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+    }
     return cudaGetLastError();
   }
   static size_t streams_smem() { return 0; }   // every stream lives in registers (bb_rstreams.cuh)

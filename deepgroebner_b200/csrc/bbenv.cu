@@ -226,6 +226,7 @@ struct bb_handle {
   unsigned serve_seq;
   cudaStream_t serve_stream; cudaEvent_t ev_serve;
   int prepare_by_warp;   // bb_run: 1 = episode preparation by one warp per episode even where the thread-per-episode kernel applies
+  int two_term;    // bb_run: 1 = the two-term runner for binomial distributions (default), 0 = always the general one
   int wide_mode;   // bb_run: reduce() by streams: -1 = when the capacities ask for long polynomials, 0 = never, 1 = always, 2 / 3 = always, small tables
   // host mirrors of the distribution tables
   std::vector<double> cp;
@@ -519,6 +520,7 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
   h->fork_cap = 0; h->fork_arena = nullptr; h->fork_st = nullptr;
   h->wide_mode = -1;
   h->prepare_by_warp = 0;
+  h->two_term = 1;
   h->host_stage = nullptr; h->dev_stage = nullptr; h->stage_bytes = 0;
   h->sel_seed_stride = 1;
   auto bail = [&](int code) { g_create_err = h->err; bb_destroy(h); return code; };
@@ -1165,6 +1167,9 @@ int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const
     A.stream_kmax = (h->wide_mode == 2 || h->wide_mode == 5) ? 6 : ((h->wide_mode == 3 || h->wide_mode == 6) ? 48 : BBS_KMAX);
     A.stream_regs = h->wide_mode == 7 ? 8 : A.stream_kmax;
     A.ctl_reducers = h->wide_mode == 8 ? 32 : 256;
+    // every generator a binomial distribution draws has two terms, so every polynomial of the run has at most two
+    // (DESIGN.md §3).  Staged ideals keep the general runner: nothing records the length of their polynomials.
+    A.two_term = h->two_term && h->P.dist.enabled && h->P.dist.kind == 0;
     if (bi > 0) CK(cudaStreamWaitEvent(s, h->stage[which].prepared, 0));
     const int workers = std::min(h->P.num_envs, count);
     if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) CK(h->K->run_streams(PB, S, A, workers, s));
@@ -1373,6 +1378,12 @@ int bb_set_wide(bb_handle* h, int mode) {
 int bb_set_prepare_mode(bb_handle* h, int by_warp) {
   if (!h) return -1;
   h->prepare_by_warp = by_warp ? 1 : 0;
+  return 0;
+}
+
+int bb_set_two_term(bb_handle* h, int on) {
+  if (!h) return -1;
+  h->two_term = on ? 1 : 0;
   return 0;
 }
 

@@ -290,6 +290,12 @@ int bb_set_selection_seed_stride(bb_handle* h, int stride);
  * performance switch that the tests use to compare the two. */
 int bb_set_prepare_mode(bb_handle* h, int by_warp);
 
+/* bb_set_two_term: which warp runner bb_run uses for binomial distributions (bb_set_distribution), whose polynomials all
+ * have at most two terms.  1 (default): a runner built for that case (register-only arithmetic, the remainder handed to
+ * update() in registers); 0: the general runner.  Both produce bit-identical records, counters and exported polynomials;
+ * this is a performance switch that the tests use to compare the two.  Other ideals always use the general runner. */
+int bb_set_two_term(bb_handle* h, int on);
+
 /* bb_set_wide: how bb_run's episode runner reduces.  0: the dividend is materialised (warp-cooperative merges, built
  * for the 2-term polynomials of binomial ideals); 1: the dividend is a set of streams into the term arena, one round per
  * lead term and O(1) work per addition (built for long polynomials, e.g. cyclic-n), run by one CTA per environment
