@@ -108,7 +108,8 @@ def _ptr(t):
 
 
 def resident_envs(device=0, nvars=3):
-    """Slots of the persistent episode runner that are co-resident on the device (one wave of bb_run)."""
+    """Slots of one resident wave of bb_run's warp runners: the larger of the general and the two-term runner's waves
+    (bb_run launches each with no more warps than its own)."""
     lib = _lib.load()
     n = lib.bb_resident_envs(int(device), int(nvars))
     if n <= 0:

@@ -765,9 +765,11 @@ __device__ BB_ADD_BASIS_INLINE long long warp_add_basis(const BBParams& P, unsig
                                                         int sug) {
   return add_basis_body<NV, false>(P, base, m, nP, off, len, sug, 0ull, 0ull, 0u, 0u);
 }
-// two-term instantiation: the polynomial in registers, see add_basis_body
+// two-term instantiation: the polynomial in registers, see add_basis_body.  Inlined: its one call site is the two-term
+// k_run's warp_step, and without the call's register save / restore that kernel spills 248 instead of 380 bytes at its
+// 64-register cap (profiles/README.md, "Two-term runner at 32 warps per SM")
 template <int NV>
-__device__ BB_ADD_BASIS_INLINE long long warp_add_basis(const BBParams& P, unsigned char* base, int m, int nP, int off, int len,
+__device__ __forceinline__ long long warp_add_basis(const BBParams& P, unsigned char* base, int m, int nP, int off, int len,
                                                         int sug, uint64_t fk, uint64_t k1, uint32_t c0, uint32_t c1) {
   return add_basis_body<NV, true>(P, base, m, nP, off, len, sug, fk, k1, c0, c1);
 }

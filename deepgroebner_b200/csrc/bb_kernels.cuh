@@ -24,7 +24,16 @@
 #endif
 #define BB_THREADS (BB_WARPS * 32)
 #ifndef BB_MIN_BLOCKS
-#define BB_MIN_BLOCKS 3  // register cap 80 -> 24 resident warps per SM (A/B on B200, profiles/README.md v8: 2 -> 702, 3 -> 763, 4 -> 728, 5 -> 693, 6 -> 657 M env-steps/s)
+#define BB_MIN_BLOCKS 3  // register cap 80 -> 24 resident warps per SM: the general k_run (A/B on B200, profiles/README.md v8: 2 -> 702, 3 -> 763, 4 -> 728, 5 -> 693, 6 -> 657 M env-steps/s) and the step kernels
+#endif
+// The two-term k_run (k_run<NV, EXPORT, true>) has launch bounds of its own: it spills far less than the general runner
+// under a lower register cap, so it keeps more warps resident
+// (profiles/README.md, "Two-term runner at 32 warps per SM": 8 x 4 against 8 x 3, 7 x 4, 6 x 5 and 4 x 8).
+#ifndef BB_TWO_WARPS
+#define BB_TWO_WARPS BB_WARPS
+#endif
+#ifndef BB_TWO_MIN_BLOCKS
+#define BB_TWO_MIN_BLOCKS 4  // register cap 64 -> 32 resident warps per SM
 #endif
 
 #ifndef BB_ROLLOUT_MIN_BLOCKS
@@ -148,7 +157,7 @@ struct BBKernelTable {
   cudaError_t (*policy)(const BBParams&, const BBPolicy&, unsigned long long counter, int32_t* actions, float* logp,
                         float* logits, int pmax, int nwarps, cudaStream_t);
   cudaError_t (*rollout)(const BBParams&, const BBRolloutArgs&, int nwarps, cudaStream_t);
-  int (*run_blocks_per_sm)(void);
+  int (*run_warps_per_sm)(int two);   // k_run: general (0) or two-term (1); -1 on error
 };
 
 const BBKernelTable* bb_kernel_table(int nvars);  // bbenv.cu; NULL if nvars is outside 1..8
@@ -843,10 +852,9 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
 }
 
 template <int NV, bool EXPORT = false, bool TWO = false>
-__global__ void __launch_bounds__(BB_THREADS, BB_MIN_BLOCKS) k_run(const __grid_constant__ BBParams P,
-                                                                  const __grid_constant__ BBParams S,
-                                                                  const __grid_constant__ BBRunArgs A) {
-  run_worker<NV, false, BB_WARPS, EXPORT, TWO>(P, S, A);
+__global__ void __launch_bounds__(TWO ? BB_TWO_WARPS * 32 : BB_THREADS, TWO ? BB_TWO_MIN_BLOCKS : BB_MIN_BLOCKS)
+k_run(const __grid_constant__ BBParams P, const __grid_constant__ BBParams S, const __grid_constant__ BBRunArgs A) {
+  run_worker<NV, false, TWO ? BB_TWO_WARPS : BB_WARPS, EXPORT, TWO>(P, S, A);
 }
 
 // The same runner for long polynomials: reduce() by streams, the warp's stream table in dynamic shared memory.
@@ -1168,7 +1176,10 @@ struct BBLaunch {
     static bool done = false;
     if (done) return;
     done = true;
-    const int pct = 7;   // -> the 16 KB split: three runner CTAs use ~6.5 KB of it
+    // -> the 16 KB split: three general runner CTAs use ~6.5 KB of it (run_worker's arrays and the 1 KB reserved per CTA)
+    const int pct = 7;
+    static_assert(BB_TWO_MIN_BLOCKS * (BB_TWO_WARPS * (CT_COUNT * 8 + sizeof(BBEpisodeAcc)) + 1024) <= 16 * 1024,
+                  "the 16 KB split holds BB_TWO_MIN_BLOCKS two-term runner CTAs");
     cudaFuncSetAttribute(k_run<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_run<NV, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_run<NV, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
@@ -1191,8 +1202,9 @@ struct BBLaunch {
     same_carveout();
     const bool ex = A.gb_sink.lens_dev || A.basis_sink.lens_dev;
     if (A.two_term) {
-      if (ex) k_run<NV, true, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
-      else k_run<NV, false, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
+      const int g = (nwarps + BB_TWO_WARPS - 1) / BB_TWO_WARPS;
+      if (ex) k_run<NV, true, true><<<g, BB_TWO_WARPS * 32, 0, s>>>(P, S, A);
+      else k_run<NV, false, true><<<g, BB_TWO_WARPS * 32, 0, s>>>(P, S, A);
     } else {
       if (ex) k_run<NV, true><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
       else k_run<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, S, A);
@@ -1278,16 +1290,20 @@ struct BBLaunch {
     }
     return cudaErrorInvalidValue;
   }
-  static int run_blocks_per_sm() {
+  // resident warps per SM of the general (two == 0) or the two-term k_run (the instantiations with sinks have the same bounds)
+  static int run_warps_per_sm(int two) {
+    same_carveout();
     int blocks = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run<NV>, BB_THREADS, 0) != cudaSuccess) return -1;
-    return blocks;
+    const cudaError_t e = two ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run<NV, false, true>, BB_TWO_WARPS * 32, 0)
+                              : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run<NV>, BB_THREADS, 0);
+    if (e != cudaSuccess) return -1;
+    return blocks * (two ? BB_TWO_WARPS : BB_WARPS);
   }
   static const BBKernelTable* table() {
     static const BBKernelTable t = {NV, KL<NV>::w, KL<NV>::dw, KL<NV>::dshift, KL<NV>::eshift,
                                     &reset, &step, &step_obs, &serve, &prefill, &select, &observe, &final_gb, &prepare, &run, &run_streams, &streams_warps_per_sm, &run_wide, &wide_ctas_per_sm, &value, &policy,
                                     &rollout,
-                                    &run_blocks_per_sm};
+                                    &run_warps_per_sm};
     return &t;
   }
 };

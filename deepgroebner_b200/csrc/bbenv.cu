@@ -227,6 +227,7 @@ struct bb_handle {
   cudaStream_t serve_stream; cudaEvent_t ev_serve;
   int prepare_by_warp;   // bb_run: 1 = episode preparation by one warp per episode even where the thread-per-episode kernel applies
   int two_term;    // bb_run: 1 = the two-term runner for binomial distributions (default), 0 = always the general one
+  int run_wave[2];  // resident warps of the general (0) and the two-term (1) k_run on the device: the most either launches
   int wide_mode;   // bb_run: reduce() by streams: -1 = when the capacities ask for long polynomials, 0 = never, 1 = always, 2 / 3 = always, small tables
   // host mirrors of the distribution tables
   std::vector<double> cp;
@@ -449,9 +450,11 @@ int bb_resident_envs(int device, int nvars) {
   if (!K) return -1;
   if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) return -1;
   if (cudaSetDevice(device) != cudaSuccess) return -1;
-  const int blocks = K->run_blocks_per_sm();
-  if (blocks <= 0) return -1;
-  return sms * blocks * BB_WARPS;
+  // the larger wave of the two warp runners: a handle of this many slots keeps either of them fully resident, and bb_run
+  // launches the other with no more warps than its own wave
+  const int w0 = K->run_warps_per_sm(0), w1 = K->run_warps_per_sm(1);
+  if (w0 <= 0 || w1 <= 0) return -1;
+  return sms * std::max(w0, w1);
 }
 
 void bb_destroy(bb_handle* h) {
@@ -539,6 +542,11 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
   h->K = bb_kernel_table(cfg->nvars);
   if (!h->K || h->K->w != h->L.w || h->K->dw != h->L.dw || h->K->dshift != h->L.dshift || h->K->eshift != h->L.eshift) {
     h->err = "bb_create: kernel table / layout mismatch"; return bail(-6);
+  }
+  for (int two = 0; two < 2; two++) {
+    const int w = h->K->run_warps_per_sm(two);
+    if (w <= 0) { h->err = "bb_create: k_run does not fit on the device"; return bail(-2); }
+    h->run_wave[two] = w * h->sm_count;
   }
   P.F.p = h->L.p; P.F.mu = h->L.mu; P.nvars = cfg->nvars;
   P.num_envs = cfg->num_envs; P.k = cfg->k; P.cols = 2 * cfg->nvars * cfg->k;
@@ -1174,7 +1182,7 @@ int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const
     const int workers = std::min(h->P.num_envs, count);
     if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) CK(h->K->run_streams(PB, S, A, workers, s));
     else if (streams) CK(h->K->run_wide(PB, S, A, std::min(workers, wide_ctas), s));
-    else CK(h->K->run(PB, S, A, workers, s));
+    else CK(h->K->run(PB, S, A, std::min(workers, h->run_wave[A.two_term]), s));
     CK(cudaEventRecord(h->stage[which].consumed, s));
     CK(cudaEventRecord(h->bank[bk].done, s));
     if (h->timing && bi == 0) CK(cudaEventRecord(h->ev_t[2], s));
@@ -1243,7 +1251,7 @@ int bb_value(bb_handle* h, int strategy, double gamma, int rollouts, int sel_see
   const long long ntasks = (long long)N * rollouts;
   if (ntasks > 0x7fffffffLL) return fail(h, "bb_value: too many rollouts");
   // workers: one resident wave at most, and at most 8 GiB of fork arena
-  int workers = h->K->run_blocks_per_sm() * h->sm_count * BB_WARPS;
+  int workers = h->run_wave[0];   // k_value has the general k_run's launch bounds
   const long long by_mem = (long long)(((size_t)8 << 30) / h->P.slot_stride);
   workers = (int)std::max(1LL, std::min((long long)workers, std::min(ntasks, by_mem)));
   BBParams F;
