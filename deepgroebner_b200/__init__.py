@@ -7,14 +7,15 @@ there is no CPU fallback.  Importing this package does not load CUDA; constructi
 from .ideals import BinomialSpec, FixedIdealGenerator, PolySpec, cyclic, parse_ideal_dist  # noqa: F401
 
 __all__ = ["BuchbergerEnv", "LeadMonomialsEnv", "BuchbergerEngine", "BuchbergerAgent", "BinomialSpec", "PolySpec",
-           "FixedIdealGenerator", "cyclic", "parse_ideal_dist", "groebner_bases"]
+           "FixedIdealGenerator", "cyclic", "parse_ideal_dist", "groebner_bases",
+           "reduce_polynomials"]
 
 
 def __getattr__(name):  # torch / CUDA are only pulled in when an environment class is requested
     if name in ("BuchbergerEnv", "LeadMonomialsEnv", "BuchbergerEngine", "BuchbergerAgent"):
         from . import buchberger
         return getattr(buchberger, name)
-    if name == "groebner_bases":
+    if name in ("groebner_bases", "reduce_polynomials"):
         from . import strat
-        return strat.groebner_bases
+        return getattr(strat, name)
     raise AttributeError(name)

@@ -66,7 +66,7 @@ EXPORTS = [
     "bb_seed_selection", "bb_value", "bb_copy_env", "bb_set_auto_reset", "bb_step_observe", "bb_step_host", "bb_reset_host", "bb_observe_host", "bb_set_wide", "bb_set_prepare_mode", "bb_set_two_term", "bb_set_selection_seed_stride", "bb_policy_pmlp", "bb_rollout",
     "bb_seed_on", "bb_prepare", "bb_set_episode_offset", "bb_set_timing", "bb_last_run_ms", "bb_set_max_episode_length",
     "bb_set_compaction", "bb_compact", "bb_status_summary", "bb_set_obs_nvars", "bb_discount", "bb_set_serve", "bb_set_prefetch",
-    "bb_run_export",
+    "bb_run_export", "bb_reduce",
 ]
 
 _lib = None
@@ -134,6 +134,8 @@ def load():
     lib.bb_run.argtypes = [vp, i, i, i, vp, i, i, C.c_double, i, vp, vp, i, i, vp]
     lib.bb_run_export.restype = i
     lib.bb_run_export.argtypes = lib.bb_run.argtypes + [C.POINTER(BBPolySink), C.POINTER(BBPolySink)]
+    lib.bb_reduce.restype = i
+    lib.bb_reduce.argtypes = [vp, i, vp, vp, vp, vp, i, vp, vp, vp, vp, i, vp, vp, vp, C.POINTER(BBPolySink), vp]
     lib.bb_value.restype = i
     lib.bb_value.argtypes = [vp, i, C.c_double, i, i, i, vp, vp]
     lib.bb_copy_env.restype = i

@@ -98,6 +98,86 @@ class PolyBatch:
         src_term = where[ep_of_term, 1] + torch.arange(T, device=dev) - term_offsets[ep_of_term]
         return PolyBatch(ep_offsets, poly_offsets, exps.view(-1, nvars)[src_term], coefs[src_term], stored)
 
+    @staticmethod
+    def from_lists(lists, nvars, device="cuda:0", prime=32003, divisors=False):
+        """A batch from host lists: lists[e] is a list of polynomials [(coef, exps), ...], exps of any length whose entries
+        beyond nvars are zero.  Terms are sorted descending in grevlex (ascending packed key, the device's order).  Raises
+        ValueError on a duplicate monomial, a coefficient outside [1, prime), a negative exponent, and, with
+        divisors=True (the lists are divisor lists of reduce()), on the zero polynomial."""
+        ep, po, ex, cf = [0], [0], [], []
+        for G in lists:
+            for f in G:
+                terms = []
+                for c, e in f:
+                    e = tuple(int(x) for x in e)
+                    if any(e[nvars:]) or min(e, default=0) < 0:
+                        raise ValueError("exponents %r: negative, or a variable beyond nvars=%d" % (e, nvars))
+                    e = e[:nvars] + (0,) * (nvars - len(e))
+                    if not 0 < int(c) < prime:
+                        raise ValueError("coefficient %d is outside [1, %d)" % (int(c), prime))
+                    terms.append(((-sum(e),) + e[::-1], int(c), e))   # grevlex: higher degree, then smaller last exponents first
+                if divisors and not terms:
+                    raise ValueError("the zero polynomial is not a valid divisor")
+                terms.sort()
+                for a, b in zip(terms, terms[1:]):
+                    if a[0] == b[0]:
+                        raise ValueError("duplicate monomial %r in a polynomial" % (a[2],))
+                ex.extend(t[2] for t in terms)
+                cf.extend(t[1] for t in terms)
+                po.append(len(cf))
+            ep.append(len(po) - 1)
+        dev = torch.device(device)
+        return PolyBatch(torch.tensor(ep, dtype=torch.int64, device=dev), torch.tensor(po, dtype=torch.int64, device=dev),
+                         torch.tensor(ex, dtype=torch.int32).view(-1, nvars).to(dev), torch.tensor(cf, dtype=torch.int32, device=dev),
+                         torch.ones(len(lists), dtype=torch.bool, device=dev))
+
+
+def _group_queries(poly_offsets, exps, coefs, which):
+    """The queries of reduce() (polynomial q = terms poly_offsets[q] .. poly_offsets[q + 1] of exps / coefs, reduced by list
+    which[q]) reordered so that the queries of one list are adjacent: a stable argsort of which.  Returns (order, offsets,
+    exps, coefs, which) of the reordered queries; position i holds query order[i]."""
+    dev = which.device
+    order = torch.argsort(which, stable=True)
+    lens = (poly_offsets[1:] - poly_offsets[:-1])[order]
+    offsets = torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), torch.cumsum(lens, 0)])
+    T = exps.shape[0]
+    src = torch.repeat_interleave(poly_offsets[:-1][order] - offsets[:-1], lens, output_size=T) + torch.arange(T, device=dev)
+    return order, offsets, exps[src], coefs[src], which[order]
+
+
+def _ungroup(order, *grouped):
+    """Per-query results of the reordered queries back in input order."""
+    out = []
+    for t in grouped:
+        u = torch.empty_like(t)
+        u[order] = t
+        out.append(u)
+    return out
+
+
+def _remainder_batch(where, rlen, exps, coefs, ep_offsets, stored, nvars):
+    """The remainders in a packed sink (where int64 [Q, 2] and lengths rlen [Q], in query order) as a PolyBatch with the entry
+    structure ep_offsets / stored of the dividends: query q is polynomial q, empty where nothing was stored.  An entry counts as
+    stored when it was and every one of its queries was."""
+    dev = where.device
+    Q = where.shape[0]
+    ok = where[:, 0] >= 0
+    lens = torch.where(ok, rlen.to(torch.int64), 0)
+    zero = torch.zeros(1, dtype=torch.int64, device=dev)
+    poly_offsets = torch.cat([zero, torch.cumsum(lens, 0)])
+    T = int(poly_offsets[-1])
+    q_of_term = torch.repeat_interleave(torch.arange(Q, device=dev), lens, output_size=T)
+    src = where[q_of_term, 1] + torch.arange(T, device=dev) - poly_offsets[q_of_term]
+    E = ep_offsets.numel() - 1
+    entry = torch.repeat_interleave(torch.arange(E, device=dev), ep_offsets[1:] - ep_offsets[:-1], output_size=Q)
+    missing = torch.zeros(E, dtype=torch.int32, device=dev).index_add_(0, entry, (~ok).to(torch.int32))
+    return PolyBatch(ep_offsets, poly_offsets, exps.view(-1, nvars)[src], coefs[src], stored & (missing == 0))
+
+
+def _nonempty(t):
+    """t, or one zero element of its dtype where t is empty (the C-ABI takes no NULL arrays)."""
+    return t if t.numel() else torch.zeros(1, dtype=t.dtype, device=t.device)
+
 
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -506,6 +586,61 @@ class BuchbergerEngine:
                             where_dev=t["where"].data_ptr(), used_dev=t["used"].data_ptr(), cap_polys=int(polys),
                             cap_terms=int(terms))
         return t, C.byref(s), s
+
+    def reduce(self, polys, divisors, which=None, sorted=False, return_remainders=True, capacity=None):
+        """reduce(g, F) (buchberger.cpp:24-49) on the device (bb_reduce): every polynomial of entry e of the PolyBatch `polys`
+        is reduced by the polynomials of entry which[e] of the PolyBatch `divisors` (default: entry e), e.g. a run_episodes
+        (return_gb=True) batch, passed as it is.  sorted=False scans each list in its order; True scans it stable-sorted by
+        ascending lead monomial (the order of a reduced basis from run_episodes, where both give the same remainders).
+        Queries are grouped by list on the device; results come back in input order.  Returns (remainders, steps, lengths,
+        status): remainders a PolyBatch with the entry structure of `polys` (None with return_remainders=False, which attaches
+        no sink), steps / lengths / status int32 cuda tensors per polynomial (status 2 = done, BB_STATUS_* or -1 for
+        malformed input; a query that is not done has an empty remainder, and its entry is not stored).  A divisor entry
+        that was not stored gives its queries status -1.  capacity: the remainders' sink room as (polynomials, terms); a
+        call whose remainders do not fit is repeated once with the exact totals (a second launch, which the counters count).
+        Like run_episodes, a call on the stream of the step API overwrites its environments."""
+        dev, n = self.device, self.n
+        i32, i64 = torch.int32, torch.int64
+        with torch.cuda.device(dev):
+            if polys.exps.shape[1] != n or divisors.exps.shape[1] != n:
+                raise ValueError("both batches need %d exponents per term" % n)
+            E, L = len(polys), len(divisors)
+            ep = polys.ep_offsets.to(dev)
+            Q = polys.poly_offsets.numel() - 1
+            w = torch.arange(E, device=dev) if which is None else torch.as_tensor(which, device=dev).to(i64).view(-1)
+            if w.numel() != E:
+                raise ValueError("which needs one list per entry of polys")
+            if L:
+                ok = (w >= 0) & (w < L) & divisors.stored.to(dev)[w.clamp(0, L - 1)]
+                w = torch.where(ok, w, -1)
+            else:
+                w = torch.full_like(w, -1)
+            which_q = torch.repeat_interleave(w, ep[1:] - ep[:-1], output_size=Q).to(i32)
+            order, q_off, q_ex, q_cf, wq = _group_queries(polys.poly_offsets.to(dev), polys.exps.to(dev), polys.coefs.to(dev),
+                                                          which_q)
+            steps, rlen, status = (torch.zeros(Q, dtype=i32, device=dev) for _ in range(3))
+            d = [t.to(dev).contiguous() for t in (divisors.ep_offsets, divisors.poly_offsets, divisors.exps, divisors.coefs)]
+            args = [L] + [_nonempty(t) for t in d] + [Q, q_off, _nonempty(q_ex.contiguous()), _nonempty(q_cf), wq]
+            room = capacity or (Q, max(2 * int(q_ex.shape[0]), 1024))
+            sink = None
+            for attempt in range(2 if Q else 0):
+                sink = self._sink(Q, *room) if return_remainders else None
+                self._ck(self.lib.bb_reduce(self.h, *[a if isinstance(a, int) else _ptr(a) for a in args], int(bool(sorted)),
+                                            _ptr(steps), _ptr(rlen), _ptr(status), sink[1] if sink else None, _stream()),
+                         "bb_reduce")
+                if sink is None:
+                    break
+                used = sink[0]["used"].tolist()
+                if attempt or used[2] == 0:
+                    break
+                room = (used[0], used[1])
+            steps, rlen, status = _ungroup(order, steps, rlen, status)
+            rem = None
+            if return_remainders:
+                where = _ungroup(order, sink[0]["where"])[0] if sink else torch.full((Q, 2), -1, dtype=i64, device=dev)
+                t = sink[0] if sink else dict(exps=torch.zeros(0, dtype=i32, device=dev), coefs=torch.zeros(0, dtype=i32, device=dev))
+                rem = _remainder_batch(where, rlen, t["exps"], t["coefs"], ep, polys.stored.to(dev), n)
+        return rem, steps, rlen, status
 
     def value(self, strategy="degree", gamma=0.99, rollouts=None, selection_seed=0, max_steps=0, out=None):
         """BuchbergerEnv.value for every environment (bb_value): float64 cuda tensor [N].  strategy is a selection

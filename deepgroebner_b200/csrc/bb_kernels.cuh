@@ -9,6 +9,7 @@
 //   k_run      persistent: episodes pulled from a queue and run to completion with on-device selection
 //              (the loop of buchberger(), buchberger.cpp:243-263); finished slots refill at once.
 //   k_final_gb interreduce(minimalize(G))    buchberger.cpp:102-122
+//   k_reduce   reduce(g, F)                  buchberger.cpp:24-49 on caller-supplied divisor lists and dividends (bb_reduce)
 #pragma once
 #include "bb_device.cuh"
 #include "bb_policy.cuh"
@@ -132,6 +133,18 @@ struct BBMailbox {
 };
 static_assert(sizeof(BBMailbox) == 128, "mailbox header is two 64-byte lines");
 
+// bb_reduce: caller-supplied divisor lists (PolyBatch layout: list -> polynomials -> terms, int64 offsets) and dividends.
+// Queries come grouped by list; a worker warp pops `chunk` consecutive queries at a time and restages its slot only when
+// the list changes.
+struct BBReduceArgs {
+  int nlists, nq, sorted, chunk;
+  const int64_t* list_off; const int64_t* poly_off; const int32_t* exps; const int32_t* coefs;
+  const int64_t* q_off; const int32_t* q_exps; const int32_t* q_coefs; const int32_t* which;
+  int32_t* steps; int32_t* rlen; int32_t* status;
+  bb_poly_sink sink;   // lens_dev == NULL: no sink
+  int* queue;          // [1] next query, zeroed by the caller
+};
+
 struct BBKernelTable {
   int nvars, w, dw, dshift, eshift;
   cudaError_t (*reset)(const BBParams&, const uint8_t* mask, int nwarps, cudaStream_t);
@@ -158,6 +171,7 @@ struct BBKernelTable {
                         float* logits, int pmax, int nwarps, cudaStream_t);
   cudaError_t (*rollout)(const BBParams&, const BBRolloutArgs&, int nwarps, cudaStream_t);
   int (*run_warps_per_sm)(int two);   // k_run: general (0) or two-term (1); -1 on error
+  cudaError_t (*reduce)(const BBParams&, const BBReduceArgs&, int nwarps, cudaStream_t);
 };
 
 const BBKernelTable* bb_kernel_table(int nvars);  // bbenv.cu; NULL if nvars is outside 1..8
@@ -1127,6 +1141,169 @@ __global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout(c
   counters_flush(P, sh);
 }
 
+// ------------------------------------------------------------------------------------------------ reduce(g, F)
+// Packs n int32 terms (exponent rows of NV, coefficients) into (k, c), lane-strided.  Returns 0, -1 (a coefficient outside
+// [1, p) or a negative exponent) or BB_STATUS_OVERFLOW_EXPONENT (an exponent above emax or a degree above dmax).
+template <int NV>
+__device__ __forceinline__ int reduce_pack_terms(const BBField& F, const int32_t* __restrict__ ex, const int32_t* __restrict__ cf,
+                                                 long long n, uint64_t* __restrict__ k, uint32_t* __restrict__ c) {
+  typedef KL<NV> K;
+  bool bad = false, ovf = false;
+#pragma unroll 1
+  for (long long t = bb_lane(); t < n; t += 32) {
+    const int32_t co = cf[t];
+    bad |= co <= 0 || (uint32_t)co >= F.p;
+    uint64_t key = 0ull; uint32_t deg = 0u;
+#pragma unroll
+    for (int v = 0; v < NV; v++) {
+      const int32_t x = ex[t * NV + v];
+      bad |= x < 0;
+      ovf |= x > (int32_t)K::emax;
+      key |= (uint64_t)((uint32_t)x & K::fmask) << (K::eshift + v * K::w);
+      deg += (uint32_t)x & K::fmask;
+    }
+    ovf |= deg > K::dmax;
+    k[t] = key | ((uint64_t)(K::dmax - (deg & K::dmax)) << K::dshift);
+    c[t] = (uint32_t)co;
+  }
+  if (__any_sync(BB_FULL, bad)) return -1;
+  return __any_sync(BB_FULL, ovf) ? BB_STATUS_OVERFLOW_EXPONENT : 0;
+}
+
+// Stages divisor list w into the worker's slot: terms at the start of the term arena, one head record per polynomial
+// (1/LC, second term, offset, length; sugar 0), and the reducer list rlm / ridx in scan order -- as given, or stable
+// ascending by lead monomial when A.sorted (the order of G_ under sort_reducers, buchberger.cpp:308-311).  Returns 0 and
+// the list's polynomial and term counts, or the status every query of the list gets.
+template <int NV>
+__device__ __forceinline__ int reduce_stage_list(const BBParams& P, const BBReduceArgs& A, const Env& e, int w, int& nF, int& nT) {
+  const int lane = bb_lane();
+  const long long p0 = A.list_off[w], p1 = A.list_off[w + 1];
+  nF = 0; nT = 0;
+  if (p0 < 0 || p1 < p0) return -1;
+  if (p1 - p0 > P.max_basis) return BB_STATUS_OVERFLOW_BASIS;
+  const long long t0 = A.poly_off[p0], t1 = A.poly_off[p1];
+  if (t0 < 0 || t1 < t0) return -1;
+  if (t1 - t0 > P.max_terms) return BB_STATUS_OVERFLOW_TERMS;
+  uint64_t* tk = ENV_PTR(uint64_t, e, P, o_tkey);
+  uint32_t* tc = ENV_PTR(uint32_t, e, P, o_tcoef);
+  const int rc = reduce_pack_terms<NV>(P.F, A.exps + t0 * NV, A.coefs + t0, t1 - t0, tk, tc);
+  if (rc) return rc;
+  __syncwarp();
+  const int m = (int)(p1 - p0);
+  GHeadMem* gh = ENV_PTR(GHeadMem, e, P, o_ghead);
+  bool bad = false;
+#pragma unroll 1
+  for (int i = lane; i < m; i += 32) {   // every polynomial non-zero, inside the list's terms, strictly descending
+    const long long a = A.poly_off[p0 + i] - t0, b = A.poly_off[p0 + i + 1] - t0;
+    if (a < 0 || b <= a || b > t1 - t0) { bad = true; continue; }
+    for (long long t = a; t + 1 < b; t++) bad |= tk[t] >= tk[t + 1];
+    const uint64_t lm = tk[a], k1 = b - a > 1 ? tk[a + 1] : 0ull;
+    const uint32_t c1 = b - a > 1 ? tc[a + 1] : 0u;
+    reinterpret_cast<uint4*>(gh + i)[0] = make_uint4((uint32_t)lm, (uint32_t)(lm >> 32), (uint32_t)k1, (uint32_t)(k1 >> 32));
+    reinterpret_cast<uint4*>(gh + i)[1] = make_uint4((uint32_t)bb_global(P.invtab)[tc[a]] | (c1 << 16), 0u, (uint32_t)a,
+                                                     (uint32_t)(b - a));
+  }
+  if (__any_sync(BB_FULL, bad)) return -1;
+  __syncwarp();
+  uint64_t* rlm = ENV_PTR(uint64_t, e, P, o_rlm);
+  uint32_t* ridx = ENV_PTR(uint32_t, e, P, o_ridx);
+#pragma unroll 1
+  for (int i = lane; i < m; i += 32) {
+    const uint64_t li = gh[i].lm;
+    int pos = i;
+    if (A.sorted) {   // ascending lead monomial == descending key; equal lead monomials keep their order
+      pos = 0;
+      for (int j = 0; j < m; j++) { const uint64_t lj = gh[j].lm; pos += lj > li || (lj == li && j < i); }
+    }
+    rlm[pos] = li; ridx[pos] = (uint32_t)i;
+  }
+  __syncwarp();
+  nF = m; nT = (int)(t1 - t0);
+  return 0;
+}
+
+// reduce(g, F) (buchberger.cpp:24-49) of query q by the list staged in the slot (nF polynomials on nT terms): the dividend goes
+// to scratch half 0, warp_reduce runs on it, the remainder lands behind the list's terms.  Returns the query's status.
+template <int NV>
+__device__ __forceinline__ int reduce_query(const BBParams& P, const BBReduceArgs& A, Env& e, int q, int nF, int nT, int& steps,
+                                            int& rlen, Ctr& ct) {
+  typedef KL<NV> K;
+  steps = 0; rlen = 0;
+  const long long a0 = A.q_off[q], a1 = A.q_off[q + 1];
+  if (a0 < 0 || a1 < a0) return -1;
+  if (a1 - a0 > P.max_poly_terms) return BB_STATUS_OVERFLOW_SCRATCH;
+  const int n = (int)(a1 - a0);
+  uint64_t* hk = ENV_PTR(uint64_t, e, P, o_hkey);
+  uint32_t* hc = ENV_PTR(uint32_t, e, P, o_hcoef);
+  const int rc = reduce_pack_terms<NV>(P.F, A.q_exps + a0 * NV, A.q_coefs + a0, n, hk, hc);
+  if (rc) return rc;
+  __syncwarp();
+  bool bad = false;
+#pragma unroll 1
+  for (int t = bb_lane(); t + 1 < n; t += 32) bad |= hk[t] >= hk[t + 1];
+  if (__any_sync(BB_FULL, bad)) return -1;
+  Dividend h;
+  h.k0 = h.k1 = 0; h.c0 = h.c1 = 0; h.sug = 0;
+  dividend_from_scratch(P, e, h, n, 0);
+  e.guard = 0;
+  rlen = warp_reduce<NV>(P, e, h, ENV_PTR(uint64_t, e, P, o_rlm), ENV_PTR(uint32_t, e, P, o_ridx), nF, A.sorted != 0,
+                         ENV_PTR(uint64_t, e, P, o_tkey) + nT, ENV_PTR(uint32_t, e, P, o_tcoef) + nT, P.max_terms - nT, steps, ct);
+  if (rlen < 0 || (e.guard & K::g_all))
+    return rlen == -1 ? BB_STATUS_OVERFLOW_SCRATCH : (rlen == -2 ? BB_STATUS_OVERFLOW_TERMS : BB_STATUS_OVERFLOW_EXPONENT);
+  return BB_STATUS_DONE;
+}
+
+// bb_reduce: persistent worker warps, one slot each.  Per query: steps, remainder length and status (nothing else is written
+// for a query that does not end BB_STATUS_DONE), the remainder to the sink as entry q.  The traffic counters and `additions`
+// count the queries that end done; env_steps and episodes are not touched.
+template <int NV>
+__global__ void __launch_bounds__(BB_THREADS, BB_MIN_BLOCKS) k_reduce(const __grid_constant__ BBParams P,
+                                                                     const __grid_constant__ BBReduceArgs A) {
+  __shared__ unsigned long long sh[BB_WARPS][CT_COUNT];
+  unsigned long long* row = counters_row(sh);
+  const int slot = (blockIdx.x * BB_THREADS + threadIdx.x) >> 5;
+  const int lane = bb_lane();
+  if (slot < P.num_envs) {
+    Env e;
+    e.base = bb_global(P.arena + (size_t)slot * P.slot_stride);
+    e.nG = e.nP = e.nT = 0; e.status = BB_STATUS_RUNNING; e.guard = 0;
+    Ctr ct; ct.clear();
+    int staged = -1, lstat = 0, nF = 0, nT = 0;
+    for (;;) {
+      int q0 = 0;
+      if (lane == 0) q0 = atomicAdd(A.queue, A.chunk);
+      q0 = __shfl_sync(BB_FULL, q0, 0);
+      if (q0 >= A.nq) break;
+      const int q1 = q0 + A.chunk < A.nq ? q0 + A.chunk : A.nq;
+#pragma unroll 1
+      for (int q = q0; q < q1; q++) {
+        const int w = A.which[q];
+        int status = -1, steps = 0, rlen = 0;
+        if ((unsigned)w < (unsigned)A.nlists) {
+          if (w != staged) { lstat = reduce_stage_list<NV>(P, A, e, w, nF, nT); staged = w; }
+          status = lstat ? lstat : reduce_query<NV>(P, A, e, q, nF, nT, steps, rlen, ct);
+        }
+        const bool done = status == BB_STATUS_DONE;
+        if (lane == 0) {
+          A.steps[q] = done ? steps : 0; A.rlen[q] = done ? rlen : 0; A.status[q] = status;
+          if (done) row[CT_ADDS] += (unsigned)steps;
+        }
+        if (done) {
+          ct.spill(row);
+          __syncwarp();
+          if (A.sink.lens_dev)
+            warp_export_polys<NV>(ENV_PTR(uint64_t, e, P, o_tkey) + nT, ENV_PTR(uint32_t, e, P, o_tcoef) + nT, A.rlen + q, 1, 1,
+                                  rlen, A.sink, q);
+        } else {
+          ct.clear();
+        }
+        __syncwarp();
+      }
+    }
+  }
+  counters_flush(P, sh);
+}
+
 // ------------------------------------------------------------------------------------------------ launchers
 static inline int grid_for_warps(int nwarps) { return (nwarps + BB_WARPS - 1) / BB_WARPS; }
 
@@ -1187,6 +1364,7 @@ struct BBLaunch {
     cudaFuncSetAttribute(k_prepare<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_prepare_lanes<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
     cudaFuncSetAttribute(k_order<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+    cudaFuncSetAttribute(k_reduce<NV>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
   }
   static cudaError_t prepare(const BBParams& S, const BBRunArgs& A, cudaStream_t s) {
     same_carveout();
@@ -1299,11 +1477,16 @@ struct BBLaunch {
     if (e != cudaSuccess) return -1;
     return blocks * (two ? BB_TWO_WARPS : BB_WARPS);
   }
+  static cudaError_t reduce(const BBParams& P, const BBReduceArgs& A, int nwarps, cudaStream_t s) {
+    same_carveout();
+    k_reduce<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, A);
+    return cudaGetLastError();
+  }
   static const BBKernelTable* table() {
     static const BBKernelTable t = {NV, KL<NV>::w, KL<NV>::dw, KL<NV>::dshift, KL<NV>::eshift,
                                     &reset, &step, &step_obs, &serve, &prefill, &select, &observe, &final_gb, &prepare, &run, &run_streams, &streams_warps_per_sm, &run_wide, &wide_ctas_per_sm, &value, &policy,
                                     &rollout,
-                                    &run_warps_per_sm};
+                                    &run_warps_per_sm, &reduce};
     return &t;
   }
 };

@@ -207,6 +207,7 @@ struct bb_handle {
     bool ready;
     unsigned char* arena; BBEnvState* st;
     uint64_t* gkey; uint32_t* gcoef; int* glen; int* gcount; uint64_t* grlm; uint32_t* gridx; uint32_t* gflag;
+    int* queue;         // bb_reduce's query counter
     cudaEvent_t done;   // recorded after the last runner that used the bank
     cudaStream_t stream; // ... and the stream it ran on (calls on the same stream are ordered anyway)
     unsigned long long serial;   // order of use (all busy: queue behind the least recently taken)
@@ -512,7 +513,9 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
     T.order = nullptr; T.cost_key = nullptr; T.queue = nullptr; T.prepared = nullptr; T.consumed = nullptr;
     T.episodes = 0; T.seed_base = 0; T.seeds = nullptr; T.serial = 0;
   }
-  for (int b = 0; b < BB_BANKS; b++) { h->bank[b].ready = false; h->bank[b].done = nullptr; h->bank[b].stream = nullptr; h->bank[b].serial = 0; }
+  for (int b = 0; b < BB_BANKS; b++) {
+    h->bank[b].ready = false; h->bank[b].done = nullptr; h->bank[b].stream = nullptr; h->bank[b].serial = 0; h->bank[b].queue = nullptr;
+  }
   h->stage_next = 0; h->stage_serial = 0; h->side = nullptr; h->ev_entry = nullptr; h->timing = 0;
   h->ev_t[0] = h->ev_t[1] = h->ev_t[2] = nullptr;
   h->episode_offset = 0; h->nstaged = 0; h->d_seeds = nullptr; h->h_seeds = nullptr; h->ev_seeds = nullptr;
@@ -586,6 +589,7 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
   h->bank[0].ready = true;
   h->bank[0].arena = P.arena; h->bank[0].st = P.st; h->bank[0].gkey = P.gkey; h->bank[0].gcoef = P.gcoef; h->bank[0].glen = P.glen;
   h->bank[0].gcount = P.gcount; h->bank[0].grlm = P.grlm; h->bank[0].gridx = P.gridx; h->bank[0].gflag = P.gflag;
+  CKC(dev_alloc(h, &h->bank[0].queue, (size_t)1));
   CKC(cudaHostAlloc((void**)&h->h_seeds, sizeof(int) * N, cudaHostAllocDefault));
   CKC(cudaEventCreateWithFlags(&h->ev_seeds, cudaEventDisableTiming));
   CKC(cudaEventCreateWithFlags(&h->ev_entry, cudaEventDisableTiming));
@@ -1042,12 +1046,103 @@ int bb_prepare(bb_handle* h, int episodes, int seed_base, const int32_t* seeds_d
   return 0;
 }
 
-static int check_sink(bb_handle* h, const bb_poly_sink* k, const char* which) {
+static int check_sink(bb_handle* h, const bb_poly_sink* k, const char* which, const char* fn = "bb_run_export") {
   if (!k) return 0;
   if (!k->lens_dev || !k->exps_dev || !k->coefs_dev || !k->where_dev || !k->used_dev)
-    return fail(h, std::string("bb_run_export: the ") + which + " sink has a NULL buffer");
+    return fail(h, std::string(fn) + ": the " + which + " sink has a NULL buffer");
   if (k->cap_polys < 0 || k->cap_terms < 0)
-    return fail(h, std::string("bb_run_export: the ") + which + " sink has a negative capacity");
+    return fail(h, std::string(fn) + ": the " + which + " sink has a negative capacity");
+  return 0;
+}
+
+// The environment bank of a bb_run / bb_reduce call on stream s: the one this stream used last (calls on a stream are ordered
+// anyway), else the first bank no kernel on another stream may still be using (allocated on first use), else the least
+// recently taken one, which s then waits for.  PB receives the handle's parameters on that bank; returns its index or < 0.
+// The caller records the bank's `done` event after its last kernel.
+static int take_bank(bb_handle* h, cudaStream_t s, BBParams& PB) {
+  int bk = -1;
+  for (int b = 0; b < BB_BANKS && bk < 0; b++)
+    if (h->bank[b].ready && h->bank[b].stream == s) bk = b;
+  if (bk < 0) {
+    for (int b = 0; b < BB_BANKS && bk < 0; b++) {
+      bb_handle::Bank& B = h->bank[b];
+      if (!B.ready) {
+        const size_t N = (size_t)h->P.num_envs;
+        const BBParams& P = h->P;
+        CK(dev_alloc(h, &B.arena, N * P.slot_stride));
+        CK(dev_alloc(h, &B.st, N));
+        CK(dev_alloc(h, &B.gkey, N * P.max_terms));
+        CK(dev_alloc(h, &B.gcoef, N * P.max_terms));
+        CK(dev_alloc(h, &B.glen, N * P.max_basis));
+        CK(dev_alloc(h, &B.gcount, N * 2));
+        CK(dev_alloc(h, &B.grlm, N * P.max_basis));
+        CK(dev_alloc(h, &B.gridx, N * P.max_basis));
+        CK(dev_alloc(h, &B.gflag, N * P.max_basis));
+        CK(dev_alloc(h, &B.queue, (size_t)1));
+        CK(cudaDeviceSynchronize());   // the allocations' memsets ran on the legacy stream
+        B.ready = true;
+        bk = b;
+      } else if (cudaEventQuery(B.done) == cudaSuccess) {
+        bk = b;
+      } else {
+        (void)cudaGetLastError();   // cudaErrorNotReady is not an error
+      }
+    }
+    if (bk < 0) {   // every bank is in use elsewhere: queue behind the least recently taken
+      bk = 0;
+      for (int b = 1; b < BB_BANKS; b++) if (h->bank[b].serial < h->bank[bk].serial) bk = b;
+      CK(cudaStreamWaitEvent(s, h->bank[bk].done, 0));
+    }
+  }
+  h->bank[bk].stream = s;
+  h->bank[bk].serial = ++h->stage_serial;
+  PB = h->P;
+  const bb_handle::Bank& B = h->bank[bk];
+  PB.arena = B.arena; PB.st = B.st; PB.gkey = B.gkey; PB.gcoef = B.gcoef; PB.glen = B.glen; PB.gcount = B.gcount;
+  PB.grlm = B.grlm; PB.gridx = B.gridx; PB.gflag = B.gflag;
+  return bk;
+}
+
+// queries per pop of bb_reduce's workers: about four pops per worker, at most 32 queries each
+#define BB_REDUCE_POPS 4
+#define BB_REDUCE_CHUNK_MAX 32
+
+int bb_reduce(bb_handle* h, int nlists, const int64_t* list_offsets_dev, const int64_t* poly_offsets_dev,
+              const int32_t* exps_dev, const int32_t* coefs_dev, int nqueries, const int64_t* q_offsets_dev,
+              const int32_t* q_exps_dev, const int32_t* q_coefs_dev, const int32_t* which_dev, int sorted, int32_t* steps_dev,
+              int32_t* rlen_dev, int32_t* status_dev, const bb_poly_sink* rem, void* stream) {
+  if (!h) return -1;
+  if (nlists < 0 || nqueries < 0) return fail(h, "bb_reduce: negative count");
+  if (!list_offsets_dev || !poly_offsets_dev || !exps_dev || !coefs_dev || !q_offsets_dev || !q_exps_dev || !q_coefs_dev ||
+      !which_dev || !steps_dev || !rlen_dev || !status_dev)
+    return fail(h, "bb_reduce: a required pointer is NULL");
+  int rc = check_sink(h, rem, "rem", "bb_reduce");
+  if (rc < 0) return rc;
+  ENTER(h);
+  if (nqueries == 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  BBParams PB;
+  const int bk = take_bank(h, s, PB);
+  if (bk < 0) return bk;
+  BBReduceArgs A;
+  memset(&A, 0, sizeof A);
+  A.nlists = nlists; A.nq = nqueries; A.sorted = sorted ? 1 : 0;
+  A.chunk = (int)std::min<long long>(BB_REDUCE_CHUNK_MAX,
+                                     std::max<long long>(1, nqueries / ((long long)BB_REDUCE_POPS * h->run_wave[0])));
+  A.list_off = list_offsets_dev; A.poly_off = poly_offsets_dev; A.exps = exps_dev; A.coefs = coefs_dev;
+  A.q_off = q_offsets_dev; A.q_exps = q_exps_dev; A.q_coefs = q_coefs_dev; A.which = which_dev;
+  A.steps = steps_dev; A.rlen = rlen_dev; A.status = status_dev;
+  if (rem) {
+    A.sink = *rem;
+    CK(cudaMemsetAsync(rem->where_dev, 0xff, sizeof(int64_t) * 2 * (size_t)nqueries, s));
+  }
+  A.queue = h->bank[bk].queue;
+  CK(cudaMemsetAsync(A.queue, 0, sizeof(int), s));
+  // workers: one per pop at most, no more than the bank's slots and the general runner's resident wave (same launch bounds)
+  const int pops = (nqueries + A.chunk - 1) / A.chunk;
+  const int workers = std::min(std::min(pops, h->P.num_envs), h->run_wave[0]);
+  CK(h->K->reduce(PB, A, workers, s));
+  CK(cudaEventRecord(h->bank[bk].done, s));
   return 0;
 }
 
@@ -1083,49 +1178,9 @@ int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const
     if (wide_ctas <= 0) return fail(h, "bb_run: the CTA-per-environment stream runner does not fit this device");
   }
   const int nbatch = (episodes + BB_RUN_BATCH - 1) / BB_RUN_BATCH;
-  // the arena bank of this call: the one this stream used last (calls on a stream are ordered anyway), else the first bank
-  // no runner on another stream may still be using (allocated on first use), else the least recently taken one
-  int bk = -1;
-  for (int b = 0; b < BB_BANKS && bk < 0; b++)
-    if (h->bank[b].ready && h->bank[b].stream == s) bk = b;
-  if (bk < 0) {
-    for (int b = 0; b < BB_BANKS && bk < 0; b++) {
-      bb_handle::Bank& B = h->bank[b];
-      if (!B.ready) {
-        const size_t N = (size_t)h->P.num_envs;
-        const BBParams& P = h->P;
-        CK(dev_alloc(h, &B.arena, N * P.slot_stride));
-        CK(dev_alloc(h, &B.st, N));
-        CK(dev_alloc(h, &B.gkey, N * P.max_terms));
-        CK(dev_alloc(h, &B.gcoef, N * P.max_terms));
-        CK(dev_alloc(h, &B.glen, N * P.max_basis));
-        CK(dev_alloc(h, &B.gcount, N * 2));
-        CK(dev_alloc(h, &B.grlm, N * P.max_basis));
-        CK(dev_alloc(h, &B.gridx, N * P.max_basis));
-        CK(dev_alloc(h, &B.gflag, N * P.max_basis));
-        CK(cudaDeviceSynchronize());   // the allocations' memsets ran on the legacy stream
-        B.ready = true;
-        bk = b;
-      } else if (cudaEventQuery(B.done) == cudaSuccess) {
-        bk = b;
-      } else {
-        (void)cudaGetLastError();   // cudaErrorNotReady is not an error
-      }
-    }
-    if (bk < 0) {   // every bank is in use elsewhere: queue behind the least recently taken
-      bk = 0;
-      for (int b = 1; b < BB_BANKS; b++) if (h->bank[b].serial < h->bank[bk].serial) bk = b;
-      CK(cudaStreamWaitEvent(s, h->bank[bk].done, 0));
-    }
-  }
-  h->bank[bk].stream = s;
-  h->bank[bk].serial = ++h->stage_serial;
-  BBParams PB = h->P;
-  {
-    const bb_handle::Bank& B = h->bank[bk];
-    PB.arena = B.arena; PB.st = B.st; PB.gkey = B.gkey; PB.gcoef = B.gcoef; PB.glen = B.glen; PB.gcount = B.gcount;
-    PB.grlm = B.grlm; PB.gridx = B.gridx; PB.gflag = B.gflag;
-  }
+  BBParams PB;
+  const int bk = take_bank(h, s, PB);
+  if (bk < 0) return bk;
   // Batch 0: already prepared by a matching bb_prepare, or prepared here on the caller's stream.  Batches 1.. of the
   // same call are prepared on the handle's side stream while the runner works through their predecessor.
   int which = -1;

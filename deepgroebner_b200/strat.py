@@ -111,11 +111,14 @@ def _staged_engine(ideals, device, capacity, caps, **env_kw):
     return eng
 
 
+CAPACITY_ADVICE = "raise the arena capacities (capacity='general' or max_basis/max_pairs/max_terms keywords)"
+
+
 def _check_finished(stats):
     bad = (stats["status"] != 2).nonzero()[0]
     if len(bad):
-        raise RuntimeError("ideal %d did not finish (status %d): raise the arena capacities (capacity='general' or "
-                           "max_basis/max_pairs/max_terms keywords)" % (int(bad[0]), int(stats["status"][bad[0]])))
+        raise RuntimeError("ideal %d did not finish (status %d): %s" % (int(bad[0]), int(stats["status"][bad[0]]),
+                                                                         CAPACITY_ADVICE))
 
 
 def strategy_stats(ideals, strategy, seed=0, device="cuda:0", capacity=None, **caps):
@@ -146,6 +149,44 @@ def groebner_bases(ideals, selection="degree", elimination="gebauermoeller", sor
     pad = (0,) * (NVARS_MAX - eng.n)
     bases = [[[(c, e + pad) for c, e in g] for g in G] for G in out["gb"].to_lists()]
     return bases, stats
+
+
+def reduce_polynomials(polys, divisors, sorted=False, prime=32003, device="cuda:0", capacity=None, **caps):
+    """reduce(g, F) (buchberger.cpp:24-49) for lists of polynomials, on the device in one launch: polys[i] is a list of
+    polynomials, each reduced by the list divisors[i], all in the form parse_ideal_string gives ([(coef, exponents), ...]).
+    sorted=False scans each divisor list in its order, True stable-sorted by ascending lead monomial.  Returns (remainders,
+    steps): remainders[i][j] is the remainder of polys[i][j] ([(coef, 8 exponents), ...], descending grevlex, not made monic)
+    and steps[i][j] its number of reduction steps.
+    When divisors[i] is a Groebner basis of an ideal I (groebner_bases gives reduced ones), the remainder of g is its normal
+    form modulo I, and it is empty exactly when g lies in I.  A reduction that overflows the arena capacities raises."""
+    from .buchberger import BuchbergerEngine, PolyBatch, resident_envs
+    from .ideals import FixedIdealGenerator
+    import torch
+    if len(polys) != len(divisors):
+        raise ValueError("one divisor list per list of polynomials")
+    n = 1
+    for L in (polys, divisors):
+        for F in L:
+            for f in F:
+                for _, e in f:
+                    for v, x in enumerate(e):
+                        if x:
+                            n = max(n, v + 1)
+    P = PolyBatch.from_lists(polys, n, device, prime=prime)
+    D = PolyBatch.from_lists(divisors, n, device, prime=prime, divisors=True)
+    envs = max(1, min(len(divisors), resident_envs(torch.device(device).index or 0, n)))
+    eng = BuchbergerEngine(FixedIdealGenerator([[(1, (0,) * n)]], n), num_envs=envs, device=device, prime=prime,
+                           capacity=capacity or "poly", **caps)
+    rem, steps, _, status = eng.reduce(P, D, sorted=sorted)
+    st = status.cpu().numpy()
+    bad = (st != 2).nonzero()[0]
+    if len(bad):
+        raise RuntimeError("polynomial %d of the call did not reduce (status %d): %s" % (int(bad[0]), int(st[bad[0]]),
+                                                                                      CAPACITY_ADVICE))
+    pad = (0,) * (NVARS_MAX - n)
+    ep, sp = P.ep_offsets.tolist(), steps.tolist()
+    remainders = [[[(c, e + pad) for c, e in r] for r in R] for R in rem.to_lists()]
+    return remainders, [sp[ep[i]:ep[i + 1]] for i in range(len(polys))]
 
 
 def make_strat(dist, strategy, seed=None, root="data/stats", device="cuda:0", **caps):

@@ -20,6 +20,7 @@
  *   BuchbergerEnv::G, ::P   buchberger.h:195-196            bb_download_basis, bb_pairs
  *   buchberger(...) -> interreduce(minimalize(G))           bb_final_gb
  *       buchberger.cpp:265
+ *   reduce(g, F) -> (r, ReduceStats)   buchberger.h:26-28   bb_reduce (batches of dividends against device-resident lists)
  *
  * Conventions: plain pointers and sizes only (no torch types).  Every entry point returns 0 on success and a
  * negative code otherwise; bb_last_error() gives the message.  Pointers named *_dev are DEVICE pointers in the
@@ -253,6 +254,38 @@ typedef struct bb_poly_sink {
 int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const int32_t* seeds_dev, int sel_seed_base,
                   int max_steps, double gamma, int compute_gb, bb_episode_stats* stats_dev, int32_t* trace_dev,
                   int trace_episodes, int trace_cap, void* stream, const bb_poly_sink* gb, const bb_poly_sink* basis);
+
+/* bb_reduce: the division algorithm reduce(g, F) (buchberger.cpp:24-49) for a batch of dividends against caller-supplied
+ * divisor lists, on the device.  While h != 0: the first f of F (scanned in order) with LM f | LM h gives
+ * h <- h - (LT h / LT f) f and steps += 1; otherwise LT h moves to the remainder.  The remainder is not made monic.
+ *   divisor lists   exactly the layout of a run_episodes(return_gb) batch: list_offsets_dev int64 [nlists + 1] indexes
+ *                   polynomials, poly_offsets_dev int64 [npolys + 1] indexes terms, exps_dev int32 [nterms * n],
+ *                   coefs_dev int32 [nterms]; n = cfg.nvars
+ *   queries         q_offsets_dev int64 [nqueries + 1] into q_exps_dev / q_coefs_dev (same term layout); query q is reduced by
+ *                   list which_dev[q].  Queries that share a list should be adjacent: a worker restages a list only when
+ *                   it changes.
+ * Every polynomial has its terms strictly descending in grevlex with coefficients in [1, p).  sorted = 0 scans each list in
+ * the order given; sorted = 1 scans it stable-sorted by ascending lead monomial (the order of G_ under sort_reducers,
+ * buchberger.cpp:308-311), which lets the scan stop early; a reduced basis from bb_run_export is already in that order.
+ * Outputs per query: steps_dev, rlen_dev (remainder length) and status_dev, all int32 [nqueries].  Status BB_STATUS_DONE, or
+ *   BB_STATUS_OVERFLOW_EXPONENT  an exponent above the packed layout's field, or a produced monomial that leaves it
+ *   BB_STATUS_OVERFLOW_SCRATCH   a dividend longer than cfg.max_poly_terms (also while reducing)
+ *   BB_STATUS_OVERFLOW_BASIS     a list longer than cfg.max_basis
+ *   BB_STATUS_OVERFLOW_TERMS     the list plus the remainder do not fit cfg.max_terms
+ *   -1                           malformed input: terms not strictly descending, a coefficient outside [1, p), a negative
+ *                                exponent, a zero polynomial in a list, bad offsets, which outside [0, nlists)
+ * A query that does not end done gets steps = rlen = 0 and stores nothing.  rem (may be NULL: lengths, steps and status only,
+ * e.g. for ideal membership) receives the remainder of every query that ends done as entry q, one polynomial, with where_dev
+ * [nqueries * 2] and used_dev behaving as in bb_run_export (after the call used_dev[0..1] hold the exact totals).
+ * bb_counters: additions += sum of steps; terms_read, terms_written, lms_scanned and term_moves (= sum of rlen) as for the
+ * episodes, over the queries that end done; env_steps and episodes do not change.
+ * Fails with nothing enqueued for a negative count, a NULL required pointer, or a sink with a NULL buffer or a negative
+ * capacity.  The call takes a bank of environment slots by the rule of bb_run (see "Pipelines" below): like bb_run, a call on
+ * the stream the step API uses overwrites the step API's environments. */
+int bb_reduce(bb_handle* h, int nlists, const int64_t* list_offsets_dev, const int64_t* poly_offsets_dev,
+              const int32_t* exps_dev, const int32_t* coefs_dev, int nqueries, const int64_t* q_offsets_dev,
+              const int32_t* q_exps_dev, const int32_t* q_coefs_dev, const int32_t* which_dev, int sorted, int32_t* steps_dev,
+              int32_t* rlen_dev, int32_t* status_dev, const bb_poly_sink* rem, void* stream);
 
 /* Pipelines.  Calls of bb_run on ONE stream run one after the other in the handle's own environments.  A call on a second
  * stream while a runner of the first is still at work uses another bank of environment slots (up to three banks, each
