@@ -14,6 +14,7 @@ import torch
 
 from . import _lib
 from .ideals import BinomialSpec, FixedIdealGenerator, PolySpec, parse_ideal_dist
+from .rollout import PairsPolicy
 
 # arena capacities per environment: (max_basis, max_pairs, max_terms, max_poly_terms)
 CAPACITY_PRESETS = {
@@ -497,7 +498,8 @@ class BuchbergerEngine:
 
     def run_episodes(self, strategy="degree", episodes=None, seed_base=0, seeds=None, max_steps=0, gamma=0.99,
                      compute_gb=False, trace_episodes=0, trace_cap=0, to_host=True, selection_seed=0, out_host=None,
-                     out=None, return_gb=False, return_basis=False, gb_capacity=None, basis_capacity=None):
+                     out=None, return_gb=False, return_basis=False, gb_capacity=None, basis_capacity=None, greedy=False,
+                     policy_counter=0):
         """Runs `episodes` episodes to completion with on-device selection (bb_run_export).  Returns (stats, trace):
         stats is a structured array of bb_episode_stats (numpy if to_host else a uint8 cuda tensor), trace an
         int32 [trace_episodes, trace_cap, 4] array of (i, j, additions, |P| after), -1 padded.
@@ -510,11 +512,19 @@ class BuchbergerEngine:
         max_steps), as (stats, trace, {"gb": PolyBatch, "basis": PolyBatch}).  gb_capacity / basis_capacity: room of each
         sink as (polynomials, terms) over the whole call (default: SINK_ROOM per episode of the capacity preset).  A run
         whose polynomials do not fit is repeated once with the exact totals -- a second run of the same episodes, with
-        the same records (runs are deterministic).  Reading the sinks' fill synchronises the stream."""
+        the same records (runs are deterministic).  Reading the sinks' fill synchronises the stream.
+        strategy may also be a rollout.PairsPolicy built for this engine's cols: its head chooses every pair (bb_run_policy),
+        sampling (greedy=False) or taking the argmax, lowest row on ties (greedy=True).  Step t of episode e of the call
+        draws its uniform from stream net.seed + (episode offset + e) and counter policy_counter + t, so environment e of
+        the step API seeded seed_base + e and stepped with policy(net, counter=policy_counter + t) plays the same episode;
+        selection_seed does not apply."""
         episodes = self.num_envs if episodes is None else int(episodes)
         want = [k for k, on in (("gb", return_gb), ("basis", return_basis)) if on]
         compute_gb = compute_gb or return_gb
+        net = strategy if isinstance(strategy, PairsPolicy) else None
         with torch.cuda.device(self.device):
+            if net is not None:
+                W = net.device_weights(self.device, self.cols)
             nbytes = max(episodes, 1) * C.sizeof(_lib.BBEpisodeStats)
             buf = out if out is not None else getattr(self, "_run_buf", None)
             if out is not None:
@@ -544,11 +554,16 @@ class BuchbergerEngine:
                     room[k] = tuple(episodes * x for x in SINK_ROOM[self.preset][k])
             for attempt in range(2):
                 sinks = {k: self._sink(episodes, *room[k]) for k in want}
-                self._ck(self.lib.bb_run_export(self.h, _lib.SELECTION[strategy], episodes, int(seed_base), _ptr(d_seeds),
-                                                int(selection_seed), int(max_steps), float(gamma), int(bool(compute_gb)),
-                                                _ptr(buf), _ptr(trace), int(trace_episodes), int(trace_cap), _stream(),
-                                                sinks["gb"][1] if "gb" in sinks else None,
-                                                sinks["basis"][1] if "basis" in sinks else None), "bb_run_export")
+                tail = (int(max_steps), float(gamma), int(bool(compute_gb)), _ptr(buf), _ptr(trace), int(trace_episodes),
+                        int(trace_cap), _stream(), sinks["gb"][1] if "gb" in sinks else None,
+                        sinks["basis"][1] if "basis" in sinks else None)
+                if net is not None:
+                    self._ck(self.lib.bb_run_policy(self.h, net.hidden, *[_ptr(t) for t in W], int(net.seed),
+                                                    int(policy_counter), int(bool(greedy)), episodes, int(seed_base),
+                                                    _ptr(d_seeds), *tail), "bb_run_policy")
+                else:
+                    self._ck(self.lib.bb_run_export(self.h, _lib.SELECTION[strategy], episodes, int(seed_base), _ptr(d_seeds),
+                                                    int(selection_seed), *tail), "bb_run_export")
                 if not want:
                     break
                 used = {k: sinks[k][0]["used"].tolist() for k in want}

@@ -8,6 +8,7 @@
 //   k_observe  state matrix                  buchberger.cpp:354-370, 402-406
 //   k_run      persistent: episodes pulled from a queue and run to completion with on-device selection
 //              (the loop of buchberger(), buchberger.cpp:243-263); finished slots refill at once.
+//   k_run_policy the same runner with the pairs policy head (bb_policy.cuh) choosing the pairs (bb_run_policy)
 //   k_final_gb interreduce(minimalize(G))    buchberger.cpp:102-122
 //   k_reduce   reduce(g, F)                  buchberger.cpp:24-49 on caller-supplied divisor lists and dividends (bb_reduce)
 #pragma once
@@ -172,6 +173,10 @@ struct BBKernelTable {
   cudaError_t (*rollout)(const BBParams&, const BBRolloutArgs&, int nwarps, cudaStream_t);
   int (*run_warps_per_sm)(int two);   // k_run: general (0) or two-term (1); -1 on error
   cudaError_t (*reduce)(const BBParams&, const BBReduceArgs&, int nwarps, cudaStream_t);
+  // k_run with the policy head selecting (bb_run_policy), and its resident warps per SM for P.cols and W.hidden (-1 on error)
+  cudaError_t (*run_policy)(const BBParams&, const BBParams& stage, const BBRunArgs&, const BBPolicy&,
+                            unsigned long long counter0, int nwarps, cudaStream_t);
+  int (*run_policy_warps_per_sm)(const BBParams&, int hidden);
 };
 
 const BBKernelTable* bb_kernel_table(int nvars);  // bbenv.cu; NULL if nvars is outside 1..8
@@ -738,13 +743,23 @@ __global__ void __launch_bounds__(BB_PREP_THREADS, BB_PREP_MIN_BLOCKS) k_prefill
 // The loop of buchberger() (buchberger.cpp:243-263) on one environment: select, step, accumulate the trace checksum and
 // the discounted return (discounted_return += discount * reward; discount *= gamma, :250-251) until P is empty.
 // STREAMS: reduce() by streams (bb_streams.cuh), ws / st = the warp's stream state and table.  TWO: see warp_step.
-template <int NV, bool STREAMS, bool TWO = false>
+// UPL > 0: the pairs policy head (bb_policy.cuh, H = 32 * UPL, weights at wsm) selects instead of `strategy`; step t draws
+// its uniform from (W->seed + stream, counter0 + t), stream = the episode's global index.
+template <int NV, bool STREAMS, bool TWO = false, int UPL = 0>
 __device__ __forceinline__ void run_episode(const BBParams& P, Env& e, int strategy, int max_steps, double gamma,
                                             BBEpisodeAcc& acc, Ctr& ct, int& steps, int& adds, int4* trace, int trace_cap,
-                                            RegStreams* ws) {
+                                            RegStreams* ws, const BBPolicy* W = nullptr, const float* wsm = nullptr,
+                                            unsigned long long stream = 0, unsigned long long counter0 = 0) {
   const int lane = bb_lane();
   while (e.status == BB_STATUS_RUNNING && (max_steps == 0 || steps < max_steps)) {
-    const int prow = warp_select<NV>(P, e, strategy, &acc.sel_rng);
+    int prow;
+    if constexpr (UPL > 0) {
+      float lp;
+      prow = warp_policy<NV, UPL>(P, e, wsm, W->greedy, policy_uniform(W->seed, stream, counter0 + (unsigned)steps), lp,
+                                  nullptr, 0);
+    } else {
+      prow = warp_select<NV>(P, e, strategy, &acc.sel_rng);
+    }
     uint32_t pr;
     int a;
     if (STREAMS) a = warp_step_rstreams<NV>(P, e, *ws, prow, pr, ct);
@@ -784,8 +799,12 @@ __device__ __noinline__ void warp_export_episode(const BBParams& P, const BBRunA
 // record, repeat.  WARPS = warps per CTA.  EXPORT: bb_run_export's sinks may be attached (an instantiation of its own, so
 // the runner without sinks keeps the parent's code: k_run is issue- and instruction-footprint-bound, and the one extra call
 // site in its loop measured 3 % on configs[1]).  TWO: the two-term step (warp_step), for runs whose ideals are binomial.
-template <int NV, bool STREAMS, int WARPS, bool EXPORT, bool TWO = false>
-__device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S, const BBRunArgs& A) {
+// UPL > 0: the policy head selects (run_episode; W, wsm: the weights and their shared-memory image, counter0: the counter
+// of step 0).
+template <int NV, bool STREAMS, int WARPS, bool EXPORT, bool TWO = false, int UPL = 0>
+__device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S, const BBRunArgs& A,
+                                           const BBPolicy* W = nullptr, const float* wsm = nullptr,
+                                           unsigned long long counter0 = 0) {
   __shared__ unsigned long long sh[WARPS][CT_COUNT];
   __shared__ BBEpisodeAcc acc_sh[WARPS];  // per-episode accumulators only lane 0 touches: kept out of registers
   hot_init(P);
@@ -816,9 +835,9 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
       int steps = 0, adds = 0;
       if (lane == 0) { acc.th = 0ull; acc.ret = 0.0; acc.disc = 1.0; acc.sel_rng = rng_seed(A.sel_seed_base + (A.ep_offset + ep) * A.sel_seed_stride); }
       __syncwarp();
-      run_episode<NV, STREAMS, TWO>(P, e, A.strategy, A.max_steps, A.gamma, acc, ct, steps, adds,
+      run_episode<NV, STREAMS, TWO, UPL>(P, e, A.strategy, A.max_steps, A.gamma, acc, ct, steps, adds,
                                (A.trace && ep < A.trace_eps) ? reinterpret_cast<int4*>(A.trace) + (size_t)ep * A.trace_cap : nullptr,
-                               A.trace_cap, &ws);
+                               A.trace_cap, &ws, W, wsm, (unsigned long long)(A.ep_offset + ep), counter0);
       const int nonzero = e.nG - g_start, zero = steps - nonzero;
       env_store(P, slot, e);
       __syncwarp();
@@ -869,6 +888,19 @@ template <int NV, bool EXPORT = false, bool TWO = false>
 __global__ void __launch_bounds__(TWO ? BB_TWO_WARPS * 32 : BB_THREADS, TWO ? BB_TWO_MIN_BLOCKS : BB_MIN_BLOCKS)
 k_run(const __grid_constant__ BBParams P, const __grid_constant__ BBParams S, const __grid_constant__ BBRunArgs A) {
   run_worker<NV, false, TWO ? BB_TWO_WARPS : BB_WARPS, EXPORT, TWO>(P, S, A);
+}
+
+// The same runner with the pairs policy head choosing the pairs (bb_run_policy): k_rollout's head and step (the general
+// materialising warp_step for every ideal) in k_run's loop, so k_rollout's launch bounds.  The weight image lives in dynamic
+// shared memory; policy_load_weights synchronises the CTA, so it comes before any slot check.  The sinks are checked at run
+// time (an episode here is dominated by the head, not by the epilogue's call site).
+template <int NV, int UPL>
+__global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS)
+k_run_policy(const __grid_constant__ BBParams P, const __grid_constant__ BBParams S, const __grid_constant__ BBRunArgs A,
+             const __grid_constant__ BBPolicy W, unsigned long long counter0) {
+  extern __shared__ float wsm[];
+  policy_load_weights(W, P.cols, wsm);
+  run_worker<NV, false, BB_WARPS, true, false, UPL>(P, S, A, &W, wsm, counter0);
 }
 
 // The same runner for long polynomials: reduce() by streams, the warp's stream table in dynamic shared memory.
@@ -1482,11 +1514,51 @@ struct BBLaunch {
     k_reduce<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, A);
     return cudaGetLastError();
   }
+  template <int UPL>
+  static cudaError_t run_policy_upl(const BBParams& P, const BBParams& S, const BBRunArgs& A, const BBPolicy& W,
+                                    unsigned long long counter0, int nwarps, cudaStream_t s) {
+    const size_t sm = policy_smem(P, W.hidden);
+    if (sm > 48 * 1024) {
+      cudaError_t e = cudaFuncSetAttribute(k_run_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+      if (e != cudaSuccess) return e;
+    }
+    k_run_policy<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, S, A, W, counter0);
+    return cudaGetLastError();
+  }
+  static cudaError_t run_policy(const BBParams& P, const BBParams& S, const BBRunArgs& A, const BBPolicy& W,
+                                unsigned long long counter0, int nwarps, cudaStream_t s) {
+    switch (W.hidden >> 5) {
+      case 1: return run_policy_upl<1>(P, S, A, W, counter0, nwarps, s);
+      case 2: return run_policy_upl<2>(P, S, A, W, counter0, nwarps, s);
+      case 4: return run_policy_upl<4>(P, S, A, W, counter0, nwarps, s);
+      case 8: return run_policy_upl<8>(P, S, A, W, counter0, nwarps, s);
+    }
+    return cudaErrorInvalidValue;
+  }
+  template <int UPL>
+  static int run_policy_warps_upl(size_t sm) {
+    if (sm > 48 * 1024 &&
+        cudaFuncSetAttribute(k_run_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess)
+      return -1;
+    int blocks = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run_policy<NV, UPL>, BB_THREADS, sm) != cudaSuccess) return -1;
+    return blocks * BB_WARPS;
+  }
+  static int run_policy_warps_per_sm(const BBParams& P, int hidden) {
+    const size_t sm = policy_smem(P, hidden);
+    switch (hidden >> 5) {
+      case 1: return run_policy_warps_upl<1>(sm);
+      case 2: return run_policy_warps_upl<2>(sm);
+      case 4: return run_policy_warps_upl<4>(sm);
+      case 8: return run_policy_warps_upl<8>(sm);
+    }
+    return -1;
+  }
   static const BBKernelTable* table() {
     static const BBKernelTable t = {NV, KL<NV>::w, KL<NV>::dw, KL<NV>::dshift, KL<NV>::eshift,
                                     &reset, &step, &step_obs, &serve, &prefill, &select, &observe, &final_gb, &prepare, &run, &run_streams, &streams_warps_per_sm, &run_wide, &wide_ctas_per_sm, &value, &policy,
                                     &rollout,
-                                    &run_warps_per_sm, &reduce};
+                                    &run_warps_per_sm, &reduce, &run_policy, &run_policy_warps_per_sm};
     return &t;
   }
 };

@@ -229,6 +229,7 @@ struct bb_handle {
   int prepare_by_warp;   // bb_run: 1 = episode preparation by one warp per episode even where the thread-per-episode kernel applies
   int two_term;    // bb_run: 1 = the two-term runner for binomial distributions (default), 0 = always the general one
   int run_wave[2];  // resident warps of the general (0) and the two-term (1) k_run on the device: the most either launches
+  int policy_wave[4];  // resident warps of k_run_policy for hidden 32, 64, 128, 256 (0: not asked yet)
   int wide_mode;   // bb_run: reduce() by streams: -1 = when the capacities ask for long polynomials, 0 = never, 1 = always, 2 / 3 = always, small tables
   // host mirrors of the distribution tables
   std::vector<double> cp;
@@ -527,6 +528,7 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
   h->wide_mode = -1;
   h->prepare_by_warp = 0;
   h->two_term = 1;
+  for (int u = 0; u < 4; u++) h->policy_wave[u] = 0;
   h->host_stage = nullptr; h->dev_stage = nullptr; h->stage_bytes = 0;
   h->sel_seed_stride = 1;
   auto bail = [&](int code) { g_create_err = h->err; bb_destroy(h); return code; };
@@ -1146,6 +1148,11 @@ int bb_reduce(bb_handle* h, int nlists, const int64_t* list_offsets_dev, const i
   return 0;
 }
 
+static int run_batches(bb_handle* h, int strategy, const BBPolicy* W, unsigned long long counter0, int episodes, int seed_base,
+                       const int32_t* seeds_dev, int sel_seed_base, int max_steps, double gamma, int compute_gb,
+                       bb_episode_stats* stats_dev, int32_t* trace_dev, int trace_episodes, int trace_cap, void* stream,
+                       const bb_poly_sink* gb, const bb_poly_sink* basis);
+
 int bb_run(bb_handle* h, int strategy, int episodes, int seed_base, const int32_t* seeds_dev, int sel_seed_base,
            int max_steps, double gamma, int compute_gb, bb_episode_stats* stats_dev, int32_t* trace_dev,
            int trace_episodes, int trace_cap, void* stream) {
@@ -1162,14 +1169,37 @@ int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const
   int rc = check_sink(h, gb, "gb");
   if (rc == 0) rc = check_sink(h, basis, "basis");
   if (rc < 0) return rc;
+  return run_batches(h, strategy, nullptr, 0, episodes, seed_base, seeds_dev, sel_seed_base, max_steps, gamma, compute_gb,
+                     stats_dev, trace_dev, trace_episodes, trace_cap, stream, gb, basis);
+}
+
+// The body of bb_run_export and bb_run_policy (arguments already checked): batching, matching bb_prepare batches, the bank,
+// staging and the sinks.  W == NULL: built-in selection `strategy` by the runner the handle's modes pick; otherwise the
+// policy runner (k_run_policy) with weights W and step-0 counter counter0.
+static int run_batches(bb_handle* h, int strategy, const BBPolicy* W, unsigned long long counter0, int episodes, int seed_base,
+                       const int32_t* seeds_dev, int sel_seed_base, int max_steps, double gamma, int compute_gb,
+                       bb_episode_stats* stats_dev, int32_t* trace_dev, int trace_episodes, int trace_cap, void* stream,
+                       const bb_poly_sink* gb, const bb_poly_sink* basis) {
   ENTER(h);
   cudaStream_t s = (cudaStream_t)stream;
   if (episodes == 0) return 0;
-  rc = check_staged(h, "bb_run");
+  int rc = check_staged(h, W ? "bb_run_policy" : "bb_run");
   if (rc < 0) return rc;
+  // the policy runner's resident wave for this hidden width (cached: it depends only on the handle's cols and on hidden)
+  int policy_wave = 0;
+  if (W) {
+    int& w = h->policy_wave[W->hidden == 32 ? 0 : (W->hidden == 64 ? 1 : (W->hidden == 128 ? 2 : 3))];
+    if (w == 0) {
+      const int per_sm = h->K->run_policy_warps_per_sm(h->P, W->hidden);
+      if (per_sm <= 0) return fail(h, "bb_run_policy: the policy runner does not fit this device");
+      w = per_sm * h->sm_count;
+    }
+    policy_wave = w;
+  }
   // long polynomials (general capacities): reduce() by streams (bb_streams.cuh), by default with one CTA per
-  // environment (bb_wide.cuh: the shortest chain of additions); mode 4: one warp per environment
-  const bool streams = h->wide_mode != 0 && (h->wide_mode >= 1 || h->P.max_poly_terms >= 256);
+  // environment (bb_wide.cuh: the shortest chain of additions); mode 4: one warp per environment.  The policy runner always
+  // steps with the materialising reduction: its episodes are dominated by the head.
+  const bool streams = !W && h->wide_mode != 0 && (h->wide_mode >= 1 || h->P.max_poly_terms >= 256);
   int wide_ctas = 0;
   if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) {
     if (h->K->streams_warps_per_sm() <= 0) return fail(h, "bb_run: the stream runner does not fit this device");
@@ -1232,10 +1262,11 @@ int bb_run_export(bb_handle* h, int strategy, int episodes, int seed_base, const
     A.ctl_reducers = h->wide_mode == 8 ? 32 : 256;
     // every generator a binomial distribution draws has two terms, so every polynomial of the run has at most two
     // (DESIGN.md §3).  Staged ideals keep the general runner: nothing records the length of their polynomials.
-    A.two_term = h->two_term && h->P.dist.enabled && h->P.dist.kind == 0;
+    A.two_term = !W && h->two_term && h->P.dist.enabled && h->P.dist.kind == 0;
     if (bi > 0) CK(cudaStreamWaitEvent(s, h->stage[which].prepared, 0));
     const int workers = std::min(h->P.num_envs, count);
-    if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) CK(h->K->run_streams(PB, S, A, workers, s));
+    if (W) CK(h->K->run_policy(PB, S, A, *W, counter0, std::min(workers, policy_wave), s));
+    else if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) CK(h->K->run_streams(PB, S, A, workers, s));
     else if (streams) CK(h->K->run_wide(PB, S, A, std::min(workers, wide_ctas), s));
     else CK(h->K->run(PB, S, A, std::min(workers, h->run_wave[A.two_term]), s));
     CK(cudaEventRecord(h->stage[which].consumed, s));
@@ -1501,6 +1532,25 @@ int bb_rollout(bb_handle* h, int hidden, const float* W1_dev, const float* b1_de
   if (h->P.auto_reset) { rc = pre_refill(h, (cudaStream_t)stream, true); if (rc < 0) return rc; }
   CK(h->K->rollout(h->P, A, h->P.num_envs, (cudaStream_t)stream));
   return 0;
+}
+
+int bb_run_policy(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev,
+                  const float* b2_dev, uint64_t seed, uint64_t counter0, int greedy,
+                  int episodes, int seed_base, const int32_t* seeds_dev, int max_steps, double gamma, int compute_gb,
+                  bb_episode_stats* stats_dev, int32_t* trace_dev, int trace_episodes, int trace_cap, void* stream,
+                  const bb_poly_sink* gb, const bb_poly_sink* basis) {
+  if (!h) return -1;
+  int rc = check_policy(h, hidden, W1_dev, b1_dev, w2_dev, b2_dev);
+  if (rc < 0) return rc;
+  if (episodes < 0 || !stats_dev) return fail(h, "bb_run_policy: bad argument");
+  if (gb && !compute_gb) return fail(h, "bb_run_policy: a gb sink needs compute_gb != 0");
+  rc = check_sink(h, gb, "gb", "bb_run_policy");
+  if (rc == 0) rc = check_sink(h, basis, "basis", "bb_run_policy");
+  if (rc < 0) return rc;
+  BBPolicy W;
+  W.hidden = hidden; W.W1 = W1_dev; W.b1 = b1_dev; W.w2 = w2_dev; W.b2 = b2_dev; W.seed = seed; W.greedy = greedy ? 1 : 0;
+  return run_batches(h, 0, &W, counter0, episodes, seed_base, seeds_dev, 0, max_steps, gamma, compute_gb, stats_dev, trace_dev,
+                     trace_episodes, trace_cap, stream, gb, basis);
 }
 
 static int unpack_polys(bb_handle* h, const std::vector<uint64_t>& keys, const std::vector<uint32_t>& cf,

@@ -17,6 +17,8 @@
  *   buchberger(F, selection, ...)  buchberger.h:127-147     bb_run_export (whole episodes, all nine SelectionTypes;
  *                                                             every episode's reduced basis into a device sink), bb_run
  *   policy_model(state) + categorical   pg.py:323-326       bb_policy_pmlp / bb_rollout (PMLP head, networks.py:522-571)
+ *   pg.Agent.run_episode to completion  pg.py:451-472       bb_run_policy (whole episodes, the PMLP head selecting, with
+ *                                                             bb_run_export's records, traces and sinks)
  *   BuchbergerEnv::G, ::P   buchberger.h:195-196            bb_download_basis, bb_pairs
  *   buchberger(...) -> interreduce(minimalize(G))           bb_final_gb
  *       buchberger.cpp:265
@@ -420,6 +422,22 @@ int bb_policy_pmlp(bb_handle* h, int hidden, const float* W1_dev, const float* b
 int bb_rollout(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev, const float* b2_dev,
                uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev, float* logprob_dev,
                float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax, void* stream);
+
+/* bb_run_policy: bb_run_export with the PMLP head of bb_policy_pmlp choosing every pair instead of a SelectionType -- the
+ * trained agent evaluated on whole episodes (pg.Agent.run_episode, pg.py:451-472, run to completion), with the same
+ * records, traces, sinks, batching, bb_prepare matching, banks, max_steps truncation and bb_counters as bb_run_export.
+ * Weights, hidden and greedy are those of bb_policy_pmlp (greedy: argmax, the lowest row on ties).  Step t of episode e of
+ * the call draws its uniform from stream seed + (offset + e) and counter counter0 + t, where offset is bb_set_episode_offset's
+ * value: a record depends only on the episode's global index, never on the slot, the handle's size, the batching or the
+ * sharding.  So environment e of the step API, seeded seed_base + e and driven by bb_policy_pmlp(seed, counter0 + t) + bb_step
+ * at its step t, plays exactly episode e of bb_run_policy(seed, counter0, ..., seed_base).  Every step uses the
+ * materialising reduction, whatever bb_set_wide and bb_set_two_term say (identical episodes).  Fails (nothing enqueued) for
+ * what bb_policy_pmlp refuses, episodes < 0, stats_dev == NULL, a gb sink with compute_gb == 0, and a bad sink. */
+int bb_run_policy(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev,
+                  const float* b2_dev, uint64_t seed, uint64_t counter0, int greedy,
+                  int episodes, int seed_base, const int32_t* seeds_dev, int max_steps, double gamma, int compute_gb,
+                  bb_episode_stats* stats_dev, int32_t* trace_dev, int trace_episodes, int trace_cap, void* stream,
+                  const bb_poly_sink* gb, const bb_poly_sink* basis);
 
 /* bb_discount: discounted suffix sums inside episode segments, the primitive of pg.discount_rewards (pg.py:18-39) and
  * of the generalised advantage estimates (pg.compute_advantages, pg.py:42-78) on the [N, T] trajectories bb_rollout
