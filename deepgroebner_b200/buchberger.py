@@ -677,9 +677,9 @@ class BuchbergerEngine:
 
     def set_wide(self, mode=-1):
         """How run_episodes reduces (bb_set_wide): -1 auto, 0 materialised dividend, 1 dividend as a set of streams run by
-        one CTA per environment (long polynomials), 4 the same by one warp per environment; 2 / 3 (as 1) and 5 / 6 (as 4)
-        with 6 / 48 stream slots (consolidation path), 7 as 1 with 8 register slots (shared-memory table), 8 as 1 with
-        32 reducers in the control warp's registers (memory scan of the rest).  Results are identical; only speed differs."""
+        one CTA per environment (long polynomials); 2 / 3 as 1 with 6 / 48 stream slots (consolidation path), 7 as 1 with
+        8 register slots (shared-memory table), 8 as 1 with 32 reducers in the control warp's registers (memory scan of the
+        rest); 4 / 5 / 6 are kept for compatibility and equal 1 / 2 / 3.  Results are identical; only speed differs."""
         self._ck(self.lib.bb_set_wide(self.h, int(mode)), "bb_set_wide")
 
     def set_prepare_mode(self, by_warp=False):

@@ -9,17 +9,18 @@
 //   k_run      persistent: episodes pulled from a queue and run to completion with on-device selection
 //              (the loop of buchberger(), buchberger.cpp:243-263); finished slots refill at once.
 //   k_run_policy the same runner with the pairs policy head (bb_policy.cuh) choosing the pairs (bb_run_policy)
+//   k_run_wide the same runner with one CTA per environment slot and reduce() by streams (bb_wide.cuh: long polynomials)
 //   k_final_gb interreduce(minimalize(G))    buchberger.cpp:102-122
 //   k_reduce   reduce(g, F)                  buchberger.cpp:24-49 on caller-supplied divisor lists and dividends (bb_reduce)
 #pragma once
+#include <type_traits>
+
 #include "bb_device.cuh"
 #include "bb_policy.cuh"
-#include "bb_streams.cuh"
 #if defined(BBW_CLOCK) || defined(BBW_INSTR)
 #include <cstdio>
 #endif
 #include "bb_wide.cuh"
-#include "bb_rstreams.cuh"
 
 #ifndef BB_WARPS
 #define BB_WARPS 8
@@ -59,7 +60,7 @@ struct BBRunArgs {
   int32_t* trace;
   int trace_eps, trace_cap;
   int prepare_by_warp;  // 1: k_prepare (one warp per episode) even where k_prepare_lanes applies (tests compare the two)
-  int stream_kmax;   // stream slots a step's reduction may use (BBS_KMAX; less under bb_set_wide(2 / 3 / 5 / 6)), see bb_streams.cuh
+  int stream_kmax;   // k_run_wide: stream slots a step's reduction may use (BBS_KMAX; 6 / 48 under bb_set_wide(2 / 3)), see bb_wide.cuh
   int stream_regs;   // k_run_wide: how many of them are register slots (BBW_SLOTS; 8 under bb_set_wide(7))
   int ctl_reducers;  // k_run_wide: reducers of G_ in the control warp's registers (256; 32 under bb_set_wide(8))
   int* queue;        // [0]: next queue position; [BB_LPT_HIST .. +BB_LPT_BUCKETS): histogram of the cost keys of the batch, then as many cursors
@@ -161,10 +162,7 @@ struct BBKernelTable {
   cudaError_t (*final_gb)(const BBParams&, int slot, int* ok_out, cudaStream_t);
   cudaError_t (*prepare)(const BBParams& stage, const BBRunArgs&, cudaStream_t);  // k_prepare + k_order
   cudaError_t (*run)(const BBParams&, const BBParams& stage, const BBRunArgs&, int nwarps, cudaStream_t);
-  // the same runner with reduce() by streams (bb_streams.cuh: long polynomials)
-  cudaError_t (*run_streams)(const BBParams&, const BBParams& stage, const BBRunArgs&, int nwarps, cudaStream_t);
-  int (*streams_warps_per_sm)(void);   // 0 if it does not fit
-  // ... and by one CTA per environment (bb_wide.cuh: shortest chain of additions); nctas worker CTAs
+  // the same runner with reduce() by streams and one CTA per environment (bb_wide.cuh: long polynomials); nctas worker CTAs
   cudaError_t (*run_wide)(const BBParams&, const BBParams& stage, const BBRunArgs&, int nctas, cudaStream_t);
   int (*wide_ctas_per_sm)(void);
   cudaError_t (*value)(const BBParams&, const BBParams& fork, const BBValueArgs&, int nwarps, cudaStream_t);
@@ -742,13 +740,12 @@ __global__ void __launch_bounds__(BB_PREP_THREADS, BB_PREP_MIN_BLOCKS) k_prefill
 
 // The loop of buchberger() (buchberger.cpp:243-263) on one environment: select, step, accumulate the trace checksum and
 // the discounted return (discounted_return += discount * reward; discount *= gamma, :250-251) until P is empty.
-// STREAMS: reduce() by streams (bb_streams.cuh), ws / st = the warp's stream state and table.  TWO: see warp_step.
-// UPL > 0: the pairs policy head (bb_policy.cuh, H = 32 * UPL, weights at wsm) selects instead of `strategy`; step t draws
-// its uniform from (W->seed + stream, counter0 + t), stream = the episode's global index.
-template <int NV, bool STREAMS, bool TWO = false, int UPL = 0>
+// TWO: see warp_step.  UPL > 0: the pairs policy head (bb_policy.cuh, H = 32 * UPL, weights at wsm) selects instead of
+// `strategy`; step t draws its uniform from (W->seed + stream, counter0 + t), stream = the episode's global index.
+template <int NV, bool TWO = false, int UPL = 0>
 __device__ __forceinline__ void run_episode(const BBParams& P, Env& e, int strategy, int max_steps, double gamma,
                                             BBEpisodeAcc& acc, Ctr& ct, int& steps, int& adds, int4* trace, int trace_cap,
-                                            RegStreams* ws, const BBPolicy* W = nullptr, const float* wsm = nullptr,
+                                            const BBPolicy* W = nullptr, const float* wsm = nullptr,
                                             unsigned long long stream = 0, unsigned long long counter0 = 0) {
   const int lane = bb_lane();
   while (e.status == BB_STATUS_RUNNING && (max_steps == 0 || steps < max_steps)) {
@@ -761,9 +758,7 @@ __device__ __forceinline__ void run_episode(const BBParams& P, Env& e, int strat
       prow = warp_select<NV>(P, e, strategy, &acc.sel_rng);
     }
     uint32_t pr;
-    int a;
-    if (STREAMS) a = warp_step_rstreams<NV>(P, e, *ws, prow, pr, ct);
-    else a = warp_step<NV, TWO>(P, e, prow, pr, ct);
+    const int a = warp_step<NV, TWO>(P, e, prow, pr, ct);
     if (lane == 0) {
       const int pi = pr & 0xffffu, pj = pr >> 16;
       acc.th = trace_hash_step(acc.th, pr, a);
@@ -801,7 +796,7 @@ __device__ __noinline__ void warp_export_episode(const BBParams& P, const BBRunA
 // site in its loop measured 3 % on configs[1]).  TWO: the two-term step (warp_step), for runs whose ideals are binomial.
 // UPL > 0: the policy head selects (run_episode; W, wsm: the weights and their shared-memory image, counter0: the counter
 // of step 0).
-template <int NV, bool STREAMS, int WARPS, bool EXPORT, bool TWO = false, int UPL = 0>
+template <int NV, int WARPS, bool EXPORT, bool TWO = false, int UPL = 0>
 __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S, const BBRunArgs& A,
                                            const BBPolicy* W = nullptr, const float* wsm = nullptr,
                                            unsigned long long counter0 = 0) {
@@ -814,8 +809,6 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
   BBEpisodeAcc& acc = acc_sh[threadIdx.x >> 5];
   const int slot = (blockIdx.x * (WARPS * 32) + threadIdx.x) >> 5;
   const int lane = bb_lane();
-  RegStreams ws;
-  ws.clear(); ws.kmax = A.stream_kmax < BBR_ROWS * 32 ? A.stream_kmax : BBR_ROWS * 32; ws.cz = 0;
   if (slot < P.num_envs) {
     Ctr ct; ct.clear();
     for (;;) {
@@ -835,9 +828,9 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
       int steps = 0, adds = 0;
       if (lane == 0) { acc.th = 0ull; acc.ret = 0.0; acc.disc = 1.0; acc.sel_rng = rng_seed(A.sel_seed_base + (A.ep_offset + ep) * A.sel_seed_stride); }
       __syncwarp();
-      run_episode<NV, STREAMS, TWO, UPL>(P, e, A.strategy, A.max_steps, A.gamma, acc, ct, steps, adds,
+      run_episode<NV, TWO, UPL>(P, e, A.strategy, A.max_steps, A.gamma, acc, ct, steps, adds,
                                (A.trace && ep < A.trace_eps) ? reinterpret_cast<int4*>(A.trace) + (size_t)ep * A.trace_cap : nullptr,
-                               A.trace_cap, &ws, W, wsm, (unsigned long long)(A.ep_offset + ep), counter0);
+                               A.trace_cap, W, wsm, (unsigned long long)(A.ep_offset + ep), counter0);
       const int nonzero = e.nG - g_start, zero = steps - nonzero;
       env_store(P, slot, e);
       __syncwarp();
@@ -887,7 +880,7 @@ __device__ __forceinline__ void run_worker(const BBParams& P, const BBParams& S,
 template <int NV, bool EXPORT = false, bool TWO = false>
 __global__ void __launch_bounds__(TWO ? BB_TWO_WARPS * 32 : BB_THREADS, TWO ? BB_TWO_MIN_BLOCKS : BB_MIN_BLOCKS)
 k_run(const __grid_constant__ BBParams P, const __grid_constant__ BBParams S, const __grid_constant__ BBRunArgs A) {
-  run_worker<NV, false, TWO ? BB_TWO_WARPS : BB_WARPS, EXPORT, TWO>(P, S, A);
+  run_worker<NV, TWO ? BB_TWO_WARPS : BB_WARPS, EXPORT, TWO>(P, S, A);
 }
 
 // The same runner with the pairs policy head choosing the pairs (bb_run_policy): k_rollout's head and step (the general
@@ -900,21 +893,7 @@ k_run_policy(const __grid_constant__ BBParams P, const __grid_constant__ BBParam
              const __grid_constant__ BBPolicy W, unsigned long long counter0) {
   extern __shared__ float wsm[];
   policy_load_weights(W, P.cols, wsm);
-  run_worker<NV, false, BB_WARPS, true, false, UPL>(P, S, A, &W, wsm, counter0);
-}
-
-// The same runner for long polynomials: reduce() by streams, the warp's stream table in dynamic shared memory.
-#ifndef BBS_WARPS
-#define BBS_WARPS 4
-#endif
-#ifndef BBS_MIN_CTAS
-#define BBS_MIN_CTAS 2
-#endif
-template <int NV, bool EXPORT = false>
-__global__ void __launch_bounds__(BBS_WARPS * 32, BBS_MIN_CTAS) k_run_streams(const __grid_constant__ BBParams P,
-                                                                             const __grid_constant__ BBParams S,
-                                                                             const __grid_constant__ BBRunArgs A) {
-  run_worker<NV, true, BBS_WARPS, EXPORT>(P, S, A);
+  run_worker<NV, BB_WARPS, true, false, UPL>(P, S, A, &W, wsm, counter0);
 }
 
 // block-strided copy of n 32-bit words
@@ -1089,7 +1068,7 @@ __global__ void __launch_bounds__(BB_THREADS, BB_MIN_BLOCKS) k_value(const __gri
         if (lane == 0) { acc.th = 0ull; acc.ret = 0.0; acc.disc = 1.0; acc.sel_rng = rng_seed(seed); }
         __syncwarp();
         int steps = 0, adds = 0;
-        run_episode<NV, false>(F, e, strategy, A.max_steps, A.gamma, acc, ct, steps, adds, nullptr, 0, nullptr);
+        run_episode<NV>(F, e, strategy, A.max_steps, A.gamma, acc, ct, steps, adds, nullptr, 0);
         __syncwarp();
         ret = acc.ret;
         if (e.status != BB_STATUS_DONE && !(A.max_steps && steps >= A.max_steps)) ret = __longlong_as_double(0x7ff8000000000000LL);  // fault: NaN
@@ -1421,24 +1400,6 @@ struct BBLaunch {
     }
     return cudaGetLastError();
   }
-  static size_t streams_smem() { return 0; }   // every stream lives in registers (bb_rstreams.cuh)
-  static int streams_warps_per_sm() {
-    const size_t sm = streams_smem();
-    if (cudaFuncSetAttribute(k_run_streams<NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess) return 0;
-    int blocks = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run_streams<NV>, BBS_WARPS * 32, sm) != cudaSuccess) return 0;
-    return blocks * BBS_WARPS;
-  }
-  static cudaError_t run_streams(const BBParams& P, const BBParams& S, const BBRunArgs& A, int nwarps, cudaStream_t s) {
-    const size_t sm = streams_smem();
-    const bool ex = A.gb_sink.lens_dev || A.basis_sink.lens_dev;
-    cudaError_t e = cudaFuncSetAttribute(ex ? k_run_streams<NV, true> : k_run_streams<NV>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    if (e != cudaSuccess) return e;
-    if (ex) k_run_streams<NV, true><<<(nwarps + BBS_WARPS - 1) / BBS_WARPS, BBS_WARPS * 32, sm, s>>>(P, S, A);
-    else k_run_streams<NV><<<(nwarps + BBS_WARPS - 1) / BBS_WARPS, BBS_WARPS * 32, sm, s>>>(P, S, A);
-    return cudaGetLastError();
-  }
   static int wide_ctas_per_sm() {
     const size_t sm = sizeof(WideStreams);
     if (cudaFuncSetAttribute(k_run_wide<NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess) return 0;
@@ -1458,47 +1419,42 @@ struct BBLaunch {
     return cudaGetLastError();
   }
   static size_t policy_smem(const BBParams& P, int hidden) { return sizeof(float) * (size_t)policy_smem_floats(P.cols, hidden); }
-  template <int UPL>
-  static cudaError_t policy_upl(const BBParams& P, const BBPolicy& W, unsigned long long counter, int32_t* actions, float* logp,
-                                float* logits, int pmax, int g, size_t sm, cudaStream_t s) {
-    if (sm > 48 * 1024) {
-      cudaError_t e = cudaFuncSetAttribute(k_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-      if (e != cudaSuccess) return e;
+  // The policy kernels exist for hidden = 32 * UPL, UPL in {1, 2, 4, 8}: body(std::integral_constant<int, UPL>()) for the UPL
+  // of `hidden`, `bad` for any other width.
+  template <class R, class Body>
+  static R with_upl(int hidden, R bad, Body body) {
+    switch (hidden >> 5) {
+      case 1: return body(std::integral_constant<int, 1>());
+      case 2: return body(std::integral_constant<int, 2>());
+      case 4: return body(std::integral_constant<int, 4>());
+      case 8: return body(std::integral_constant<int, 8>());
     }
-    k_policy<NV, UPL><<<g, BB_THREADS, sm, s>>>(P, W, counter, actions, logp, logits, pmax);
-    return cudaGetLastError();
+    return bad;
   }
   static cudaError_t policy(const BBParams& P, const BBPolicy& W, unsigned long long counter, int32_t* actions, float* logp,
                             float* logits, int pmax, int nwarps, cudaStream_t s) {
     const size_t sm = policy_smem(P, W.hidden);
-    const int g = grid_for_warps(nwarps);
-    switch (W.hidden >> 5) {
-      case 1: return policy_upl<1>(P, W, counter, actions, logp, logits, pmax, g, sm, s);
-      case 2: return policy_upl<2>(P, W, counter, actions, logp, logits, pmax, g, sm, s);
-      case 4: return policy_upl<4>(P, W, counter, actions, logp, logits, pmax, g, sm, s);
-      case 8: return policy_upl<8>(P, W, counter, actions, logp, logits, pmax, g, sm, s);
-    }
-    return cudaErrorInvalidValue;
-  }
-  template <int UPL>
-  static cudaError_t rollout_upl(const BBParams& P, const BBRolloutArgs& A, int g, size_t sm, cudaStream_t s) {
-    if (sm > 48 * 1024) {
-      cudaError_t e = cudaFuncSetAttribute(k_rollout<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-      if (e != cudaSuccess) return e;
-    }
-    k_rollout<NV, UPL><<<g, BB_THREADS, sm, s>>>(P, A);
-    return cudaGetLastError();
+    return with_upl(W.hidden, cudaErrorInvalidValue, [&](auto upl) {
+      constexpr int UPL = decltype(upl)::value;
+      if (sm > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(k_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        if (e != cudaSuccess) return e;
+      }
+      k_policy<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, W, counter, actions, logp, logits, pmax);
+      return cudaGetLastError();
+    });
   }
   static cudaError_t rollout(const BBParams& P, const BBRolloutArgs& A, int nwarps, cudaStream_t s) {
     const size_t sm = policy_smem(P, A.W.hidden);
-    const int g = grid_for_warps(nwarps);
-    switch (A.W.hidden >> 5) {
-      case 1: return rollout_upl<1>(P, A, g, sm, s);
-      case 2: return rollout_upl<2>(P, A, g, sm, s);
-      case 4: return rollout_upl<4>(P, A, g, sm, s);
-      case 8: return rollout_upl<8>(P, A, g, sm, s);
-    }
-    return cudaErrorInvalidValue;
+    return with_upl(A.W.hidden, cudaErrorInvalidValue, [&](auto upl) {
+      constexpr int UPL = decltype(upl)::value;
+      if (sm > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(k_rollout<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        if (e != cudaSuccess) return e;
+      }
+      k_rollout<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, A);
+      return cudaGetLastError();
+    });
   }
   // resident warps per SM of the general (two == 0) or the two-term k_run (the instantiations with sinks have the same bounds)
   static int run_warps_per_sm(int two) {
@@ -1514,49 +1470,34 @@ struct BBLaunch {
     k_reduce<NV><<<grid_for_warps(nwarps), BB_THREADS, 0, s>>>(P, A);
     return cudaGetLastError();
   }
-  template <int UPL>
-  static cudaError_t run_policy_upl(const BBParams& P, const BBParams& S, const BBRunArgs& A, const BBPolicy& W,
-                                    unsigned long long counter0, int nwarps, cudaStream_t s) {
-    const size_t sm = policy_smem(P, W.hidden);
-    if (sm > 48 * 1024) {
-      cudaError_t e = cudaFuncSetAttribute(k_run_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-      if (e != cudaSuccess) return e;
-    }
-    k_run_policy<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, S, A, W, counter0);
-    return cudaGetLastError();
-  }
   static cudaError_t run_policy(const BBParams& P, const BBParams& S, const BBRunArgs& A, const BBPolicy& W,
                                 unsigned long long counter0, int nwarps, cudaStream_t s) {
-    switch (W.hidden >> 5) {
-      case 1: return run_policy_upl<1>(P, S, A, W, counter0, nwarps, s);
-      case 2: return run_policy_upl<2>(P, S, A, W, counter0, nwarps, s);
-      case 4: return run_policy_upl<4>(P, S, A, W, counter0, nwarps, s);
-      case 8: return run_policy_upl<8>(P, S, A, W, counter0, nwarps, s);
-    }
-    return cudaErrorInvalidValue;
-  }
-  template <int UPL>
-  static int run_policy_warps_upl(size_t sm) {
-    if (sm > 48 * 1024 &&
-        cudaFuncSetAttribute(k_run_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess)
-      return -1;
-    int blocks = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run_policy<NV, UPL>, BB_THREADS, sm) != cudaSuccess) return -1;
-    return blocks * BB_WARPS;
+    const size_t sm = policy_smem(P, W.hidden);
+    return with_upl(W.hidden, cudaErrorInvalidValue, [&](auto upl) {
+      constexpr int UPL = decltype(upl)::value;
+      if (sm > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(k_run_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        if (e != cudaSuccess) return e;
+      }
+      k_run_policy<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, S, A, W, counter0);
+      return cudaGetLastError();
+    });
   }
   static int run_policy_warps_per_sm(const BBParams& P, int hidden) {
     const size_t sm = policy_smem(P, hidden);
-    switch (hidden >> 5) {
-      case 1: return run_policy_warps_upl<1>(sm);
-      case 2: return run_policy_warps_upl<2>(sm);
-      case 4: return run_policy_warps_upl<4>(sm);
-      case 8: return run_policy_warps_upl<8>(sm);
-    }
-    return -1;
+    return with_upl(hidden, -1, [&](auto upl) {
+      constexpr int UPL = decltype(upl)::value;
+      if (sm > 48 * 1024 &&
+          cudaFuncSetAttribute(k_run_policy<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess)
+        return -1;
+      int blocks = 0;
+      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, k_run_policy<NV, UPL>, BB_THREADS, sm) != cudaSuccess) return -1;
+      return blocks * BB_WARPS;
+    });
   }
   static const BBKernelTable* table() {
     static const BBKernelTable t = {NV, KL<NV>::w, KL<NV>::dw, KL<NV>::dshift, KL<NV>::eshift,
-                                    &reset, &step, &step_obs, &serve, &prefill, &select, &observe, &final_gb, &prepare, &run, &run_streams, &streams_warps_per_sm, &run_wide, &wide_ctas_per_sm, &value, &policy,
+                                    &reset, &step, &step_obs, &serve, &prefill, &select, &observe, &final_gb, &prepare, &run, &run_wide, &wide_ctas_per_sm, &value, &policy,
                                     &rollout,
                                     &run_warps_per_sm, &reduce, &run_policy, &run_policy_warps_per_sm};
     return &t;

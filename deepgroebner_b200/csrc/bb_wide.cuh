@@ -1,4 +1,39 @@
-// bb_wide.cuh -- the stream reducer (bb_streams.cuh) run by a whole CTA (BBW_WARPS warps) on ONE environment, sm_100a.
+// bb_wide.cuh -- reduce() for LONG polynomials (cyclic-n and other non-binomial ideals, BASELINE configs[4]) without
+// ever materialising the dividend, run by a whole CTA (BBW_WARPS warps) on ONE environment, sm_100a.
+//
+// warp_reduce / warp_merge (bb_device.cuh) are built for binomial ideals, where a polynomial is two terms.  On cyclic-6
+// (SURVEY 8 a4/a6) a dividend of ~100 (up to ~550) terms is reduced ~83 times per step by polynomials of ~37 terms, and an
+// episode is a serial chain of ~80 000 such additions (697 000 in the longest of 1024): materialising
+// h <- h - (LT h / LT f) f (buchberger.cpp:33-35) costs O(|h| + |f|) work per addition and, whatever the parallel merge,
+// several dependent passes over memory.  Round 2 built and measured three block-wide merges for it (merge path, a
+// two-barrier bitmap merge, streams with one barrier per lead term: 1.85 / 1.5 / 1.5 us per addition) before settling on:
+//
+//   h = sum over STREAMS i of  nc_i * m_i * tail(f_i)        (the S-polynomial's two halves, then one stream per addition)
+//
+// A stream is a cursor into the term arena plus its multiplier; its current term (scaled) is its HEAD.  The lead term of
+// h is the smallest head key (keys ascend as monomials descend) with the SUM of the coefficients of every head that
+// carries it; a zero sum is a cancelled monomial and is skipped.  This is the division algorithm of buchberger.cpp:24-49
+// with Polynomial operator+ (polynomials.cpp:148-177) evaluated lazily: the sequence of lead terms, the reducer chosen
+// for each (first in G_ whose lead monomial divides), the number of additions (the reward) and the remainder are those
+// of the reference, term for term and bit for bit -- only the order in which coefficients are summed differs, and
+// addition mod p is associative.  An addition costs O(1) and each term of a reducer is touched once.
+//
+// One ROUND per lead term M: (a) M's first divisor among the reducer lead monomials (buchberger.cpp:27-32), (b) every
+// stream whose head is M advances -- the next raw term was prefetched into registers a round earlier -- and each thread
+// takes the minimum over its heads with the coefficient sum at it, (c) REDUX reductions give the next lead term.  A divisor
+// f opens a new stream whose head comes straight from f's head record (no dependent load).  Measured on the longest
+// cyclic-6 episode (697 000 additions): 955 000 rounds (73 % additions, 21 % remainder terms, 6 % cancelled monomials)
+// for 26 M stream terms, i.e. ~27 streams advance per round and a few hundred are live: the monomials of h and of the
+// reducers' multiples coincide massively, which is why h stays short while the streams are many.
+//
+// A stream slot is free when its head key is all ones; a new stream takes a free slot, so the tables stay as small as the
+// number of LIVE streams.  If no slot is free, h is consolidated: every pending term is written in order to a scratch list
+// behind the slot's term arena and h goes on as ONE stream over it (bb_set_wide(2 / 3) cap the slots so that the tests
+// reach this).
+//
+// Episode records are bit-identical to the materialising runner's (bb_set_wide(0): warp_merge / warp_reduce, an
+// independent second implementation); of the traffic counters, terms_read / terms_written (|h| per addition) are not
+// observable without materialising h and count the reducers' lengths only.
 //
 // A cyclic-6 launch is as long as its longest episode (697 000 dependent additions in the longest of 1024 seeded-Random
 // episodes), so what decides it is the latency of one ROUND (one lead monomial of the dividend: its coefficient, its
@@ -21,7 +56,7 @@
 //
 // A new stream takes the first free register slot of the block (the fold reports it), so the register slots hold the LIVE
 // streams; only when all BBW_SLOTS are live does a stream go to the shared-memory table behind them (append only;
-// scanned by its owner thread each round), and only when that is full too is h consolidated (bb_streams.cuh).
+// scanned by its owner thread each round), and only when that is full too is h consolidated (see above).
 // bb_set_wide(2 / 3): 6 / 48 register slots and no table (consolidations every few additions); bb_set_wide(7): 8 register
 // slots and the whole table (the shared-memory path on every step); bb_set_wide(8): the control warp keeps 32 reducers in
 // registers instead of 256 (its scan of the rest of G_ in memory on most rounds).
@@ -29,7 +64,23 @@
 // Every routine that touches the per-thread state is inlined: a call would take the state's address and move it from
 // registers to local memory (LDL / STL on the chain of every round: 1.35 -> 1.06 us per addition when that was removed).
 #pragma once
-#include "bb_streams.cuh"
+#include "bb_device.cuh"
+
+#ifndef BBS_KMAX
+#define BBS_KMAX 1024           // BBRunArgs::stream_kmax when bb_set_wide does not cap the streams
+#endif
+#define BBS_NONE 0xffffffffu
+
+// The scratch list of a consolidation lies BEHIND the term arena of the slot (bbenv.cu lays hkey right after tkey and
+// hcoef right after tcoef, max_terms a multiple of 8), so term index max_terms + i addresses scratch term i through the
+// same two base pointers and a stream's cursor needs no flag.  Two halves of max_poly_terms terms: a consolidation writes
+// one while the stream over the other is still being read.
+
+__device__ __forceinline__ uint32_t bbf_reduce(const BBField& F, uint32_t x) {   // x mod p for any x < 2^32
+  const uint32_t q = __umulhi(x, F.mu);
+  const uint32_t r = x - q * F.p;
+  return r >= F.p ? r - F.p : r;
+}
 
 #ifndef BBW_WARPS
 #define BBW_WARPS 8
@@ -282,7 +333,7 @@ __device__ __forceinline__ void wide_open(WideState& ws, WideStreams& st, const 
 #endif
 }
 
-// Consolidation (bb_streams.cuh): h from its lead monomial M on goes to scratch half ws.cz in order, one stream over it
+// Consolidation (see the top of this file): h from its lead monomial M on goes to scratch half ws.cz in order, one stream over it
 // (register slot 0) remains and M becomes its head monomial, all ones if nothing is left.  Returns the number of terms, -1
 // if they do not fit `cap`.
 template <int NV>

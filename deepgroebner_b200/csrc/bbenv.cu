@@ -230,7 +230,7 @@ struct bb_handle {
   int two_term;    // bb_run: 1 = the two-term runner for binomial distributions (default), 0 = always the general one
   int run_wave[2];  // resident warps of the general (0) and the two-term (1) k_run on the device: the most either launches
   int policy_wave[4];  // resident warps of k_run_policy for hidden 32, 64, 128, 256 (0: not asked yet)
-  int wide_mode;   // bb_run: reduce() by streams: -1 = when the capacities ask for long polynomials, 0 = never, 1 = always, 2 / 3 = always, small tables
+  int wide_mode;   // bb_run: reduce() by streams (k_run_wide): -1 = when the capacities ask for long polynomials, 0 = never, 1 = always, 2 / 3 / 7 / 8 = always, test configurations (bb_set_wide); 4 / 5 / 6 = 1 / 2 / 3
   // host mirrors of the distribution tables
   std::vector<double> cp;
   std::vector<char> staged;   // bb_set_ideals: which environments hold a staged ideal
@@ -261,7 +261,7 @@ static cudaError_t dev_alloc(bb_handle* h, T** p, size_t count) {
 
 // One contiguous arena per slot from the capacities in P: 8-byte arrays first, every array 32-byte aligned, stride a
 // multiple of 128.  Returns false if a slot would exceed 2 GiB.  hkey lies directly behind tkey and hcoef directly behind
-// tcoef (max_terms is a multiple of 8, so no padding): scratch term i is term max_terms + i of the arena (bb_streams.cuh).
+// tcoef (max_terms is a multiple of 8, so no padding): scratch term i is term max_terms + i of the arena (bb_wide.cuh).
 static bool layout_arena(BBParams& P) {
   size_t o = 0;
   auto take = [&o](size_t bytes) { size_t at = o; o = (o + bytes + 31) & ~(size_t)31; return (unsigned)at; };
@@ -1196,14 +1196,16 @@ static int run_batches(bb_handle* h, int strategy, const BBPolicy* W, unsigned l
     }
     policy_wave = w;
   }
-  // long polynomials (general capacities): reduce() by streams (bb_streams.cuh), by default with one CTA per
-  // environment (bb_wide.cuh: the shortest chain of additions); mode 4: one warp per environment.  The policy runner always
-  // steps with the materialising reduction: its episodes are dominated by the head.
-  const bool streams = !W && h->wide_mode != 0 && (h->wide_mode >= 1 || h->P.max_poly_terms >= 256);
+  // long polynomials (general capacities): reduce() by streams with one CTA per environment (bb_wide.cuh: the shortest
+  // chain of additions).  Modes 4 / 5 / 6 are kept for compatibility and run as 1 / 2 / 3.  The policy runner always steps
+  // with the materialising reduction: its episodes are dominated by the head.
+  const int mode = h->wide_mode >= 4 && h->wide_mode <= 6 ? h->wide_mode - 3 : h->wide_mode;
+  const bool streams = !W && mode != 0 && (mode >= 1 || h->P.max_poly_terms >= 256);
+  const int stream_kmax = mode == 2 ? 6 : (mode == 3 ? 48 : BBS_KMAX);
+  const int stream_regs = mode == 7 ? 8 : stream_kmax;
+  const int ctl_reducers = mode == 8 ? 32 : 256;
   int wide_ctas = 0;
-  if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) {
-    if (h->K->streams_warps_per_sm() <= 0) return fail(h, "bb_run: the stream runner does not fit this device");
-  } else if (streams) {
+  if (streams) {
     wide_ctas = h->K->wide_ctas_per_sm() * h->sm_count;
     if (wide_ctas <= 0) return fail(h, "bb_run: the CTA-per-environment stream runner does not fit this device");
   }
@@ -1257,16 +1259,13 @@ static int run_batches(bb_handle* h, int strategy, const BBPolicy* W, unsigned l
     if (gb) A.gb_sink = *gb;
     if (basis) A.basis_sink = *basis;
     A.trace = trace_dev; A.trace_eps = trace_dev ? trace_episodes : 0; A.trace_cap = trace_cap;
-    A.stream_kmax = (h->wide_mode == 2 || h->wide_mode == 5) ? 6 : ((h->wide_mode == 3 || h->wide_mode == 6) ? 48 : BBS_KMAX);
-    A.stream_regs = h->wide_mode == 7 ? 8 : A.stream_kmax;
-    A.ctl_reducers = h->wide_mode == 8 ? 32 : 256;
+    A.stream_kmax = stream_kmax; A.stream_regs = stream_regs; A.ctl_reducers = ctl_reducers;
     // every generator a binomial distribution draws has two terms, so every polynomial of the run has at most two
     // (DESIGN.md §3).  Staged ideals keep the general runner: nothing records the length of their polynomials.
     A.two_term = !W && h->two_term && h->P.dist.enabled && h->P.dist.kind == 0;
     if (bi > 0) CK(cudaStreamWaitEvent(s, h->stage[which].prepared, 0));
     const int workers = std::min(h->P.num_envs, count);
     if (W) CK(h->K->run_policy(PB, S, A, *W, counter0, std::min(workers, policy_wave), s));
-    else if (streams && h->wide_mode >= 4 && h->wide_mode <= 6) CK(h->K->run_streams(PB, S, A, workers, s));
     else if (streams) CK(h->K->run_wide(PB, S, A, std::min(workers, wide_ctas), s));
     else CK(h->K->run(PB, S, A, std::min(workers, h->run_wave[A.two_term]), s));
     CK(cudaEventRecord(h->stage[which].consumed, s));
@@ -1464,7 +1463,7 @@ int bb_set_obs_nvars(bb_handle* h, int n_obs) {
 
 int bb_set_wide(bb_handle* h, int mode) {
   if (!h) return -1;
-  if (mode < -1 || mode > 8) return fail(h, "bb_set_wide: mode must be -1 (auto), 0 (off), 1 (on), 2 or 3 (on, 6 / 48 stream slots), 4 (on, one warp per environment), 5 or 6 (as 4, 6 / 48 stream slots), 7 (as 1, 8 register slots + the shared-memory table), 8 (as 1, 32 reducers in the control warp's registers)");
+  if (mode < -1 || mode > 8) return fail(h, "bb_set_wide: mode must be -1 (auto), 0 (off), 1 (on), 2 or 3 (on, 6 / 48 stream slots), 4, 5 or 6 (as 1, 2 or 3), 7 (as 1, 8 register slots + the shared-memory table), 8 (as 1, 32 reducers in the control warp's registers)");
   h->wide_mode = mode;
   return 0;
 }

@@ -335,13 +335,13 @@ int bb_set_two_term(bb_handle* h, int on);
  * for the 2-term polynomials of binomial ideals); 1: the dividend is a set of streams into the term arena, one round per
  * lead term and O(1) work per addition (built for long polynomials, e.g. cyclic-n), run by one CTA per environment
  * (shortest chain of additions: a cyclic-6 launch lasts as long as its longest episode; 256 streams in registers, 768
- * more in shared memory); 4: the same by one warp per environment with 128 streams in registers; -1 (default): 1 when
- * the capacities are sized for long polynomials (max_poly_terms >= 256), else 0.  Test modes: 2 / 3 as 1 and 5 / 6 as 4
- * with 6 / 48 stream slots (consolidation of the dividend into a scratch list every few additions); 7 as 1 with 8
- * register slots (the shared-memory table on every step); 8 as 1 with 32 instead of 256 reducers in the control warp's
- * registers (the rest of the reducer list scanned in memory).  Every mode produces bit-identical episodes; this is a
- * performance switch.  Of the bb_counters, terms_read / terms_written count |h| per addition only where h is
- * materialised (mode 0). */
+ * more in shared memory); -1 (default): 1 when the capacities are sized for long polynomials (max_poly_terms >= 256),
+ * else 0.  Test modes: 2 / 3 as 1 with 6 / 48 stream slots (consolidation of the dividend into a scratch list every few
+ * additions); 7 as 1 with 8 register slots (the shared-memory table on every step); 8 as 1 with 32 instead of 256
+ * reducers in the control warp's registers (the rest of the reducer list scanned in memory).  Modes 4, 5 and 6 are kept
+ * for compatibility and are the same as 1, 2 and 3.  Every mode produces bit-identical episodes; this is a performance
+ * switch.  Of the bb_counters, terms_read / terms_written count |h| per addition only where h is materialised
+ * (mode 0). */
 int bb_set_wide(bb_handle* h, int mode);
 
 /* bb_value: BuchbergerEnv::value(strategy, gamma) (buchberger.cpp:332-351) for every environment at once:

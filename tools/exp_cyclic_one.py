@@ -1,4 +1,4 @@
-"""Diagnostic (also the command of the k_run_wide / k_run_streams ncu captures): n cyclic-6 episodes (seeded Random, stream
+"""Diagnostic (also the command of the k_run_wide ncu captures): n cyclic-6 episodes (seeded Random, stream
 seeds seed .. seed + n - 1) on n environment slots under bb_set_wide(mode).  Defaults: the longest of the 1024 episodes of
 the bench (seed 1234 + 241, 696 993 additions) alone = the serial chain that bounds a launch containing it.
   python tools/exp_cyclic_one.py [seed] [mode] [n]"""
