@@ -713,10 +713,17 @@ class BuchbergerEngine:
                                              int(pmax or 0), _stream()), "bb_policy_pmlp")
         return (actions, logp, allp) if return_all else (actions, logp)
 
-    def rollout(self, net, T, counter0=0, greedy=False, store_obs=False, pmax=None, out=None):
+    def rollout(self, net, T, counter0=0, greedy=False, store_obs=False, pmax=None, out=None, value=None, value_gamma=0.99,
+                value_rollouts=None, value_seed=0, value_max_steps=0):
         """T fused steps of every environment (bb_rollout).  Returns a dict of [N, T] cuda tensors: actions, logp,
-        reward, done, lengths (+ obs [N, T, pmax, cols] when store_obs)."""
+        reward, done, lengths (+ obs [N, T, pmax, cols] when store_obs).  value: a selection name or 'sample' (as in
+        value()) -- the dict gains "value", float64 [N, T]: value(value, value_gamma, value_rollouts, value_seed,
+        value_max_steps) of the state each step starts from, computed in the same launch (bb_rollout_value)."""
         N, dev = self.num_envs, self.device
+        vcode = vr = 0
+        if value is not None:
+            vcode = _lib.VALUE_SAMPLE if value == "sample" else _lib.SELECTION[value]
+            vr = (0 if value == "sample" else 1) if value_rollouts is None else value_rollouts
         with torch.cuda.device(dev):
             W1, b1, w2, b2 = net.device_weights(dev, self.cols)
             o = out or {}
@@ -729,10 +736,15 @@ class BuchbergerEngine:
             if store_obs:
                 pmax = int(pmax or 64)
                 obs = o.setdefault("obs", torch.empty((N, T, pmax, self.cols), dtype=torch.int32, device=dev))
-            self._ck(self.lib.bb_rollout(self.h, net.hidden, _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2), int(net.seed),
-                                         int(counter0), int(bool(greedy)), int(T), _ptr(o["actions"]), _ptr(o["logp"]),
-                                         _ptr(o["reward"]), _ptr(o["done"]), _ptr(o["lengths"]), _ptr(obs),
-                                         int(pmax or 0), _stream()), "bb_rollout")
+            args = (self.h, net.hidden, _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2), int(net.seed), int(counter0),
+                    int(bool(greedy)), int(T), _ptr(o["actions"]), _ptr(o["logp"]), _ptr(o["reward"]), _ptr(o["done"]),
+                    _ptr(o["lengths"]), _ptr(obs), int(pmax or 0))
+            if value is None:
+                self._ck(self.lib.bb_rollout(*args, _stream()), "bb_rollout")
+            else:
+                v = o.setdefault("value", torch.empty((N, T), dtype=torch.float64, device=dev))
+                self._ck(self.lib.bb_rollout_value(*args, vcode, float(value_gamma), int(vr), int(value_seed),
+                                                   int(value_max_steps), _ptr(v), _stream()), "bb_rollout_value")
         return o
 
     def copy_env(self, dst_env, src, src_env):

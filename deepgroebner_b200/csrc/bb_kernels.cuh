@@ -168,7 +168,8 @@ struct BBKernelTable {
   cudaError_t (*value)(const BBParams&, const BBParams& fork, const BBValueArgs&, int nwarps, cudaStream_t);
   cudaError_t (*policy)(const BBParams&, const BBPolicy&, unsigned long long counter, int32_t* actions, float* logp,
                         float* logits, int pmax, int nwarps, cudaStream_t);
-  cudaError_t (*rollout)(const BBParams&, const BBRolloutArgs&, int nwarps, cudaStream_t);
+  // k_rollout, or k_rollout_value with V != NULL (F: the fork arena, one slot per environment)
+  cudaError_t (*rollout)(const BBParams&, const BBRolloutArgs&, const BBParams* F, const BBValueArgs* V, int nwarps, cudaStream_t);
   int (*run_warps_per_sm)(int two);   // k_run: general (0) or two-term (1); -1 on error
   cudaError_t (*reduce)(const BBParams&, const BBReduceArgs&, int nwarps, cudaStream_t);
   // k_run with the policy head selecting (bb_run_policy), and its resident warps per SM for P.cols and W.hidden (-1 on error)
@@ -1101,12 +1102,48 @@ __global__ void __launch_bounds__(BB_THREADS) k_policy(const __grid_constant__ B
   if (bb_lane() == 0) { actions[slot] = a; if (logp) logp[slot] = lp; }
 }
 
+// BuchbergerEnv::value of the running environment `slot` (live state e) for bb_rollout_value: what k_value's tasks of one
+// environment do, one rollout after another in this warp, in the environment's own slot of the fork arena F.  Returns the
+// max of the returns, NaN if any rollout ends in a fault (k_value's observable rule).  The live slot is only read; the
+// rollouts' traffic counters are dropped.  Out of line, so the rollout loop around it keeps its own register allocation.
+template <int NV>
+__device__ __noinline__ double warp_state_value(const BBParams& P, const BBParams& F, const BBValueArgs& V, int slot, Env e,
+                                                BBEpisodeAcc& acc) {
+  const int lane = bb_lane();
+  unsigned char* db = F.arena + (size_t)slot * F.slot_stride;
+  const unsigned char* sb = e.base;
+  double v = -__builtin_inf();
+#pragma unroll 1
+  for (int r = 0; r < V.rollouts; r++) {
+    warp_copy_env(F, db, P, sb, e);
+    Env f = e;
+    f.base = db;
+    __syncwarp();
+    int strategy = V.strategy, seed = V.sel_seed_base + r;
+    if (strategy == BB_VALUE_SAMPLE) { strategy = r == 0 ? BB_SELECT_DEGREE : BB_SELECT_RANDOM; seed = V.sel_seed_base + r - 1; }
+    if (lane == 0) { acc.th = 0ull; acc.ret = 0.0; acc.disc = 1.0; acc.sel_rng = rng_seed(seed); }
+    __syncwarp();
+    Ctr ct; ct.clear();
+    int steps = 0, adds = 0;
+    run_episode<NV>(F, f, strategy, V.max_steps, V.gamma, acc, ct, steps, adds, nullptr, 0);
+    __syncwarp();
+    double ret = acc.ret;
+    if (f.status != BB_STATUS_DONE && !(V.max_steps && steps >= V.max_steps)) ret = __longlong_as_double(0x7ff8000000000000LL);  // fault: NaN
+    if (ret != ret) v = ret;   // sticks: NaN < x is false
+    else if (v < ret) v = ret;
+    __syncwarp();
+  }
+  return v;
+}
+
 // Fused rollout (the loop of pg.Agent.run_episode, pg.py:451-472, for every environment at once): each warp runs T
 // steps of its environment -- policy head, categorical sample, step, auto-reset -- with no host round trip and no
-// synchronisation between environments.  Trajectories are written environment-major.
-template <int NV, int UPL>
-__global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout(const __grid_constant__ BBParams P,
-                                                           const __grid_constant__ BBRolloutArgs A) {
+// synchronisation between environments.  Trajectories are written environment-major.  VALUE (k_rollout_value): V->value[e, t]
+// is the value of the state step t starts from (warp_state_value; 0.0 where the environment is not running), F the fork
+// arena and acc the warp's accumulator in shared memory; nothing else the rollout writes changes.
+template <int NV, int UPL, bool VALUE>
+__device__ __forceinline__ void rollout_worker(const BBParams& P, const BBRolloutArgs& A, const BBParams* F,
+                                               const BBValueArgs* V, BBEpisodeAcc* acc) {
   extern __shared__ float wsm[];
   __shared__ unsigned long long sh[BB_WARPS][CT_COUNT];
   hot_init(P);
@@ -1126,6 +1163,10 @@ __global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout(c
       const size_t o = (size_t)slot * A.T + t;
       if (A.lengths && lane == 0) A.lengths[o] = e.nP;
       if (A.obs) warp_observe<NV>(P, e, A.obs + o * A.pmax * P.cols, A.pmax, ct);
+      if constexpr (VALUE) {
+        const double v = e.status == BB_STATUS_RUNNING ? warp_state_value<NV>(P, *F, *V, slot, e, acc[threadIdx.x >> 5]) : 0.0;
+        if (lane == 0) V->value[o] = v;
+      }
       int a = -1; float lp = 0.0f; double r = 0.0;
       if (e.status == BB_STATUS_RUNNING) {
         a = warp_policy<NV, UPL>(P, e, wsm, A.W.greedy, policy_uniform(A.W.seed, (unsigned long long)slot, A.counter0 + t),
@@ -1150,6 +1191,20 @@ __global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout(c
     ct.spill(row);
   }
   counters_flush(P, sh);
+}
+
+template <int NV, int UPL>
+__global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout(const __grid_constant__ BBParams P,
+                                                           const __grid_constant__ BBRolloutArgs A) {
+  rollout_worker<NV, UPL, false>(P, A, nullptr, nullptr, nullptr);
+}
+
+template <int NV, int UPL>
+__global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS)
+k_rollout_value(const __grid_constant__ BBParams P, const __grid_constant__ BBRolloutArgs A, const __grid_constant__ BBParams F,
+                const __grid_constant__ BBValueArgs V) {
+  __shared__ BBEpisodeAcc acc_sh[BB_WARPS];  // value rollouts' accumulators, lane 0 only: kept out of registers
+  rollout_worker<NV, UPL, true>(P, A, &F, &V, acc_sh);
 }
 
 // ------------------------------------------------------------------------------------------------ reduce(g, F)
@@ -1444,10 +1499,19 @@ struct BBLaunch {
       return cudaGetLastError();
     });
   }
-  static cudaError_t rollout(const BBParams& P, const BBRolloutArgs& A, int nwarps, cudaStream_t s) {
+  static cudaError_t rollout(const BBParams& P, const BBRolloutArgs& A, const BBParams* F, const BBValueArgs* V, int nwarps,
+                             cudaStream_t s) {
     const size_t sm = policy_smem(P, A.W.hidden);
     return with_upl(A.W.hidden, cudaErrorInvalidValue, [&](auto upl) {
       constexpr int UPL = decltype(upl)::value;
+      if (V) {
+        if (sm > 48 * 1024) {
+          cudaError_t e = cudaFuncSetAttribute(k_rollout_value<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+          if (e != cudaSuccess) return e;
+        }
+        k_rollout_value<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, A, *F, *V);
+        return cudaGetLastError();
+      }
       if (sm > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_rollout<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         if (e != cudaSuccess) return e;

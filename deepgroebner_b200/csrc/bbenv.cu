@@ -1518,18 +1518,45 @@ int bb_policy_pmlp(bb_handle* h, int hidden, const float* W1_dev, const float* b
 int bb_rollout(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev, const float* b2_dev,
                uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev, float* logprob_dev,
                float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax, void* stream) {
+  return bb_rollout_value(h, hidden, W1_dev, b1_dev, w2_dev, b2_dev, seed, counter0, greedy, T, actions_dev, logprob_dev,
+                          reward_dev, done_dev, lengths_dev, obs_dev, pmax, BB_SELECT_DEGREE, 0.99, 1, 0, 0, nullptr, stream);
+}
+
+int bb_rollout_value(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev,
+                     const float* b2_dev, uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev,
+                     float* logprob_dev, float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax,
+                     int value_strategy, double value_gamma, int value_rollouts, int value_sel_seed, int value_max_steps,
+                     double* value_dev, void* stream) {
   if (!h) return -1;
   int rc = check_policy(h, hidden, W1_dev, b1_dev, w2_dev, b2_dev);
   if (rc < 0) return rc;
   if (T < 1 || (obs_dev && pmax < 1)) return fail(h, "bb_rollout: bad argument");
+  // bb_value's rules
+  if (value_strategy == BB_VALUE_SAMPLE) value_rollouts = value_rollouts > 0 ? value_rollouts : 101;
+  else if ((unsigned)value_strategy > 8u) return fail(h, "bb_rollout_value: bad value strategy");
+  else if (value_strategy != BB_SELECT_RANDOM || value_rollouts < 1) value_rollouts = 1;
   ENTER(h);
+  cudaStream_t s = (cudaStream_t)stream;
   BBRolloutArgs A;
   A.W.hidden = hidden; A.W.W1 = W1_dev; A.W.b1 = b1_dev; A.W.w2 = w2_dev; A.W.b2 = b2_dev; A.W.seed = seed;
   A.W.greedy = greedy ? 1 : 0;
   A.T = T; A.counter0 = counter0; A.actions = actions_dev; A.logp = logprob_dev; A.reward = reward_dev; A.done = done_dev;
   A.lengths = lengths_dev; A.obs = obs_dev; A.pmax = pmax;
-  if (h->P.auto_reset) { rc = pre_refill(h, (cudaStream_t)stream, true); if (rc < 0) return rc; }
-  CK(h->K->rollout(h->P, A, h->P.num_envs, (cudaStream_t)stream));
+  BBParams F;
+  BBValueArgs V;
+  if (value_dev) {   // one fork slot per environment: environment e's value rollouts run in slot e
+    const int N = h->P.num_envs;
+    if ((long long)N > (long long)(((size_t)8 << 30) / h->P.slot_stride))
+      return fail(h, "bb_rollout_value: the fork arena (one slot per environment) would exceed 8 GiB");
+    if (N > h->fork_cap) CK(cudaStreamSynchronize(s));
+    rc = fork_params(h, std::max(N, h->fork_cap), F);
+    if (rc < 0) return rc;
+    F.num_envs = N;
+    V.strategy = value_strategy; V.rollouts = value_rollouts; V.sel_seed_base = value_sel_seed; V.max_steps = value_max_steps;
+    V.gamma = value_gamma; V.value = value_dev; V.queue = nullptr; V.ntasks = 0;
+  }
+  if (h->P.auto_reset) { rc = pre_refill(h, s, true); if (rc < 0) return rc; }
+  CK(h->K->rollout(h->P, A, value_dev ? &F : nullptr, value_dev ? &V : nullptr, h->P.num_envs, s));
   return 0;
 }
 

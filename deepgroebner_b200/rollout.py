@@ -58,16 +58,21 @@ class PairsPolicy:
         return torch.log_softmax(z, dim=-1)
 
 
-def collect(env, net, T, counter0=0, greedy=False, store_obs=True, pmax=64, max_episode_length=None):
+def collect(env, net, T, counter0=0, greedy=False, store_obs=True, pmax=64, max_episode_length=None, value=None, gamma=0.99,
+            value_rollouts=None, value_seed=0):
     """Runs T steps of every environment of a LeadMonomialsEnv under policy `net` and returns a TrajectoryBatch.
     The environments must have been reset; auto-reset keeps every slot busy.  max_episode_length cuts episodes as
     pg.Agent.run_episode does (pg.py:470-471; train.py's default is 500).  States with more than pmax rows keep their
-    action and log-probability but cannot be stored: TrajectoryBatch.get() leaves them out (and counts them)."""
+    action and log-probability but cannot be stored: TrajectoryBatch.get() leaves them out (and counts them).
+    value: 'degree', 'sample' or another selection name -- every state's env.value(value, gamma) is computed in the same
+    launch (the baseline pg.Agent.run_episode stores with a value model, pg.py:461-462) and finish() / get() use it.
+    Pass the `gam` of finish() / get() as gamma, as pg.py passes its own gam to env.value."""
     eng = env.engine
     eng.set_auto_reset(True)
     if max_episode_length is not None:
         eng.set_max_episode_length(max_episode_length)
-    out = eng.rollout(net, T, counter0=counter0, greedy=greedy, store_obs=store_obs, pmax=pmax)
+    out = eng.rollout(net, T, counter0=counter0, greedy=greedy, store_obs=store_obs, pmax=pmax, value=value,
+                      value_gamma=gamma, value_rollouts=value_rollouts, value_seed=value_seed)
     return TrajectoryBatch(out, engine=eng)
 
 
@@ -106,7 +111,9 @@ def compute_advantages(rewards, values, done, gam, lam, engine=None):
 
 
 class TrajectoryBatch:
-    """[N, T] trajectories on device with the TrajectoryBuffer post-processing of the reference."""
+    """[N, T] trajectories on device with the TrajectoryBuffer post-processing of the reference.  When `out` has "value"
+    (rollout(value=...)), finish() and get() called with values=None use those values as the baseline; they should have
+    been computed with the gamma later given to finish() / get() as gam (pg.py passes self.gam to env.value)."""
 
     def __init__(self, out, engine=None):
         self.engine = engine   # with it, the discounted sums run as one kernel each (bb_discount)
@@ -115,6 +122,7 @@ class TrajectoryBatch:
         self.reward, self.lengths = out["reward"], out["lengths"]
         self.done = out["done"].bool()
         self.obs = out.get("obs")
+        self.value = out.get("value")
         N, T = self.reward.shape
         # a step belongs to a FINISHED trajectory iff some done follows it (inclusive) inside the window
         later = torch.flip(torch.cummax(torch.flip(self.done, [1]).to(torch.uint8), dim=1).values, [1]).bool()
@@ -140,7 +148,10 @@ class TrajectoryBatch:
         return ends_r - prev_r[idx], ends_s - prev_s[idx]
 
     def finish(self, gam=0.99, lam=0.97, values=None):
-        """TrajectoryBuffer.finish for every episode segment: returns (rewards_to_go, advantages), float64 [N, T]."""
+        """TrajectoryBuffer.finish for every episode segment: returns (rewards_to_go, advantages), float64 [N, T].
+        values None: the batch's own values if it has them, else zeros."""
+        if values is None:
+            values = self.value
         v = torch.zeros_like(self.reward) if values is None else values
         return (discount_rewards(self.reward, self.done, gam, self.engine),
                 compute_advantages(self.reward, v, self.done, gam, lam, self.engine))

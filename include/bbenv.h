@@ -12,7 +12,8 @@
  *   void reset()                         pxd:13             bb_reset / bb_set_ideals
  *   double step(int)                     pxd:14             bb_step
  *   vector[int] state, int cols          pxd:17-18          bb_observe, bb_cols
- *   double value(string,double)          pxd:16             bb_value (fork + rollouts from the live state)
+ *   double value(string,double)          pxd:16             bb_value (fork + rollouts from the live state);
+ *                                                             bb_rollout_value (every state of a fused rollout)
  *   LeadMonomialsEnv(const&)  (copy())   pxd:12             bb_copy_env
  *   buchberger(F, selection, ...)  buchberger.h:127-147     bb_run_export (whole episodes, all nine SelectionTypes;
  *                                                             every episode's reduced basis into a device sink), bb_run
@@ -350,7 +351,8 @@ int bb_set_wide(bb_handle* h, int mode);
  * is untouched.  strategy = BB_SELECT_RANDOM runs `rollouts` rollouts per environment (stream seeds sel_seed_base + r)
  * and keeps the best; BB_VALUE_SAMPLE is value("sample"): one Degree rollout and rollouts-1 (default 100) Random
  * rollouts seeded sel_seed_base + 0..99, best kept (:333-341; the reference seeds these from std::random_device).
- * A rollout that overflows an arena yields NaN for its environment. */
+ * A rollout that overflows an arena yields NaN for its environment.  bb_rollout_value computes the same value for every
+ * state of a fused rollout. */
 int bb_value(bb_handle* h, int strategy, double gamma, int rollouts, int sel_seed_base, int max_steps,
              double* value_dev, void* stream);
 
@@ -422,6 +424,27 @@ int bb_policy_pmlp(bb_handle* h, int hidden, const float* W1_dev, const float* b
 int bb_rollout(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev, const float* b2_dev,
                uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev, float* logprob_dev,
                float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax, void* stream);
+
+/* bb_rollout_value: bb_rollout that also writes value_dev double [N, T] (environment-major): value[e][t] = bb_value of the
+ * state step t of environment e starts from (the state obs[e][t] shows, with |P| = lengths[e][t]), i.e. the baseline
+ * pg.Agent.run_episode stores when the agent has a value model 'degree' / 'sample' (pg.py:461-462), computed inside the
+ * same launch; 0.0 where the environment is not running.  value_strategy, value_gamma, value_rollouts, value_sel_seed and
+ * value_max_steps are bb_value's strategy, gamma, rollouts, sel_seed_base and max_steps, with bb_value's rules (seeds,
+ * rollout counts, NaN for a rollout that overflows an arena); pass bb_value the gamma of the advantages (pg.py passes its
+ * own gam).  So with auto-reset on, the loop
+ *     for t in 0..T-1:  bb_value(v[:, t]); bb_policy_pmlp(counter0 + t); bb_step
+ * gives bit-identical values, actions, log-probabilities, rewards, done flags and lengths.  Everything else bb_rollout
+ * writes -- outputs, the environments after the call, their random streams and prefetch queues, bb_stats and
+ * bb_counters -- is identical to bb_rollout with the same arguments: the value rollouts run in a fork arena of one slot
+ * per environment (kept with bb_value's, 8 GiB at most) and their traffic is not counted.  The rollouts of one state run
+ * one after another in that environment's warp, so 'sample' (101 rollouts) costs about 101 times 'degree' per step.
+ * value_dev == NULL is bb_rollout (the value arguments are still checked).  Fails (nothing enqueued) for what bb_rollout
+ * refuses, a bad value strategy, and a fork arena that cannot be allocated or would exceed 8 GiB. */
+int bb_rollout_value(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev,
+                     const float* b2_dev, uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev,
+                     float* logprob_dev, float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax,
+                     int value_strategy, double value_gamma, int value_rollouts, int value_sel_seed, int value_max_steps,
+                     double* value_dev, void* stream);
 
 /* bb_run_policy: bb_run_export with the PMLP head of bb_policy_pmlp choosing every pair instead of a SelectionType -- the
  * trained agent evaluated on whole episodes (pg.Agent.run_episode, pg.py:451-472, run to completion), with the same
