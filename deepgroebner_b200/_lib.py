@@ -66,7 +66,7 @@ EXPORTS = [
     "bb_seed_selection", "bb_value", "bb_copy_env", "bb_set_auto_reset", "bb_step_observe", "bb_step_host", "bb_reset_host", "bb_observe_host", "bb_set_wide", "bb_set_prepare_mode", "bb_set_two_term", "bb_set_selection_seed_stride", "bb_policy_pmlp", "bb_rollout",
     "bb_seed_on", "bb_prepare", "bb_set_episode_offset", "bb_set_timing", "bb_last_run_ms", "bb_set_max_episode_length",
     "bb_set_compaction", "bb_compact", "bb_status_summary", "bb_set_obs_nvars", "bb_discount", "bb_set_serve", "bb_set_prefetch",
-    "bb_run_export", "bb_reduce", "bb_run_policy", "bb_rollout_value",
+    "bb_run_export", "bb_reduce", "bb_run_policy", "bb_rollout_value", "bb_rollout_rows",
 ]
 
 _lib = None
@@ -173,6 +173,8 @@ def load():
     lib.bb_rollout.argtypes = [vp, i, vp, vp, vp, vp, u64, u64, i, i, vp, vp, vp, vp, vp, vp, i, vp]
     lib.bb_rollout_value.restype = i
     lib.bb_rollout_value.argtypes = lib.bb_rollout.argtypes[:-1] + [i, C.c_double, i, i, i, vp, vp]
+    lib.bb_rollout_rows.restype = i
+    lib.bb_rollout_rows.argtypes = lib.bb_rollout_value.argtypes[:-1] + [vp, C.c_int64, vp]
     lib.bb_run_policy.restype = i
     lib.bb_run_policy.argtypes = [vp, i, vp, vp, vp, vp, u64, u64, i, i, i, vp, i, C.c_double, i, vp, vp, i, i, vp,
                                   C.POINTER(BBPolySink), C.POINTER(BBPolySink)]

@@ -713,13 +713,25 @@ class BuchbergerEngine:
                                              int(pmax or 0), _stream()), "bb_policy_pmlp")
         return (actions, logp, allp) if return_all else (actions, logp)
 
+    # rows_per_env=True: max(max_pairs, ROWS_PER_STEP * T) rows per environment, the memory of the dense block at
+    # pmax = 64, but a wide state uses the rows narrow ones leave.  Measured (profiles/README.md, N = 16384, T = 64, an
+    # untrained policy): 3-20-10-weighted uses at most 3138 of 4096 rows; 5-5-10-uniform (62 rows a state) halts 7693 of
+    # 16384 environments, which continue in the next call.
+    ROWS_PER_STEP = 64
+
     def rollout(self, net, T, counter0=0, greedy=False, store_obs=False, pmax=None, out=None, value=None, value_gamma=0.99,
-                value_rollouts=None, value_seed=0, value_max_steps=0):
+                value_rollouts=None, value_seed=0, value_max_steps=0, rows_per_env=None):
         """T fused steps of every environment (bb_rollout).  Returns a dict of [N, T] cuda tensors: actions, logp,
         reward, done, lengths (+ obs [N, T, pmax, cols] when store_obs).  value: a selection name or 'sample' (as in
         value()) -- the dict gains "value", float64 [N, T]: value(value, value_gamma, value_rollouts, value_seed,
-        value_max_steps) of the state each step starts from, computed in the same launch (bb_rollout_value)."""
+        value_max_steps) of the state each step starts from, computed in the same launch (bb_rollout_value).
+        rows_per_env: an int (at least max_pairs), or True for max(max_pairs, ROWS_PER_STEP * T) -- the dict gains
+        "rows", int32 [N, rows_per_env, cols]: the rows of every state an action is taken from, back to back in step
+        order (bb_rollout_rows).  An environment whose next state does not fit into what is left of its rows halts:
+        its remaining steps have action -1 and done 0, and the next call continues from that state."""
         N, dev = self.num_envs, self.device
+        if rows_per_env is True:
+            rows_per_env = max(self.caps["max_pairs"], self.ROWS_PER_STEP * int(T))
         vcode = vr = 0
         if value is not None:
             vcode = _lib.VALUE_SAMPLE if value == "sample" else _lib.SELECTION[value]
@@ -739,12 +751,17 @@ class BuchbergerEngine:
             args = (self.h, net.hidden, _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2), int(net.seed), int(counter0),
                     int(bool(greedy)), int(T), _ptr(o["actions"]), _ptr(o["logp"]), _ptr(o["reward"]), _ptr(o["done"]),
                     _ptr(o["lengths"]), _ptr(obs), int(pmax or 0))
-            if value is None:
+            if value is None and rows_per_env is None:
                 self._ck(self.lib.bb_rollout(*args, _stream()), "bb_rollout")
             else:
-                v = o.setdefault("value", torch.empty((N, T), dtype=torch.float64, device=dev))
-                self._ck(self.lib.bb_rollout_value(*args, vcode, float(value_gamma), int(vr), int(value_seed),
-                                                   int(value_max_steps), _ptr(v), _stream()), "bb_rollout_value")
+                v = rows = None
+                if value is not None:
+                    v = o.setdefault("value", torch.empty((N, T), dtype=torch.float64, device=dev))
+                if rows_per_env is not None:
+                    rows = o.setdefault("rows", torch.empty((N, int(rows_per_env), self.cols), dtype=torch.int32, device=dev))
+                self._ck(self.lib.bb_rollout_rows(*args, vcode, float(value_gamma), int(vr), int(value_seed),
+                                                  int(value_max_steps), _ptr(v), _ptr(rows), int(rows_per_env or 0),
+                                                  _stream()), "bb_rollout_rows")
         return o
 
     def copy_env(self, dst_env, src, src_env):

@@ -112,6 +112,10 @@ struct BBRolloutArgs {
   // outputs, all [N, T] (environment-major: one trajectory is contiguous); any may be NULL
   int32_t* actions; float* logp; float* reward; uint8_t* done; int32_t* lengths;
   int32_t* obs; int pmax;         // optional [N, T, pmax, cols] state matrices BEFORE each step, padded with -1
+  // optional row store [N, rows_per_env, cols]: the rows of every state an action is taken from, back to back in step
+  // order; an environment whose next state does not fit into what is left of its region halts (bb_rollout_rows)
+  int32_t* rows; long long rows_per_env;
+  int rows_budget;                // min(rows_per_env, INT_MAX): the rows one environment may take in one call
 };
 
 // Mailbox of the single-environment server (k_serve), in mapped pinned host memory.  The host writes a command and bumps
@@ -1141,7 +1145,11 @@ __device__ __noinline__ double warp_state_value(const BBParams& P, const BBParam
 // synchronisation between environments.  Trajectories are written environment-major.  VALUE (k_rollout_value): V->value[e, t]
 // is the value of the state step t starts from (warp_state_value; 0.0 where the environment is not running), F the fork
 // arena and acc the warp's accumulator in shared memory; nothing else the rollout writes changes.
-template <int NV, int UPL, bool VALUE>
+// ROWS (k_rollout_rows, k_rollout_value) with A.rows != NULL: the running state's |P| rows go to the next free rows of the
+// environment's region.  When they do not fit, the environment halts at that step t: steps t..T-1 take no action (action
+// -1, done 0, every other output 0, obs all -1) and the environment keeps that state for the next call.  ROWS is a template
+// parameter so that k_rollout (ROWS false) keeps its code: a runtime branch alone made it 4 % slower on a B200.
+template <int NV, int UPL, bool VALUE, bool ROWS>
 __device__ __forceinline__ void rollout_worker(const BBParams& P, const BBRolloutArgs& A, const BBParams* F,
                                                const BBValueArgs* V, BBEpisodeAcc* acc) {
   extern __shared__ float wsm[];
@@ -1158,9 +1166,16 @@ __device__ __forceinline__ void rollout_worker(const BBParams& P, const BBRollou
       warp_next_episode<NV>(P, slot, row);
       env_load(P, slot, e);
     }
+    int used = 0;   // rows of the row store taken so far
+    int t = 0;
 #pragma unroll 1
-    for (int t = 0; t < A.T; t++) {
+    for (; t < A.T; t++) {
       const size_t o = (size_t)slot * A.T + t;
+      if (ROWS && A.rows && e.status == BB_STATUS_RUNNING) {
+        if (e.nP > A.rows_budget - used) break;   // the budget rule: halt here
+        warp_observe<NV>(P, e, A.rows + ((size_t)slot * A.rows_per_env + used) * P.cols, e.nP, ct);
+        used += e.nP;
+      }
       if (A.lengths && lane == 0) A.lengths[o] = e.nP;
       if (A.obs) warp_observe<NV>(P, e, A.obs + o * A.pmax * P.cols, A.pmax, ct);
       if constexpr (VALUE) {
@@ -1187,6 +1202,22 @@ __device__ __forceinline__ void rollout_worker(const BBParams& P, const BBRollou
         env_load(P, slot, e);
       }
     }
+    if constexpr (ROWS) {
+      for (int u = t + lane; u < A.T; u += 32) {   // steps t..T-1 of an environment the row budget halted
+        const size_t o = (size_t)slot * A.T + u;
+        if (A.actions) A.actions[o] = -1;
+        if (A.logp) A.logp[o] = 0.0f;
+        if (A.reward) A.reward[o] = 0.0f;
+        if (A.done) A.done[o] = 0;
+        if (A.lengths) A.lengths[o] = 0;
+        if constexpr (VALUE) V->value[o] = 0.0;
+      }
+      if (A.obs && t < A.T) {
+        int32_t* ob = A.obs + ((size_t)slot * A.T + t) * A.pmax * P.cols;
+        const size_t n = (size_t)(A.T - t) * A.pmax * P.cols;
+        for (size_t x = lane; x < n; x += 32) ob[x] = -1;
+      }
+    }
     env_store(P, slot, e);
     ct.spill(row);
   }
@@ -1196,7 +1227,13 @@ __device__ __forceinline__ void rollout_worker(const BBParams& P, const BBRollou
 template <int NV, int UPL>
 __global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout(const __grid_constant__ BBParams P,
                                                            const __grid_constant__ BBRolloutArgs A) {
-  rollout_worker<NV, UPL, false>(P, A, nullptr, nullptr, nullptr);
+  rollout_worker<NV, UPL, false, false>(P, A, nullptr, nullptr, nullptr);
+}
+
+template <int NV, int UPL>
+__global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS) k_rollout_rows(const __grid_constant__ BBParams P,
+                                                                const __grid_constant__ BBRolloutArgs A) {
+  rollout_worker<NV, UPL, false, true>(P, A, nullptr, nullptr, nullptr);
 }
 
 template <int NV, int UPL>
@@ -1204,7 +1241,7 @@ __global__ void __launch_bounds__(BB_THREADS, BB_ROLLOUT_MIN_BLOCKS)
 k_rollout_value(const __grid_constant__ BBParams P, const __grid_constant__ BBRolloutArgs A, const __grid_constant__ BBParams F,
                 const __grid_constant__ BBValueArgs V) {
   __shared__ BBEpisodeAcc acc_sh[BB_WARPS];  // value rollouts' accumulators, lane 0 only: kept out of registers
-  rollout_worker<NV, UPL, true>(P, A, &F, &V, acc_sh);
+  rollout_worker<NV, UPL, true, true>(P, A, &F, &V, acc_sh);
 }
 
 // ------------------------------------------------------------------------------------------------ reduce(g, F)
@@ -1512,11 +1549,12 @@ struct BBLaunch {
         k_rollout_value<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, A, *F, *V);
         return cudaGetLastError();
       }
+      auto k = A.rows ? k_rollout_rows<NV, UPL> : k_rollout<NV, UPL>;
       if (sm > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(k_rollout<NV, UPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         if (e != cudaSuccess) return e;
       }
-      k_rollout<NV, UPL><<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, A);
+      k<<<grid_for_warps(nwarps), BB_THREADS, sm, s>>>(P, A);
       return cudaGetLastError();
     });
   }

@@ -4,6 +4,7 @@
 #include <emmintrin.h>
 
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -1527,10 +1528,22 @@ int bb_rollout_value(bb_handle* h, int hidden, const float* W1_dev, const float*
                      float* logprob_dev, float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax,
                      int value_strategy, double value_gamma, int value_rollouts, int value_sel_seed, int value_max_steps,
                      double* value_dev, void* stream) {
+  return bb_rollout_rows(h, hidden, W1_dev, b1_dev, w2_dev, b2_dev, seed, counter0, greedy, T, actions_dev, logprob_dev,
+                         reward_dev, done_dev, lengths_dev, obs_dev, pmax, value_strategy, value_gamma, value_rollouts,
+                         value_sel_seed, value_max_steps, value_dev, nullptr, 0, stream);
+}
+
+int bb_rollout_rows(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev,
+                    const float* b2_dev, uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev,
+                    float* logprob_dev, float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax,
+                    int value_strategy, double value_gamma, int value_rollouts, int value_sel_seed, int value_max_steps,
+                    double* value_dev, int32_t* rows_dev, int64_t rows_per_env, void* stream) {
   if (!h) return -1;
   int rc = check_policy(h, hidden, W1_dev, b1_dev, w2_dev, b2_dev);
   if (rc < 0) return rc;
   if (T < 1 || (obs_dev && pmax < 1)) return fail(h, "bb_rollout: bad argument");
+  // every environment can store the state it starts the call from
+  if (rows_dev && rows_per_env < h->P.max_pairs) return fail(h, "bb_rollout_rows: rows_per_env is below max_pairs");
   // bb_value's rules
   if (value_strategy == BB_VALUE_SAMPLE) value_rollouts = value_rollouts > 0 ? value_rollouts : 101;
   else if ((unsigned)value_strategy > 8u) return fail(h, "bb_rollout_value: bad value strategy");
@@ -1541,7 +1554,8 @@ int bb_rollout_value(bb_handle* h, int hidden, const float* W1_dev, const float*
   A.W.hidden = hidden; A.W.W1 = W1_dev; A.W.b1 = b1_dev; A.W.w2 = w2_dev; A.W.b2 = b2_dev; A.W.seed = seed;
   A.W.greedy = greedy ? 1 : 0;
   A.T = T; A.counter0 = counter0; A.actions = actions_dev; A.logp = logprob_dev; A.reward = reward_dev; A.done = done_dev;
-  A.lengths = lengths_dev; A.obs = obs_dev; A.pmax = pmax;
+  A.lengths = lengths_dev; A.obs = obs_dev; A.pmax = pmax; A.rows = rows_dev; A.rows_per_env = rows_dev ? rows_per_env : 0;
+  A.rows_budget = (int)std::min<int64_t>(A.rows_per_env, INT_MAX);
   BBParams F;
   BBValueArgs V;
   if (value_dev) {   // one fork slot per environment: environment e's value rollouts run in slot e

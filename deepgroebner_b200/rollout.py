@@ -9,7 +9,9 @@ stepping together on device.
 * ``TrajectoryBatch``  -- rewards-to-go and generalised advantage estimates per episode segment
                           (pg.discount_rewards / pg.compute_advantages, pg.py:18-78), the "only finished
                           trajectories" rule of TrajectoryBuffer (pg.py:183-226: data up to ``self.start``), the
-                          single-action filter and the -1 padded batches the reference networks consume.
+                          single-action filter and the -1 padded batches the reference networks consume; with
+                          the row store of ``collect(rows_per_env=...)`` every state is kept at its own row count,
+                          as the reference's buffer keeps it, and ``batches()`` pads each minibatch on its own.
 """
 import math
 
@@ -58,21 +60,27 @@ class PairsPolicy:
         return torch.log_softmax(z, dim=-1)
 
 
-def collect(env, net, T, counter0=0, greedy=False, store_obs=True, pmax=64, max_episode_length=None, value=None, gamma=0.99,
-            value_rollouts=None, value_seed=0):
+def collect(env, net, T, counter0=0, greedy=False, store_obs=None, pmax=64, max_episode_length=None, value=None, gamma=0.99,
+            value_rollouts=None, value_seed=0, rows_per_env=None):
     """Runs T steps of every environment of a LeadMonomialsEnv under policy `net` and returns a TrajectoryBatch.
     The environments must have been reset; auto-reset keeps every slot busy.  max_episode_length cuts episodes as
     pg.Agent.run_episode does (pg.py:470-471; train.py's default is 500).  States with more than pmax rows keep their
     action and log-probability but cannot be stored: TrajectoryBatch.get() leaves them out (and counts them).
     value: 'degree', 'sample' or another selection name -- every state's env.value(value, gamma) is computed in the same
     launch (the baseline pg.Agent.run_episode stores with a value model, pg.py:461-462) and finish() / get() use it.
-    Pass the `gam` of finish() / get() as gamma, as pg.py passes its own gam to env.value."""
+    Pass the `gam` of finish() / get() as gamma, as pg.py passes its own gam to env.value.
+    rows_per_env: an int or True (BuchbergerEngine.rollout) -- every state is stored at its own row count, as the
+    reference's TrajectoryBuffer stores it, so get() drops none; environments whose rows run out halt (see
+    TrajectoryBatch.halted) and continue in the next call.  store_obs (default: only without rows_per_env) adds the
+    dense [N, T, pmax, cols] block."""
     eng = env.engine
     eng.set_auto_reset(True)
     if max_episode_length is not None:
         eng.set_max_episode_length(max_episode_length)
+    if store_obs is None:
+        store_obs = rows_per_env is None
     out = eng.rollout(net, T, counter0=counter0, greedy=greedy, store_obs=store_obs, pmax=pmax, value=value,
-                      value_gamma=gamma, value_rollouts=value_rollouts, value_seed=value_seed)
+                      value_gamma=gamma, value_rollouts=value_rollouts, value_seed=value_seed, rows_per_env=rows_per_env)
     return TrajectoryBatch(out, engine=eng)
 
 
@@ -113,7 +121,11 @@ def compute_advantages(rewards, values, done, gam, lam, engine=None):
 class TrajectoryBatch:
     """[N, T] trajectories on device with the TrajectoryBuffer post-processing of the reference.  When `out` has "value"
     (rollout(value=...)), finish() and get() called with values=None use those values as the baseline; they should have
-    been computed with the gamma later given to finish() / get() as gam (pg.py passes self.gam to env.value)."""
+    been computed with the gamma later given to finish() / get() as gam (pg.py passes self.gam to env.value).
+
+    States come from `out["rows"]` (rows mode, rollout(rows_per_env=...)) when it is there, else from `out["obs"]`
+    (dense mode).  In rows mode every state is kept at its own row count: offsets[e, t] is the first row of step t's
+    state in environment e's region, and no sample is dropped for its width."""
 
     def __init__(self, out, engine=None):
         self.engine = engine   # with it, the discounted sums run as one kernel each (bb_discount)
@@ -122,11 +134,19 @@ class TrajectoryBatch:
         self.reward, self.lengths = out["reward"], out["lengths"]
         self.done = out["done"].bool()
         self.obs = out.get("obs")
+        self.rows = out.get("rows")
         self.value = out.get("value")
         N, T = self.reward.shape
         # a step belongs to a FINISHED trajectory iff some done follows it (inclusive) inside the window
         later = torch.flip(torch.cummax(torch.flip(self.done, [1]).to(torch.uint8), dim=1).values, [1]).bool()
         self.finished = later & (self.actions >= 0)
+        self.offsets, self.halted = None, 0
+        if self.rows is not None:
+            # bb_rollout_rows' layout: the states of the steps that took an action, back to back in step order
+            took = self.lengths.to(torch.int64) * (self.actions >= 0)
+            self.offsets = torch.cumsum(took, dim=1) - took
+            # environments the row budget stopped: the only outputs with action -1 and done 0
+            self.halted = int(((self.actions < 0) & ~self.done).any(dim=1).sum())
 
     def episode_stats(self):
         """(returns, lengths) of the episodes that finished inside the window, as 1-D tensors."""
@@ -156,18 +176,55 @@ class TrajectoryBatch:
         return (discount_rewards(self.reward, self.done, gam, self.engine),
                 compute_advantages(self.reward, v, self.done, gam, lam, self.engine))
 
-    def get(self, gam=0.99, lam=0.97, values=None, normalize_advantages=True):
-        """The flat training set of TrajectoryBuffer.get (pg.py:183-226): steps of finished trajectories whose state
-        had more than one row, as (obs [M, pmax, cols] padded -1, actions, logprobs, advantages, rewards_to_go)."""
+    def _samples(self, gam, lam, values, normalize_advantages):
+        """The training set as (env, step, actions, logprobs, advantages, rewards_to_go), 1-D, in (env, step) order."""
         rtg, adv = self.finish(gam, lam, values)
         keep = self.finished
         a = adv[keep].to(torch.float32)
         if normalize_advantages and a.numel() > 1:
             a = (a - a.mean()) / a.std(unbiased=False)
         multi = self.lengths[keep] != 1
-        if self.obs is not None:   # a state with more rows than were stored cannot be a training sample
+        if self.obs is not None and self.rows is None:   # a state with more rows than were stored cannot be a sample
             fits = self.lengths[keep] <= self.obs.shape[2]
             self.dropped_wide = int((multi & ~fits).sum())
             multi = multi & fits
-        obs = self.obs[keep][multi] if self.obs is not None else None
-        return obs, self.actions[keep][multi], self.logp[keep][multi], a[multi], rtg[keep][multi].to(torch.float32)
+        e, t = keep.nonzero(as_tuple=True)
+        return e[multi], t[multi], self.actions[keep][multi], self.logp[keep][multi], a[multi], rtg[keep][multi].to(torch.float32)
+
+    def states(self, e, t):
+        """The state matrices of steps (e[i], t[i]) as [M, rows, cols], padded with -1 to the largest of them."""
+        L = self.lengths[e, t].to(torch.int64)
+        width = int(L.max()) if L.numel() else 0
+        if self.rows is None:
+            return self.obs[e, t, :width]
+        R, cols = self.rows.shape[1], self.rows.shape[2]
+        j = torch.arange(width, device=L.device)
+        valid = j < L[:, None]
+        at = e.to(torch.int64)[:, None] * R + torch.where(valid, self.offsets[e, t][:, None] + j, 0)
+        return torch.where(valid[..., None], self.rows.reshape(-1, cols)[at], -1)
+
+    def get(self, gam=0.99, lam=0.97, values=None, normalize_advantages=True):
+        """The flat training set of TrajectoryBuffer.get (pg.py:183-226): steps of finished trajectories whose state
+        had more than one row, as (obs [M, rows, cols] padded -1, actions, logprobs, advantages, rewards_to_go).
+        Dense mode: rows = pmax, and states wider than pmax are left out (counted in dropped_wide).  Rows mode: rows =
+        the largest kept state."""
+        e, t, actions, logp, a, rtg = self._samples(gam, lam, values, normalize_advantages)
+        if self.rows is not None:
+            obs = self.states(e, t)
+        else:
+            obs = self.obs[e, t] if self.obs is not None else None
+        return obs, actions, logp, a, rtg
+
+    def batches(self, batch_size, gam=0.99, lam=0.97, values=None, normalize_advantages=True, seed=None):
+        """get()'s training set as minibatches (obs, actions, logprobs, advantages, rewards_to_go) of batch_size
+        samples (the last may be smaller); each obs is padded with -1 to the largest state of its own minibatch, as
+        the reference pads its batches.  Advantages are normalised over the whole set.  seed None keeps get()'s order;
+        an int shuffles the samples with torch.Generator().manual_seed(seed)."""
+        e, t, actions, logp, a, rtg = self._samples(gam, lam, values, normalize_advantages)
+        M = e.numel()
+        order = torch.arange(M) if seed is None else torch.randperm(M, generator=torch.Generator().manual_seed(seed))
+        order = order.to(e.device)
+        have = self.rows is not None or self.obs is not None
+        for i in range(0, M, batch_size):
+            s = order[i:i + batch_size]
+            yield (self.states(e[s], t[s]) if have else None), actions[s], logp[s], a[s], rtg[s]

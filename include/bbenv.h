@@ -18,6 +18,7 @@
  *   buchberger(F, selection, ...)  buchberger.h:127-147     bb_run_export (whole episodes, all nine SelectionTypes;
  *                                                             every episode's reduced basis into a device sink), bb_run
  *   policy_model(state) + categorical   pg.py:323-326       bb_policy_pmlp / bb_rollout (PMLP head, networks.py:522-571)
+ *   TrajectoryBuffer states (unpadded)  pg.py:162-241       bb_rollout_rows (every state at its own row count)
  *   pg.Agent.run_episode to completion  pg.py:451-472       bb_run_policy (whole episodes, the PMLP head selecting, with
  *                                                             bb_run_export's records, traces and sinks)
  *   BuchbergerEnv::G, ::P   buchberger.h:195-196            bb_download_basis, bb_pairs
@@ -445,6 +446,26 @@ int bb_rollout_value(bb_handle* h, int hidden, const float* W1_dev, const float*
                      float* logprob_dev, float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax,
                      int value_strategy, double value_gamma, int value_rollouts, int value_sel_seed, int value_max_steps,
                      double* value_dev, void* stream);
+
+/* bb_rollout_rows: bb_rollout_value (value_dev may be NULL) that also stores the state matrix of every step at its own
+ * row count -- the reference's TrajectoryBuffer, which keeps each state unpadded and pads only when it forms a batch
+ * (pg.py:162-241) -- so no state is lost to a pmax.  rows_dev int32 [N, rows_per_env, cols]: environment e owns rows
+ * rows_dev[e][0 .. rows_per_env) (of which one call fills at most 2^31 - 1).  The |P| = lengths[e][t] rows of each state an action is taken from (actions[e][t] >= 0)
+ * go there back to back, in step order, without padding; rows past the last state are untouched.  So the rows of step t
+ * start at row  sum of lengths[e][t'] over t' < t with actions[e][t'] >= 0  of e's region.
+ * Budget rule: when the rows of the state step t of environment e starts from do not fit into what is left of e's region,
+ * e takes no further step in this call: steps t..T-1 get action -1, logprob 0, reward 0, done 0, lengths 0, value 0.0 and
+ * obs all -1, and e keeps the state of step t, so the next call continues it and no state is lost.  This is the only way
+ * an output has action -1 with done 0 (a slot that is not running reports done 1).  Halted steps are not env-steps;
+ * bb_counters' obs_rows counts the rows written (row store and obs).  Every step before the halt is exactly what the same
+ * call without a row store gives (step t still samples with counter counter0 + t).  rows_dev and obs_dev are independent.
+ * rows_dev == NULL is bb_rollout_value.  Fails (nothing enqueued) for what bb_rollout_value refuses, and for rows_dev !=
+ * NULL with rows_per_env < bb_config.max_pairs: that minimum lets every environment store the state it starts from. */
+int bb_rollout_rows(bb_handle* h, int hidden, const float* W1_dev, const float* b1_dev, const float* w2_dev,
+                    const float* b2_dev, uint64_t seed, uint64_t counter0, int greedy, int T, int32_t* actions_dev,
+                    float* logprob_dev, float* reward_dev, uint8_t* done_dev, int32_t* lengths_dev, int32_t* obs_dev, int pmax,
+                    int value_strategy, double value_gamma, int value_rollouts, int value_sel_seed, int value_max_steps,
+                    double* value_dev, int32_t* rows_dev, int64_t rows_per_env, void* stream);
 
 /* bb_run_policy: bb_run_export with the PMLP head of bb_policy_pmlp choosing every pair instead of a SelectionType -- the
  * trained agent evaluated on whole episodes (pg.Agent.run_episode, pg.py:451-472, run to completion), with the same
